@@ -337,6 +337,16 @@ int kp_loss_head_bwd(const float* pred, const float* image, int64_t N, const int
                      float* grad_dist /* [N] or NULL */, float* const* grad_il_ptrs /* HOST array [n_levels] or NULL */,
                      void* stream);
 
+/* ---- eval-image metrics: per image of a batch the PSNR (data_range 1) and SSIM (11x11 gaussian window, sigma 1.5,
+ *      k1 0.01, k2 0.03, data_range = max(range(pred), range(target)) of the image) that utils/image_metrics.py computes
+ *      one image at a time (NS/models/kplanes.py:454-515).  pred, target: fp32 [B,H,W,3]; out: fp32 [B,2] = (psnr, ssim).
+ *      The SSIM mean runs over the (H-10)*(W-10)*3 windows lying wholly inside the image (exactly what image_metrics.ssim
+ *      keeps after its reflect-pad + crop); H or W < 11 is an error.  scratch: kp_image_metrics_scratch_bytes(B, H, W)
+ *      device bytes, 16-byte aligned.  3 launches, no host synchronisation, no float atomics (bitwise reproducible),
+ *      graph-capturable. ---- */
+int64_t kp_image_metrics_scratch_bytes(int B, int H, int W);
+int kp_image_metrics(const float* pred, const float* target, int B, int H, int W, void* scratch, float* out, void* stream);
+
 /* ---- (e) data-parallel gradient all-reduce over NVLink peer memory (replaces the NCCL all-reduce torch DDP issues
  *      around NS/engine/trainer.py:382-412).  Every rank allocates one ARENA = [KP_PEER_SIGNAL_BYTES of flag words |
  *      data], exports its CUDA-IPC handle, and opens the arenas of the other ranks of the node.  kp_peer_allreduce

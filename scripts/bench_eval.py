@@ -1,0 +1,162 @@
+#!/usr/bin/env python
+"""bench_eval.py -- evaluation of a trained scene on B200s: Evaluator.get_average_eval_image_metrics over 8 eval images at
+1920x1080 rendered from the 32x field (bench.py's cfg3 model, the BASELINE config-5 workload), and kp_image_metrics against
+the torch restatement of PSNR + SSIM (utils/image_metrics.py) on the same frames and the same device.
+
+    python scripts/bench_eval.py                                                       # 1 GPU
+    python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 scripts/bench_eval.py   # 8 GPUs (images i % 8 == rank)
+
+Prints one JSON line (rank 0).  The eval targets are the model's own frames plus seeded noise: the metric values are
+not a quality statement, the times are the point.  Kernel timing: CUDA events around each pass, after warm-up, with a
+512 MB buffer written between passes so neither pass reads its frames from L2 (126 MB).
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+import torch  # noqa: E402
+
+
+def card_info(index: int) -> dict:
+    try:
+        out = subprocess.run(["nvidia-smi", f"--id={index}", "--query-gpu=name,power.limit,clocks.max.sm",
+                              "--format=csv,noheader"], capture_output=True, text=True, timeout=30).stdout.strip()
+        name, power, clock = (p.strip() for p in out.split(","))
+        return {"name": name, "power_limit": power, "sm_max_clock": clock}
+    except Exception as exc:  # the device name from torch is still recorded
+        return {"name": torch.cuda.get_device_name(index), "power_limit": f"unknown ({exc})"}
+
+
+def eval_cameras(n: int, h: int, w: int, dev):
+    """bench.py's eval_leg camera path: a short arc of the broadcast ring, looking at the origin."""
+    from soccernerfs_b200.cameras.cameras import Cameras
+
+    ang = torch.linspace(0.0, 1.0, n) * 0.6
+    pos = torch.stack([torch.cos(ang), torch.sin(ang), torch.full_like(ang, 0.35)], dim=-1)
+    fwd = -pos / pos.norm(dim=-1, keepdim=True)
+    right = torch.cross(fwd, torch.tensor([0.0, 0.0, 1.0]).expand_as(fwd), dim=-1)
+    right = right / right.norm(dim=-1, keepdim=True)
+    up = torch.cross(right, fwd, dim=-1)
+    c2w = torch.cat([torch.stack([right, up, -fwd], dim=-1), pos[..., None]], dim=-1)
+    return Cameras(c2w.to(dev), 1600.0, 1600.0, w / 2, h / 2, w, h, times=torch.linspace(0, 1, n)[:, None].to(dev))
+
+
+def kernel_vs_torch(pred, target, reps: int) -> dict:
+    """Median ms of ops.image_metrics on the batch vs image_metrics.psnr + ssim image by image (as
+    get_image_metrics_and_images calls them), with L2 overwritten before every pass."""
+    from soccernerfs_b200 import ops
+    from soccernerfs_b200.utils import image_metrics
+
+    flush = torch.empty(512 * 2**20 // 4, dtype=torch.float32, device=pred.device)
+    p4 = [torch.moveaxis(p, -1, 0)[None] for p in pred]
+    t4 = [torch.moveaxis(t, -1, 0)[None] for t in target]
+
+    def torch_pass():
+        return [(image_metrics.psnr(t, p), image_metrics.ssim(t, p)) for p, t in zip(p4, t4)]
+
+    def timed(fn):
+        times = []
+        for _ in range(reps):
+            flush.fill_(1.0)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            fn()
+            e1.record()
+            torch.cuda.synchronize()
+            times.append(e0.elapsed_time(e1))
+        return sorted(times)[len(times) // 2], times
+
+    for _ in range(3):
+        ops.image_metrics(pred, target)
+        torch_pass()
+    torch.cuda.synchronize()
+    ours = ops.image_metrics(pred, target).cpu()
+    ref = torch.tensor([[float(a), float(b)] for a, b in torch_pass()])
+    k_ms, k_all = timed(lambda: ops.image_metrics(pred, target))
+    t_ms, t_all = timed(torch_pass)
+    b, h, w = pred.shape[:3]
+    bytes_read = 2 * b * h * w * 3 * 4 * 2  # both images, read by the stats pass and by the SSIM pass
+    return {"images": b, "hw": [h, w], "kp_image_metrics_ms": k_ms, "torch_psnr_ssim_ms": t_ms, "speedup": t_ms / k_ms,
+            "kp_ms_all": k_all, "torch_ms_all": t_all, "kp_bytes_read_min": bytes_read,
+            "kp_effective_gbs": bytes_read / (k_ms * 1e-3) / 1e9,
+            "torch_tf32_conv": bool(torch.backends.cudnn.allow_tf32),
+            "max_abs_diff_psnr": float((ours[:, 0] - ref[:, 0]).abs().max()),
+            "max_abs_diff_ssim": float((ours[:, 1] - ref[:, 1]).abs().max()), "l2_flush": "512 MB written before every pass"}
+
+
+def main() -> None:
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--images", type=int, default=8)
+    ap.add_argument("--height", type=int, default=1080)
+    ap.add_argument("--width", type=int, default=1920)
+    ap.add_argument("--repeats", type=int, default=3, help="timed calls of get_average_eval_image_metrics")
+    ap.add_argument("--kernel-reps", type=int, default=20)
+    ap.add_argument("--out", help="also write the JSON result to this file")
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_eval.py measures on a CUDA device; none is visible")
+
+    import bench
+    from soccernerfs_b200.data.datamanagers.dynamic_datamanager import DynamicDataManager, DynamicDataManagerConfig
+    from soccernerfs_b200.engine.evaluator import Evaluator
+
+    rank, world, local = bench._dist_setup()
+    dev = torch.device("cuda", local)
+    torch.cuda.set_device(dev)
+    model = bench.build_model("cfg3", dev)
+    model.eval()
+    cams = eval_cameras(args.images, args.height, args.width, dev)
+    gen = torch.Generator(device=dev).manual_seed(7)
+    renders, frames = [], []
+    with torch.no_grad():
+        from soccernerfs_b200.engine.frame_renderer import FrameRenderer
+
+        renderer = FrameRenderer(model, cams)
+        for i in range(args.images):  # every rank builds the same targets (same model, same seed)
+            f = renderer.render(i, device_frames=True)["rgb"]
+            renders.append(f)
+            frames.append((f + 0.03 * torch.randn(f.shape, generator=gen, device=dev)).clamp(0, 1))
+        del renderer
+    targets = torch.stack(frames)
+    cfg = DynamicDataManagerConfig(use_importance_sampling=False)
+    dm = DynamicDataManager(cfg, cams, targets, device=dev, eval_cameras=cams, eval_images=targets)
+    evaluator = Evaluator(model, dm, rank=rank, world=world)
+    evaluator.get_average_eval_image_metrics(0)  # warm-up: tile graphs captured, kernels loaded
+    calls = []
+    for r in range(args.repeats):
+        if world > 1:
+            torch.distributed.barrier()
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        res = evaluator.get_average_eval_image_metrics(r + 1)  # ends with the metrics on the host of every rank
+        calls.append(time.perf_counter() - t0)
+        torch.cuda.synchronize()
+    result = {"metric": "eval over the eval split (Evaluator.get_average_eval_image_metrics)",
+              "workload": f"kplanes-32x(cfg3 field), {args.images} eval images at {args.width}x{args.height}, chunk "
+                          f"{model.config.eval_num_rays_per_chunk}, whole images per rank (i % world == rank)",
+              "gpus": world, "card": card_info(local), "seconds_per_call": sorted(calls)[len(calls) // 2],
+              "seconds_per_image": sorted(calls)[len(calls) // 2] / args.images, "seconds_per_call_all": calls,
+              "results": res}
+    if rank == 0:
+        result["kernel"] = kernel_vs_torch(torch.stack(renders), targets, args.kernel_reps)
+        line = json.dumps(result)
+        print(line)
+        if args.out:
+            os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+            with open(args.out, "w") as f:
+                f.write(line + "\n")
+    if world > 1:
+        torch.distributed.barrier()
+        torch.distributed.destroy_process_group()
+
+
+if __name__ == "__main__":
+    main()

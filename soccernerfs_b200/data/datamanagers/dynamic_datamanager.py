@@ -14,7 +14,8 @@ live on the device and ``next_train`` (NS/data/datamanagers/base_datamanager.py:
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+import random
+from dataclasses import dataclass, replace
 from typing import Any, Dict, Iterator, Literal, Optional, Tuple
 
 import torch
@@ -117,16 +118,19 @@ class DeviceImageCache:
 
 
 class DynamicDataManager:
-    """The train side of ``DynamicDataManager`` / ``VanillaDataManager.next_train`` (dynamic_datamanager.py:60-113,
-    base_datamanager.py:486-494) on a device-resident image cache: pixel sampler -> pixel gather -> ray generator, every
-    tensor a CUDA tensor.  ``cameras``: one camera per cached image (nerfstudio's convention: ``image_idx`` indexes them),
-    carrying ``times`` and ``ids``."""
+    """``DynamicDataManager`` / ``VanillaDataManager`` (dynamic_datamanager.py:60-113, base_datamanager.py:486-494) on
+    device-resident image caches: pixel sampler -> pixel gather -> ray generator, every tensor a CUDA tensor.  ``cameras``:
+    one camera per cached image (nerfstudio's convention: ``image_idx`` indexes them), carrying ``times`` and ``ids``.
+    ``next_train`` serves the train split; ``next_eval`` / ``next_eval_image`` the optional eval split."""
 
     def __init__(self, config: DynamicDataManagerConfig, cameras, images: torch.Tensor, device="cuda",
-                 extras: Optional[Dict[str, torch.Tensor]] = None, prefetch: bool = False, **sampler_kwargs: Any) -> None:
+                 extras: Optional[Dict[str, torch.Tensor]] = None, prefetch: bool = False, eval_cameras=None,
+                 eval_images: Optional[torch.Tensor] = None, **sampler_kwargs: Any) -> None:
         """``prefetch``: the batch ``next_train`` returns was produced on a side stream while the previous step ran, and
         the next one is enqueued there before returning -- the ~0.5 ms of sampler / gather / ray-generation kernels and
-        their launch latencies leave the training stream (same batches in the same order as without it)."""
+        their launch latencies leave the training stream (same batches in the same order as without it).
+        ``eval_cameras`` / ``eval_images`` [B,H,W,3]: the eval split, cached on the device beside the train images (without
+        importance maps: eval batches are drawn uniformly)."""
         from ...model_components.ray_generators import RayGenerator
 
         self.config = config
@@ -144,6 +148,18 @@ class DynamicDataManager:
         self.train_count = 0
         self._side = torch.cuda.Stream(device=self.device) if prefetch else None
         self._ready = None  # (ray_bundle, batch, event) produced ahead on the side stream
+        self.eval_cameras = self.eval_image_cache = None
+        if (eval_cameras is None) != (eval_images is None):
+            raise ValueError("eval_cameras and eval_images come together")
+        if eval_cameras is not None:
+            self.eval_cameras = eval_cameras.to(self.device)
+            if len(self.eval_cameras) != eval_images.shape[0]:
+                raise ValueError(f"{eval_images.shape[0]} eval images for {len(self.eval_cameras)} eval cameras")
+            self.eval_image_cache = DeviceImageCache(eval_images, replace(config, use_importance_sampling=False), device=self.device)
+            self.iter_eval_image_dataloader = iter(self.eval_image_cache)
+            self.eval_pixel_sampler = PixelSampler(config.eval_num_rays_per_batch)
+            self.eval_ray_generator = RayGenerator(self.eval_cameras)
+        self.eval_count = 0
 
     def _produce(self) -> Tuple[Any, Dict[str, Any]]:
         image_batch = next(self.iter_train_image_dataloader)
@@ -183,3 +199,22 @@ class DynamicDataManager:
             t.record_stream(main)  # allocated on the side stream, consumed on the training stream
         self._produce_ahead(main)
         return ray_bundle, batch
+
+    def _need_eval(self) -> None:
+        if self.eval_image_cache is None:
+            raise RuntimeError("this datamanager has no eval split: pass eval_cameras and eval_images")
+
+    def next_eval(self, step: int) -> Tuple[Any, Dict[str, Any]]:
+        """-> (RayBundle, batch) of ``eval_num_rays_per_batch`` pixels drawn uniformly from the eval images
+        (``VanillaDataManager.next_eval``)."""
+        self._need_eval()
+        self.eval_count += 1
+        batch = self.eval_pixel_sampler.sample(next(self.iter_eval_image_dataloader))
+        return self.eval_ray_generator(batch["indices"]), batch
+
+    def next_eval_image(self, step: int) -> Tuple[int, Dict[str, torch.Tensor]]:
+        """-> (camera index, {"image": [H,W,3] device tensor}) of a random eval image (``VanillaDataManager.next_eval_image``:
+        a random draw of the eval dataloader); render the camera with ``engine.frame_renderer.FrameRenderer``."""
+        self._need_eval()
+        i = random.randrange(len(self.eval_cameras))
+        return i, {"image": self.eval_image_cache.batch["image"][i]}

@@ -1,0 +1,163 @@
+"""Evaluation of a trained model over its eval split: the eval side of ``VanillaPipeline``
+(``get_eval_loss_dict``, ``get_eval_image_metrics_and_images``, ``get_average_eval_image_metrics``,
+NS/pipelines/base_pipeline.py:343-352) and the JSON that ``ns-eval`` writes (REF/nerfstudio/scripts/eval.py:20-44).
+
+``get_average_eval_image_metrics`` keeps the frames on the device: each image is rendered by ``FrameRenderer`` into device
+tensors, and the PSNR / SSIM of all of a rank's images come from one ``ops.image_metrics`` call (three kernel launches)
+instead of the torch restatement and its host synchronisations per image.  With ``world > 1`` rank r renders the images
+``i % world == r``; one ``all_gather`` brings every image's row to every rank, and each key is averaged in image order,
+so the result does not depend on the world size.
+"""
+from __future__ import annotations
+
+from typing import Any, Callable, Dict, List, Sequence, Tuple
+
+import torch
+
+from .. import ops
+from ..configs.method_configs import KPLANES_TRAINER
+from ..utils import image_metrics
+from .frame_renderer import FrameRenderer
+
+
+def images_of_rank(n_images: int, rank: int, world: int) -> List[int]:
+    """Eval images rank ``rank`` of ``world`` renders: i % world == rank."""
+    return list(range(rank, n_images, world))
+
+
+def average_metrics(rows: Dict[int, Dict[str, float]], keys: Sequence[str]) -> Dict[str, float]:
+    """Mean of every key over the images, in image order, as the reference averages its per-image dicts
+    (``float(torch.mean(torch.tensor([...])))``)."""
+    order = sorted(rows)
+    return {k: float(torch.mean(torch.tensor([rows[i][k] for i in order]))) for k in keys}
+
+
+def pack_rows(rows: Dict[int, Dict[str, float]], keys: Sequence[str], n_rows: int) -> torch.Tensor:
+    """float64 [n_rows, 1 + len(keys)] = (image index, values...) for ``all_gather``; unused rows have index -1."""
+    out = torch.full((n_rows, 1 + len(keys)), -1.0, dtype=torch.float64)
+    for r, i in enumerate(sorted(rows)):
+        out[r, 0] = i
+        out[r, 1:] = torch.tensor([rows[i][k] for k in keys], dtype=torch.float64)
+    return out
+
+
+def unpack_rows(packed: Sequence[torch.Tensor], keys: Sequence[str]) -> Dict[int, Dict[str, float]]:
+    rows: Dict[int, Dict[str, float]] = {}
+    for t in packed:
+        for row in t.cpu().tolist():
+            if row[0] >= 0:
+                rows[int(row[0])] = dict(zip(keys, row[1:]))
+    return rows
+
+
+def eval_report(results: Dict[str, float], experiment_name: str, checkpoint: str,
+                method_name: str = KPLANES_TRAINER["method_name"]) -> Dict[str, Any]:
+    """The JSON ``ns-eval`` writes: {experiment_name, method_name, checkpoint, results}."""
+    return {"experiment_name": experiment_name, "method_name": method_name, "checkpoint": str(checkpoint),
+            "results": dict(results)}
+
+
+class Evaluator:
+    """Eval metrics of ``model`` on the eval split of ``datamanager`` (a ``DynamicDataManager`` built with
+    ``eval_cameras`` / ``eval_images``).  ``rank`` / ``world``: this process' share of ``get_average_eval_image_metrics``
+    (``torch.distributed`` must be initialised when ``world > 1``)."""
+
+    def __init__(self, model, datamanager, rank: int = 0, world: int = 1) -> None:
+        if datamanager.eval_cameras is None:
+            raise ValueError("Evaluator: the datamanager has no eval split (eval_cameras / eval_images)")
+        self.model, self.datamanager = model, datamanager
+        self.rank, self.world = rank, world
+        outputs = ["rgb", "depth", "accumulation", "median_rgb"]
+        outputs += [f"prop_depth_{i}" for i in range(getattr(model.config, "num_proposal_iterations", 0))]
+        # whole frames per rank: the renderer itself is not sharded
+        self.renderer = FrameRenderer(model, datamanager.eval_cameras, outputs=outputs)
+        self._warm: set = set()
+        self._lpips = None
+        self._lpips_checked = False
+
+    def _size(self, i: int) -> Tuple[int, int]:
+        cams = self.datamanager.eval_cameras
+        return cams._height_host[i], cams._width_host[i]
+
+    def get_eval_loss_dict(self, step: int) -> Tuple[Dict[str, torch.Tensor], Dict[str, torch.Tensor], Dict[str, torch.Tensor]]:
+        """-> (outputs, loss_dict, metrics_dict) of the model in eval mode on a ``next_eval`` batch."""
+        was_training = self.model.training
+        self.model.eval()
+        try:
+            with torch.no_grad():
+                ray_bundle, batch = self.datamanager.next_eval(step)
+                outputs = self.model(ray_bundle)
+                metrics_dict = self.model.get_metrics_dict(outputs, batch)
+                loss_dict = self.model.get_loss_dict(outputs, batch, metrics_dict)
+        finally:
+            self.model.train(was_training)
+        return outputs, loss_dict, metrics_dict
+
+    def get_eval_image_metrics_and_images(self, step: int) -> Tuple[Dict[str, float], Dict[str, torch.Tensor]]:
+        """One random eval image, rendered whole and passed to the model's ``get_image_metrics_and_images``."""
+        i, batch = self.datamanager.next_eval_image(step)
+        outputs = self.renderer.render(i, device_frames=True)
+        metrics_dict, images_dict = self.model.get_image_metrics_and_images(outputs, batch)
+        h, w = self._size(i)
+        metrics_dict["image_idx"] = i
+        metrics_dict["num_rays"] = h * w
+        return metrics_dict, images_dict
+
+    def _render_timed(self, i: int) -> Tuple[torch.Tensor, Callable[[], float]]:
+        """-> (rgb [H,W,3] on the device, seconds of the render: call once the stream has passed the render)."""
+        if self._size(i) not in self._warm:  # the first frame of a size captures the tile graphs: not part of the time
+            self.renderer.render(i, device_frames=True)
+            self._warm.add(self._size(i))
+        start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        start.record()
+        rgb = self.renderer.render(i, device_frames=True)["rgb"]
+        end.record()
+        return rgb, lambda: start.elapsed_time(end) / 1e3
+
+    def _lpips_metric(self, device):
+        if not self._lpips_checked:  # the model's rule: LPIPS only when its pretrained network is available
+            self._lpips = image_metrics.optional_lpips(device)
+            self._lpips_checked = True
+        return self._lpips
+
+    def _rank_rows(self, mine: Sequence[int]) -> Dict[int, Dict[str, float]]:
+        """Per-image rows {psnr, ssim, [lpips], num_rays_per_sec, fps} of this rank's images."""
+        if not mine:
+            return {}
+        renders = [self._render_timed(i) for i in mine]
+        pred = torch.stack([rgb for rgb, _ in renders])
+        target = self.datamanager.eval_image_cache.batch["image"][torch.tensor(mine, device=pred.device)]
+        values = ops.image_metrics(pred, target).tolist()  # the one host synchronisation: the events have completed too
+        lpips = self._lpips_metric(pred.device)
+        rows = {}
+        for k, i in enumerate(mine):
+            h, w = self._size(i)
+            row = {"psnr": values[k][0], "ssim": values[k][1]}
+            if lpips is not None:
+                row["lpips"] = float(lpips(torch.moveaxis(target[k], -1, 0)[None], torch.moveaxis(pred[k], -1, 0)[None]))
+            row["num_rays_per_sec"] = h * w / renders[k][1]()
+            row["fps"] = row["num_rays_per_sec"] / (h * w)
+            rows[i] = row
+        return rows
+
+    def _keys(self, device) -> List[str]:
+        return ["psnr", "ssim"] + (["lpips"] if self._lpips_metric(device) is not None else []) + ["num_rays_per_sec", "fps"]
+
+    def _all_gather(self, rows: Dict[int, Dict[str, float]], keys: Sequence[str], n_images: int) -> Dict[int, Dict[str, float]]:
+        import torch.distributed as dist
+
+        dev = torch.device("cuda", torch.cuda.current_device())
+        packed = pack_rows(rows, keys, -(-n_images // self.world)).to(dev)
+        gathered = [torch.empty_like(packed) for _ in range(self.world)]
+        dist.all_gather(gathered, packed)
+        return unpack_rows(gathered, keys)
+
+    def get_average_eval_image_metrics(self, step: int = 0) -> Dict[str, float]:
+        """Every eval image: ``psnr``, ``ssim`` (and ``lpips`` when available), ``num_rays_per_sec`` and ``fps`` averaged
+        over the images (``VanillaPipeline.get_average_eval_image_metrics``)."""
+        n = len(self.datamanager.eval_cameras)
+        rows = self._rank_rows(images_of_rank(n, self.rank, self.world))
+        keys = self._keys(self.datamanager.device)
+        if self.world > 1:
+            rows = self._all_gather(rows, keys, n)
+        return average_metrics(rows, keys)

@@ -871,6 +871,28 @@ def ist_map(images: torch.Tensor, nbr_offsets: torch.Tensor, nbrs: torch.Tensor,
     return out
 
 
+def image_metrics(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+    """Per-image (psnr, ssim) of a batch on the device (kp_image_metrics): pred, target fp32 CUDA [B,H,W,3] with
+    H, W >= 11 -> fp32 [B,2].  Equal to ``utils.image_metrics.psnr`` / ``ssim`` applied image by image to the
+    [1,3,H,W] forms; no host synchronisation, so it can be captured in a CUDA graph."""
+    if pred.dim() != 4 or pred.shape[-1] != 3 or target.shape != pred.shape:
+        raise ValueError(f"image_metrics: pred and target must both be [B,H,W,3] (got {tuple(pred.shape)}, {tuple(target.shape)})")
+    if pred.dtype != torch.float32 or target.dtype != torch.float32:
+        raise TypeError("image_metrics: pred and target must be float32")
+    if not pred.is_cuda or target.device != pred.device:
+        raise RuntimeError("image_metrics: pred and target must be CUDA tensors on one device (there is no CPU path)")
+    b, h, w = pred.shape[:3]
+    if h < 11 or w < 11:
+        raise ValueError(f"image_metrics: {h}x{w} images are smaller than the 11x11 SSIM window")
+    pred, target = pred.contiguous(), target.contiguous()
+    out = torch.empty((b, 2), dtype=torch.float32, device=pred.device)
+    if b == 0:
+        return out
+    scratch = torch.empty(int(_lib.load().kp_image_metrics_scratch_bytes(b, h, w)), dtype=torch.uint8, device=pred.device)
+    call("kp_image_metrics", ptr(pred), ptr(target), b, h, w, c_void_p(scratch.data_ptr()), ptr(out), stream_ptr())
+    return out
+
+
 _HEAD_WS: Dict = {}
 
 
