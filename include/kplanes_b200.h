@@ -347,6 +347,25 @@ int kp_loss_head_bwd(const float* pred, const float* image, int64_t N, const int
 int64_t kp_image_metrics_scratch_bytes(int B, int H, int W);
 int kp_image_metrics(const float* pred, const float* target, int B, int H, int W, void* scratch, float* out, void* stream);
 
+/* ---- frame composition for a rendered camera path (the per-frame image work of ns-render, REF/nerfstudio/scripts/
+ *      render.py: colour-map every requested output and concatenate them along the width): P <= KP_COMPOSE_MAX_PANELS
+ *      panels of one frame -> out uint8 [H, W*P, 3], panel p in columns [p*W, (p+1)*W).  panels: HOST array [P] of fp32
+ *      device pointers, [H,W,3] for KP_PANEL_COLOR, [H,W,1] otherwise; kinds: HOST array [P].  The mapping is that of
+ *      KPlanesModel.get_image_metrics_and_images (utils/colormaps.py): colour as is; accumulation -> viridis[(int64)(a*255)];
+ *      depth -> turbo[(int64)(d'*255)] * acc + (1 - acc), d' = clip((d - min) * rn(1/den), 0, 1), den =
+ *      fp32(double(max) - double(min) + 1e-10), min / max over the frame's panel; accumulation: fp32 [H,W,1], needed with a
+ *      depth panel.  turbo, viridis: fp32 [256,3] device tables (utils/colormaps._table); a colour-map index outside
+ *      [0, 255] is clamped.  Every channel is quantised as floor(clamp(x, 0, 1) * 255 + 0.5), NaN -> 0.  Bit-identical to
+ *      that torch restatement on the device.  scratch: kp_compose_frame_scratch_bytes(H, W, P) device bytes, 8-byte
+ *      aligned.  1 launch (2 with a depth panel), no host synchronisation, graph-capturable. ---- */
+#define KP_COMPOSE_MAX_PANELS 8
+#define KP_PANEL_COLOR 0
+#define KP_PANEL_ACCUMULATION 1
+#define KP_PANEL_DEPTH 2
+int64_t kp_compose_frame_scratch_bytes(int H, int W, int P);
+int kp_compose_frame(const float* const* panels, const int* kinds, int P, int H, int W, const float* accumulation,
+                     const float* turbo, const float* viridis, void* scratch, uint8_t* out, void* stream);
+
 /* ---- (e) data-parallel gradient all-reduce over NVLink peer memory (replaces the NCCL all-reduce torch DDP issues
  *      around NS/engine/trainer.py:382-412).  Every rank allocates one ARENA = [KP_PEER_SIGNAL_BYTES of flag words |
  *      data], exports its CUDA-IPC handle, and opens the arenas of the other ranks of the node.  kp_peer_allreduce

@@ -84,6 +84,8 @@ SIGNATURES = {
     "kp_importance_pixels": ([_P, c_int, c_int64, c_int, _P, c_int, c_int, ctypes.c_uint64, _P, _P, _P], c_int),
     "kp_image_metrics_scratch_bytes": ([c_int, c_int, c_int], c_int64),
     "kp_image_metrics": ([_P, _P, c_int, c_int, c_int, _P, _P, _P], c_int),
+    "kp_compose_frame_scratch_bytes": ([c_int, c_int, c_int], c_int64),
+    "kp_compose_frame": ([_P, POINTER(c_int), c_int, c_int, c_int, _P, _P, _P, _P, _P, _P], c_int),
     "kp_loss_head_fwd": ([_P, _P, c_int64, _P, _P, _P, c_int, c_float, c_float, c_float, _P, c_int, _P, _P, _P, _P, _P], c_int),
     "kp_loss_head_bwd": ([_P, _P, c_int64, _P, c_int, c_float, c_float, c_float, _P, _P, _P, _P, _P, _P], c_int),
     "kp_peer_alloc": ([c_int64, POINTER(c_void_p), _P], c_int),

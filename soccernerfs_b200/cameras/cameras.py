@@ -150,6 +150,23 @@ class Cameras:
                       distortion_params=self.distortion_params, camera_type=self.camera_type, times=self.times, ids=self.ids)
         return out
 
+    def rescale_output_resolution(self, scaling_factor: Union[float, int, torch.Tensor]) -> None:
+        """Scale the output resolution in place (cameras.py ``rescale_output_resolution``, ns-render's
+        ``--downscale-factor``): fx, fy, cx, cy times the factor, height / width = (size * factor) cast to int64.
+        ``scaling_factor``: a number or a tensor [num_cameras] / [num_cameras, 1]."""
+        if isinstance(scaling_factor, (float, int)):
+            scaling_factor = torch.tensor([scaling_factor]).to(self.device).broadcast_to(self.cx.shape)
+        elif torch.is_tensor(scaling_factor) and tuple(scaling_factor.shape) in ((self.size,), (self.size, 1)):
+            scaling_factor = scaling_factor.to(self.device, torch.float32).reshape(self.size, 1)  # fp32 intrinsics
+        else:
+            raise ValueError(f"scaling_factor must be a number or a tensor of shape [{self.size}] or [{self.size}, 1]")
+        self.fx, self.fy = self.fx * scaling_factor, self.fy * scaling_factor
+        self.cx, self.cy = self.cx * scaling_factor, self.cy * scaling_factor
+        self.height = (self.height * scaling_factor).to(torch.int64)
+        self.width = (self.width * scaling_factor).to(torch.int64)
+        self._height_host, self._width_host = self.height.view(-1).tolist(), self.width.view(-1).tolist()
+        self._intrinsics = None  # packed again from the new fx, fy, cx, cy on the next ray generation
+
     def get_image_coords(self, pixel_offset: float = 0.5, index=None) -> torch.Tensor:
         """[H,W,2] (y, x) pixel-centre coordinates (cameras.py:299-326)."""
         if index is None:

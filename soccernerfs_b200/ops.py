@@ -893,6 +893,68 @@ def image_metrics(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
     return out
 
 
+COMPOSE_MAX_PANELS = 8
+_COLORMAP_TABLES: Dict = {}
+
+
+def panel_kind(name: str) -> int:
+    """How ``compose_frame`` maps a rendered output: 1 = accumulation (viridis), 2 = a depth (turbo, blended with the
+    accumulation; ns-render's rule: any name containing "depth"), 0 = a colour shown as it is."""
+    if name == "accumulation":
+        return 1
+    return 2 if "depth" in name else 0
+
+
+def _colormap_tables(device) -> Tuple[torch.Tensor, torch.Tensor]:
+    key = str(device)
+    if key not in _COLORMAP_TABLES:  # copied once per device: no host-to-device copy per frame
+        from .utils import colormaps
+
+        _COLORMAP_TABLES[key] = tuple(colormaps._table(c).to(device).contiguous() for c in ("turbo", "viridis"))
+    return _COLORMAP_TABLES[key]
+
+
+def compose_frame(frames: Dict[str, torch.Tensor], names: Sequence[str]) -> torch.Tensor:
+    """The outputs ``names`` of one rendered frame (fp32 CUDA [H,W,3] colours, [H,W,1] accumulation / depths) ->
+    uint8 [H, W*len(names), 3], side by side in that order, colour-mapped as ``get_image_metrics_and_images`` maps them
+    (utils/colormaps.py; see ``panel_kind``) and quantised as floor(clamp(x, 0, 1) * 255 + 0.5) (kp_compose_frame).
+    A depth panel also needs ``frames["accumulation"]``.  On the current stream, no host synchronisation."""
+    names = list(names)
+    if not 1 <= len(names) <= COMPOSE_MAX_PANELS:
+        raise ValueError(f"compose_frame: 1..{COMPOSE_MAX_PANELS} outputs per frame (got {len(names)})")
+    missing = [n for n in names if n not in frames]
+    if missing:
+        raise ValueError(f"compose_frame: {missing} not among the frame's outputs {sorted(frames)}")
+    kinds = [panel_kind(n) for n in names]
+    acc = frames.get("accumulation") if 2 in kinds else None
+    if 2 in kinds and acc is None:
+        raise ValueError("compose_frame: a depth panel is blended with the accumulation, which the frame lacks")
+    first = frames[names[0]]
+    h, w = first.shape[:2]
+    panels = []
+    for name, kind in zip(names, kinds):
+        t = frames[name]
+        if t.dim() != 3 or tuple(t.shape[:2]) != (h, w) or t.shape[2] != (3 if kind == 0 else 1):
+            raise ValueError(f"compose_frame: {name} is {tuple(t.shape)}; expected [{h},{w},{3 if kind == 0 else 1}]")
+        if t.dtype != torch.float32:
+            raise TypeError(f"compose_frame: {name} must be float32")
+        if not t.is_cuda or t.device != first.device:
+            raise RuntimeError("compose_frame: the outputs must be CUDA tensors on one device (there is no CPU path)")
+        panels.append(t.contiguous())
+    if acc is not None:
+        if tuple(acc.shape) != (h, w, 1) or acc.dtype != torch.float32 or acc.device != first.device:
+            raise ValueError(f"compose_frame: accumulation must be fp32 [{h},{w},1] on {first.device}")
+        acc = acc.contiguous()
+    turbo, viridis = _colormap_tables(first.device)
+    p = len(panels)
+    out = torch.empty((h, w * p, 3), dtype=torch.uint8, device=first.device)
+    scratch = torch.empty(int(_lib.load().kp_compose_frame_scratch_bytes(h, w, p)), dtype=torch.uint8, device=first.device)
+    kind_arr = (c_int32 * p)(*kinds)
+    call("kp_compose_frame", _lib.ptr_array(panels), kind_arr, p, h, w, ptr(acc), ptr(turbo), ptr(viridis),
+         c_void_p(scratch.data_ptr()), c_void_p(out.data_ptr()), stream_ptr())
+    return out
+
+
 _HEAD_WS: Dict = {}
 
 
