@@ -193,28 +193,17 @@ int kp_interlevel_fwd(const float* c /* [N,S+1] */, const float* w /* [N,S] */, 
 int kp_interlevel_bwd(const float* c, const float* w, const float* cp, const float* wp, const float* grad_loss /* [N,S] */,
                       int64_t N, int S, int Sp, float* grad_wp /* [N,Sp] */, void* stream);
 
-/* ---- (a15) plane regularisers, losses.py:356-452: for ONE channel-last plane [H,W,C]:
- *      sums[0] = sum (t[h+1]-t[h])^2, sums[1] = sum (t[w+1]-t[w])^2, sums[2] = sum (second diff along H)^2,
- *      sums[3] = sum |1-t|  (double accumulators, device, ACCUMULATED).  The backward writes / adds
- *      sum_i coef[i] * d(sums[i])/dt (coef read from device memory so no host sync is needed). */
-int kp_plane_reg_fwd(const float* plane, int H, int W, int C, uint32_t terms /* bit i: compute sums[i] */,
-                     double* sums4, void* stream);
-int kp_plane_reg_bwd(const float* plane, int H, int W, int C, const float* coef_dev4 /* DEVICE float[4] */,
-                     uint32_t terms /* bit i: include term i */, int accumulate /* 0: grad = g, 1: grad += g */,
-                     float* grad, void* stream);
-
-/* Multi-plane variants: one launch for a whole list of planes.  planes/grads: HOST arrays [P] of device pointers,
- * hwc: HOST int32 [P*3] = (H, W, C) per plane, terms: HOST uint32 [P]; sums / coef_dev: DEVICE [P,4]. */
-int kp_plane_reg_multi_fwd(const float* const* planes, const int32_t* hwc, const uint32_t* terms, int P,
-                           double* sums /* [P,4], accumulated */, void* stream);
-int kp_plane_reg_multi_bwd(const float* const* planes, float* const* grads, const int32_t* hwc, const uint32_t* terms,
-                           int P, const float* coef_dev /* [P,4] */, int accumulate, void* stream);
-
-/* Values AND gradients of the regularisers in ONE sweep per plane (the training step's form): sums as above (may be
- * NULL), and grads[p] (may be NULL) = or += sum_i coef_dev[p,i] * d(sums[p,i])/d(plane).  With accumulate = 0 the sweep
- * also stands in for the gradient buffer's memset: every element of grads[p] is written. */
+/* ---- (a15) plane regularisers, losses.py:356-452, values AND gradients in ONE sweep per plane, one launch for a
+ *      whole list of channel-last planes [H,W,C].  planes/grads: HOST arrays [P] of device pointers, hwc: HOST int32
+ *      [P*3] = (H, W, C) per plane, terms: HOST uint32 [P] (bit i selects sums[p,i]).  For plane p:
+ *        sums[p,0] = sum (t[h+1]-t[h])^2, sums[p,1] = sum (t[w+1]-t[w])^2, sums[p,2] = sum (second diff along H)^2,
+ *        sums[p,3] = sum |1-t|
+ *      (DEVICE double [P,4], ACCUMULATED; may be NULL), and grads[p] (may be NULL) = or += sum_i coef_dev[p,i] *
+ *      d(sums[p,i])/d(plane), coef_dev DEVICE float [P,4] so that no host sync is needed.  coef_dev may be NULL only when
+ *      every grads[p] is NULL (sums only).  With accumulate = 0 the sweep also stands in for the gradient buffer's
+ *      memset: every element of grads[p] is written. */
 int kp_plane_reg_fused(const float* const* planes, float* const* grads, const int32_t* hwc, const uint32_t* terms, int P,
-                       const float* coef_dev /* [P,4] */, int accumulate, double* sums /* [P,4] accumulated, or NULL */,
+                       const float* coef_dev /* [P,4], or NULL */, int accumulate, double* sums /* [P,4] accumulated, or NULL */,
                        void* stream);
 /* Same; write_range_dev (DEVICE int64 [P,2], or NULL = everything): the gradient of plane p is written only for its float4
  * elements [begin, end) -- sums still cover the whole plane.  Used by the data-parallel step with the sparse gradient

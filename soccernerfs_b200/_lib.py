@@ -63,10 +63,6 @@ SIGNATURES = {
     "kp_distortion_bwd": ([_P, _P, _P, c_int64, c_int, _P, _P], c_int),
     "kp_interlevel_fwd": ([_P, _P, _P, _P, c_int64, c_int, c_int, _P, _P], c_int),
     "kp_interlevel_bwd": ([_P, _P, _P, _P, _P, c_int64, c_int, c_int, _P, _P], c_int),
-    "kp_plane_reg_fwd": ([_P, c_int, c_int, c_int, c_uint32, _P, _P], c_int),
-    "kp_plane_reg_bwd": ([_P, c_int, c_int, c_int, _P, c_uint32, c_int, _P, _P], c_int),
-    "kp_plane_reg_multi_fwd": ([_P, _P, _P, c_int, _P, _P], c_int),
-    "kp_plane_reg_multi_bwd": ([_P, _P, _P, _P, c_int, _P, c_int, _P], c_int),
     "kp_plane_reg_fused": ([_P, _P, _P, _P, c_int, _P, c_int, _P, _P], c_int),
     "kp_plane_reg_fused_range": ([_P, _P, _P, _P, c_int, _P, c_int, _P, _P, _P], c_int),
     "kp_plane_reg_fused_shard": ([_P, _P, _P, _P, c_int, _P, c_int, _P, _P, _P], c_int),

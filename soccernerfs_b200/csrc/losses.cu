@@ -1,8 +1,6 @@
 // Loss kernels (sm_100a).
 //   kp_distortion_*  : lossfun_distortion, NS/model_components/losses.py:125-136 (O(S^2) per ray, one warp per ray)
 //   kp_interlevel_*  : outer / lossfun_outer, losses.py:46-95 (two searchsorted(side="right") + cumsum differences)
-//   kp_plane_reg_*   : compute_plane_tv / compute_plane_smoothness / |1 - t|, losses.py:356-452, as one streaming
-//                      pass over a channel-last plane (float4 per thread), analytic gradients in the backward.
 //   kp_adam_step     : torch.optim.Adam update over a flat buffer (NS/engine/optimizers.py:74-160).
 #include "common.cuh"
 
@@ -115,90 +113,6 @@ __global__ void __launch_bounds__(32 * kRaysPerBlock) interlevel_kernel(const fl
   }
 }
 
-// ---- plane regularisers -----------------------------------------------------------------------------
-__device__ __forceinline__ float4 sub4(float4 a, float4 b) { return make_float4(a.x - b.x, a.y - b.y, a.z - b.z, a.w - b.w); }
-__device__ __forceinline__ float sq4(float4 a) { return a.x * a.x + a.y * a.y + a.z * a.z + a.w * a.w; }
-
-__global__ void __launch_bounds__(256) plane_reg_fwd_kernel(const float* __restrict__ t, int H, int W, int C4,
-                                                            uint32_t terms, double* __restrict__ sums) {
-  const int64_t total = (int64_t)H * W * C4;
-  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-  const int64_t row = (int64_t)W * C4;
-  for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
-    const int h = (int)(idx / row);
-    const int wq = (int)(idx % row);
-    const int wcol = wq / C4;
-    const float4 v = ldg4(t + idx * 4);
-    if ((terms & 1u) && h + 1 < H) s0 += sq4(sub4(ldg4(t + (idx + row) * 4), v));
-    if ((terms & 2u) && wcol + 1 < W) s1 += sq4(sub4(ldg4(t + (idx + C4) * 4), v));
-    if ((terms & 4u) && h + 2 < H) {
-      const float4 v1 = ldg4(t + (idx + row) * 4), v2 = ldg4(t + (idx + 2 * row) * 4);
-      s2 += sq4(sub4(sub4(v2, v1), sub4(v1, v)));
-    }
-    if (terms & 8u) s3 += fabsf(1.f - v.x) + fabsf(1.f - v.y) + fabsf(1.f - v.z) + fabsf(1.f - v.w);
-  }
-  __shared__ double red[4][8];
-  double d[4] = {warp_sum_d((double)s0), warp_sum_d((double)s1), warp_sum_d((double)s2), warp_sum_d((double)s3)};
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (lane == 0)
-    for (int k = 0; k < 4; ++k) red[k][warp] = d[k];
-  __syncthreads();
-  if (threadIdx.x < 4) {
-    double a = 0.0;
-    for (int wv = 0; wv < (int)(blockDim.x >> 5); ++wv) a += red[threadIdx.x][wv];
-    if ((terms >> threadIdx.x) & 1u) atomicAdd(&sums[threadIdx.x], a);
-  }
-}
-
-__device__ __forceinline__ float sgn(float x) { return (x > 0.f) ? 1.f : ((x < 0.f) ? -1.f : 0.f); }
-
-__global__ void __launch_bounds__(256) plane_reg_bwd_kernel(const float* __restrict__ t, int H, int W, int C4,
-                                                            const float* __restrict__ coef, uint32_t terms, int accumulate,
-                                                            float* __restrict__ grad) {
-  const float k0 = (terms & 1u) ? coef[0] : 0.f, k1 = (terms & 2u) ? coef[1] : 0.f;
-  const float k2 = (terms & 4u) ? coef[2] : 0.f, k3 = (terms & 8u) ? coef[3] : 0.f;
-  const int64_t total = (int64_t)H * W * C4;
-  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= total) return;
-  const int64_t row = (int64_t)W * C4;
-  const int h = (int)(idx / row);
-  const int wcol = (int)(idx % row) / C4;
-  const float4 v = ldg4(t + idx * 4);
-  float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-  const float4 zero = g;
-  const bool need_h = (k0 != 0.f) || (k2 != 0.f);
-  float4 up1 = zero, up2 = zero, dn1 = zero, dn2 = zero;  // t[h+1], t[h+2], t[h-1], t[h-2]
-  if (need_h) {
-    if (h + 1 < H) up1 = ldg4(t + (idx + row) * 4);
-    if (h >= 1) dn1 = ldg4(t + (idx - row) * 4);
-  }
-  if (k0 != 0.f) {
-    if (h >= 1) g = fma4(sub4(v, dn1), 2.f * k0, g);
-    if (h + 1 < H) g = fma4(sub4(up1, v), -2.f * k0, g);
-  }
-  if (k1 != 0.f) {
-    if (wcol >= 1) g = fma4(sub4(v, ldg4(t + (idx - C4) * 4)), 2.f * k1, g);
-    if (wcol + 1 < W) g = fma4(sub4(ldg4(t + (idx + C4) * 4), v), -2.f * k1, g);
-  }
-  if (k2 != 0.f) {
-    if (h + 2 < H) up2 = ldg4(t + (idx + 2 * row) * 4);
-    if (h >= 2) dn2 = ldg4(t + (idx - 2 * row) * 4);
-    // s_k = (t[k+2]-t[k+1]) - (t[k+1]-t[k]);  d/dt[h] = 2 (s_{h-2} - 2 s_{h-1} + s_h)
-    if (h >= 2) g = fma4(sub4(sub4(v, dn1), sub4(dn1, dn2)), 2.f * k2, g);                  // s_{h-2}
-    if (h >= 1 && h + 1 < H) g = fma4(sub4(sub4(up1, v), sub4(v, dn1)), -4.f * k2, g);     // s_{h-1}
-    if (h + 2 < H) g = fma4(sub4(sub4(up2, up1), sub4(up1, v)), 2.f * k2, g);               // s_h
-  }
-  if (k3 != 0.f) {
-    g.x -= k3 * sgn(1.f - v.x); g.y -= k3 * sgn(1.f - v.y); g.z -= k3 * sgn(1.f - v.z); g.w -= k3 * sgn(1.f - v.w);
-  }
-  float4* gp = reinterpret_cast<float4*>(grad + idx * 4);
-  if (accumulate) {
-    const float4 cur = *gp;
-    g.x += cur.x; g.y += cur.y; g.z += cur.z; g.w += cur.w;
-  }
-  *gp = g;
-}
-
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g,
                                                    float* __restrict__ m, float* __restrict__ v, int64_t n, float lr_over_bc1,
                                                    float beta1, float beta2, float eps, float wd, float inv_sqrt_bc2,
@@ -294,26 +208,6 @@ extern "C" int kp_interlevel_bwd(const float* c, const float* w, const float* cp
   interlevel_kernel<true><<<(unsigned)ceil_div(N, kRaysPerBlock), 32 * kRaysPerBlock, smem, as_stream(stream)>>>(
       c, w, cp, wp, grad_loss, N, S, Sp, nullptr, grad_wp);
   KP_LAUNCH_CHECK("interlevel_bwd");
-  return 0;
-}
-
-extern "C" int kp_plane_reg_fwd(const float* plane, int H, int W, int C, uint32_t terms, double* sums4, void* stream) {
-  KP_CHECK(plane && sums4 && H >= 1 && W >= 1 && C >= 4 && C % 4 == 0, "plane_reg_fwd: bad arguments (C must be a multiple of 4)");
-  const int64_t total = (int64_t)H * W * (C / 4);
-  const int64_t blocks = std::min<int64_t>(ceil_div(total, 256), 148 * 8);
-  plane_reg_fwd_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(plane, H, W, C / 4, terms, sums4);
-  KP_LAUNCH_CHECK("plane_reg_fwd");
-  return 0;
-}
-
-extern "C" int kp_plane_reg_bwd(const float* plane, int H, int W, int C, const float* coef_dev4, uint32_t terms,
-                                int accumulate, float* grad, void* stream) {
-  KP_CHECK(plane && grad && coef_dev4 && H >= 1 && W >= 1 && C >= 4 && C % 4 == 0, "plane_reg_bwd: bad arguments");
-  if ((terms & 15u) == 0 && accumulate) return 0;
-  const int64_t total = (int64_t)H * W * (C / 4);
-  plane_reg_bwd_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, as_stream(stream)>>>(plane, H, W, C / 4, coef_dev4, terms,
-                                                                                      accumulate, grad);
-  KP_LAUNCH_CHECK("plane_reg_bwd");
   return 0;
 }
 

@@ -1,30 +1,20 @@
 // Multi-tensor streaming kernels (sm_100a): one launch covers every plane / parameter of a group.
-//   kp_plane_reg_multi_fwd/bwd : the K-Planes regularisers (NS/model_components/losses.py:356-452) over a list of
-//                                channel-last planes -- 2 launches per loss term instead of 2 per plane (the
-//                                default model has 36 planes; per-plane launches were launch-latency bound).
-//   kp_adam_multi              : torch.optim.Adam over a list of dense fp32 tensors (NS/engine/optimizers.py:74-160,
-//                                method_configs.py:546-557); hyper-parameters may come from device memory so the
-//                                step can be replayed from a CUDA graph.
-// Work is split into fixed-size chunks; a block finds its (tensor, chunk) by a short scan of a prefix table that
-// travels in the kernel parameters.
+//   kp_plane_reg_fused(_range, _shard) : values and gradients of the K-Planes regularisers
+//                                        (NS/model_components/losses.py:356-452) over a list of channel-last planes in
+//                                        one sweep (the default model has 36 planes; per-plane launches were
+//                                        launch-latency bound).
+//   kp_plane_reg_adam                  : the same regulariser stencil fused with an in-place Adam step.
+//   kp_adam_multi                      : torch.optim.Adam over a list of dense fp32 tensors (NS/engine/optimizers.py:74-160,
+//                                        method_configs.py:546-557); hyper-parameters may come from device memory so
+//                                        the step can be replayed from a CUDA graph.
+// Work is split into fixed-size chunks or tiles; a block finds its (tensor, chunk) by a short scan of a prefix table
+// that travels in the kernel parameters.
 #include "common.cuh"
 
 namespace kp {
 
 constexpr int kMaxTensors = 64;
-constexpr int kChunk = 2048;  // float4 elements per block (256 threads x 8)
-
-struct RegPlane {
-  const float* t;
-  float* g;
-  int H, W, C4;
-  uint32_t terms;
-};
-struct RegTable {
-  RegPlane pl[kMaxTensors];
-  int first_block[kMaxTensors + 1];
-  int n;
-};
+constexpr int kChunk = 2048;  // float4 elements per block of adam_multi_kernel (256 threads x 8)
 
 __device__ __forceinline__ int find_tensor(const int* first_block, int n, int b) {
   int p = 0;
@@ -36,91 +26,56 @@ __device__ __forceinline__ float4 sub4m(float4 a, float4 b) { return make_float4
 __device__ __forceinline__ float sq4m(float4 a) { return a.x * a.x + a.y * a.y + a.z * a.z + a.w * a.w; }
 __device__ __forceinline__ float sgnm(float x) { return (x > 0.f) ? 1.f : ((x < 0.f) ? -1.f : 0.f); }
 
-__global__ void __launch_bounds__(256) plane_reg_multi_fwd_kernel(const __grid_constant__ RegTable T,
-                                                                  double* __restrict__ sums) {
-  const int p = find_tensor(T.first_block, T.n, blockIdx.x);
-  const RegPlane& P = T.pl[p];
-  const float* __restrict__ t = P.t;
-  const int H = P.H, W = P.W, C4 = P.C4;
-  const uint32_t terms = P.terms;
-  const int64_t total = (int64_t)H * W * C4, row = (int64_t)W * C4;
-  const int64_t base = (int64_t)(blockIdx.x - T.first_block[p]) * kChunk;
-  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-#pragma unroll 2
-  for (int it = 0; it < kChunk / 256; ++it) {
-    const int64_t idx = base + it * 256 + threadIdx.x;
-    if (idx >= total) break;
-    const int h = (int)(idx / row);
-    const int wcol = (int)(idx % row) / C4;
-    const float4 v = ldg4(t + idx * 4);
-    if ((terms & 1u) && h + 1 < H) s0 += sq4m(sub4m(ldg4(t + (idx + row) * 4), v));
-    if ((terms & 2u) && wcol + 1 < W) s1 += sq4m(sub4m(ldg4(t + (idx + C4) * 4), v));
-    if ((terms & 4u) && h + 2 < H) {
-      const float4 v1 = ldg4(t + (idx + row) * 4), v2 = ldg4(t + (idx + 2 * row) * 4);
-      s2 += sq4m(sub4m(sub4m(v2, v1), sub4m(v1, v)));
-    }
-    if (terms & 8u) s3 += fabsf(1.f - v.x) + fabsf(1.f - v.y) + fabsf(1.f - v.z) + fabsf(1.f - v.w);
-  }
-  __shared__ double red[4][8];
-  const double d[4] = {warp_sum_d((double)s0), warp_sum_d((double)s1), warp_sum_d((double)s2), warp_sum_d((double)s3)};
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (lane == 0)
-    for (int k = 0; k < 4; ++k) red[k][warp] = d[k];
-  __syncthreads();
-  if (threadIdx.x < 4 && ((terms >> threadIdx.x) & 1u)) {
-    double a = 0.0;
-    for (int wv = 0; wv < 8; ++wv) a += red[threadIdx.x][wv];
-    atomicAdd(&sums[p * 4 + threadIdx.x], a);
-  }
+// ---------------------------------------------------------------------------------------------------------------
+// The regulariser stencil, shared by the sweep and the reg+Adam pass so that both compute the same bits.
+// (k.x, k.y, k.z, k.w) = coef[p, 0..3] of the terms selected by bit i of terms, 0 otherwise.
+__device__ __forceinline__ float4 reg_coef(const float* coef, int p, uint32_t terms) {
+  return make_float4((terms & 1u) ? coef[p * 4 + 0] : 0.f, (terms & 2u) ? coef[p * 4 + 1] : 0.f,
+                     (terms & 4u) ? coef[p * 4 + 2] : 0.f, (terms & 8u) ? coef[p * 4 + 3] : 0.f);
 }
 
-__global__ void __launch_bounds__(256) plane_reg_multi_bwd_kernel(const __grid_constant__ RegTable T,
-                                                                  const float* __restrict__ coef, int accumulate) {
-  const int p = find_tensor(T.first_block, T.n, blockIdx.x);
-  const RegPlane& P = T.pl[p];
-  const float* __restrict__ t = P.t;
-  const int H = P.H, W = P.W, C4 = P.C4;
-  const uint32_t terms = P.terms;
-  const float k0 = (terms & 1u) ? coef[p * 4 + 0] : 0.f, k1 = (terms & 2u) ? coef[p * 4 + 1] : 0.f;
-  const float k2 = (terms & 4u) ? coef[p * 4 + 2] : 0.f, k3 = (terms & 8u) ? coef[p * 4 + 3] : 0.f;
-  const int64_t total = (int64_t)H * W * C4, row = (int64_t)W * C4;
-  const int64_t base = (int64_t)(blockIdx.x - T.first_block[p]) * kChunk;
-  const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int it = 0; it < kChunk / 256; ++it) {
-    const int64_t idx = base + it * 256 + threadIdx.x;
-    if (idx >= total) break;
-    const int h = (int)(idx / row);
-    const int wcol = (int)(idx % row) / C4;
-    const float4 v = ldg4(t + idx * 4);
-    float4 g = zero, up1 = zero, up2 = zero, dn1 = zero, dn2 = zero;
-    if (k0 != 0.f || k2 != 0.f) {
-      if (h + 1 < H) up1 = ldg4(t + (idx + row) * 4);
-      if (h >= 1) dn1 = ldg4(t + (idx - row) * 4);
-    }
-    if (k0 != 0.f) {
-      if (h >= 1) g = fma4(sub4m(v, dn1), 2.f * k0, g);
-      if (h + 1 < H) g = fma4(sub4m(up1, v), -2.f * k0, g);
-    }
-    if (k1 != 0.f) {
-      if (wcol >= 1) g = fma4(sub4m(v, ldg4(t + (idx - C4) * 4)), 2.f * k1, g);
-      if (wcol + 1 < W) g = fma4(sub4m(ldg4(t + (idx + C4) * 4), v), -2.f * k1, g);
-    }
-    if (k2 != 0.f) {
-      if (h + 2 < H) up2 = ldg4(t + (idx + 2 * row) * 4);
-      if (h >= 2) dn2 = ldg4(t + (idx - 2 * row) * 4);
-      if (h >= 2) g = fma4(sub4m(sub4m(v, dn1), sub4m(dn1, dn2)), 2.f * k2, g);
-      if (h >= 1 && h + 1 < H) g = fma4(sub4m(sub4m(up1, v), sub4m(v, dn1)), -4.f * k2, g);
-      if (h + 2 < H) g = fma4(sub4m(sub4m(up2, up1), sub4m(up1, v)), 2.f * k2, g);
-    }
-    if (k3 != 0.f) {
-      g.x -= k3 * sgnm(1.f - v.x); g.y -= k3 * sgnm(1.f - v.y); g.z -= k3 * sgnm(1.f - v.z); g.w -= k3 * sgnm(1.f - v.w);
-    }
-    float4* gp = reinterpret_cast<float4*>(P.g + idx * 4);
-    if (accumulate) {
-      const float4 cur = *gp;
-      g.x += cur.x; g.y += cur.y; g.z += cur.z; g.w += cur.w;
-    }
-    *gp = g;
+// One float4 element c = row h of a channel-last plane with H rows.  a, b / d, e are rows h-2, h-1 / h+1, h+2 of the
+// same column (zero outside the plane); l() / r() return the W neighbours and are called only where has_l / has_r, so a
+// caller can read them where they live.  Adds to s the terms whose first element is c (only when cnt) and returns
+// sum_i k_i * d(sums[i]) / dc, sums[i] as in kp_plane_reg_fused (include/kplanes_b200.h).
+template <class L, class R>
+__device__ __forceinline__ float4 reg_stencil(uint32_t terms, const float4& k, int h, int H, bool has_l, bool has_r, bool cnt,
+                                              const float4& a, const float4& b, const float4& c, const float4& d,
+                                              const float4& e, const L& l, const R& r, float4& s) {
+  float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (terms & 1u) {  // squared first difference along H
+    if (h + 1 < H) { const float4 df = sub4m(d, c); if (cnt) s.x += sq4m(df); g = fma4(df, -2.f * k.x, g); }
+    if (h >= 1) g = fma4(sub4m(c, b), 2.f * k.x, g);
+  }
+  if (terms & 2u) {  // squared first difference along W
+    if (has_r) { const float4 df = sub4m(r(), c); if (cnt) s.y += sq4m(df); g = fma4(df, -2.f * k.y, g); }
+    if (has_l) g = fma4(sub4m(c, l()), 2.f * k.y, g);
+  }
+  if (terms & 4u) {  // squared second difference along H
+    if (h + 2 < H) { const float4 dd = sub4m(sub4m(e, d), sub4m(d, c)); if (cnt) s.z += sq4m(dd); g = fma4(dd, 2.f * k.z, g); }
+    if (h >= 1 && h + 1 < H) g = fma4(sub4m(sub4m(d, c), sub4m(c, b)), -4.f * k.z, g);
+    if (h >= 2) g = fma4(sub4m(sub4m(c, b), sub4m(b, a)), 2.f * k.z, g);
+  }
+  if (terms & 8u) {  // |1 - t|
+    if (cnt) s.w += fabsf(1.f - c.x) + fabsf(1.f - c.y) + fabsf(1.f - c.z) + fabsf(1.f - c.w);
+    g.x -= k.w * sgnm(1.f - c.x); g.y -= k.w * sgnm(1.f - c.y); g.z -= k.w * sgnm(1.f - c.z); g.w -= k.w * sgnm(1.f - c.w);
+  }
+  return g;
+}
+
+// Block reduction (256 threads) of the per-thread sums s: adds the block's totals of the selected terms to
+// plane_sums[0..3].  Called by every thread of the block.
+__device__ __forceinline__ void add_reg_sums(double* plane_sums, uint32_t terms, const float4& s) {
+  __shared__ double red[4][8];
+  const double dd[4] = {warp_sum_d((double)s.x), warp_sum_d((double)s.y), warp_sum_d((double)s.z), warp_sum_d((double)s.w)};
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (lane == 0)
+    for (int k = 0; k < 4; ++k) red[k][warp] = dd[k];
+  __syncthreads();
+  if (threadIdx.x < 4 && ((terms >> threadIdx.x) & 1u)) {
+    double acc = 0.0;
+    for (int wv = 0; wv < 8; ++wv) acc += red[threadIdx.x][wv];
+    atomicAdd(&plane_sums[threadIdx.x], acc);
   }
 }
 
@@ -131,31 +86,39 @@ __global__ void __launch_bounds__(256) plane_reg_multi_bwd_kernel(const __grid_c
 //   coef . d(sums)/d(plane) into the gradient bucket -- which also replaces the bucket's memset (the scatter kernels
 //   then add the data gradients on top).  Compared with memset + forward sweep + read-modify-write backward sweep this
 //   moves 2x instead of 5x the plane bytes.
-// Decomposition: a block owns 256 consecutive float4 columns of RROWS rows and walks down H keeping the rows
+// Decomposition: a block owns 256 consecutive float4 columns of kRegRows rows and walks down H keeping the rows
 // h-2 .. h+2 in registers (each element is loaded once per block + halo); the W neighbours come from L1.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kRegRows = 32;
-struct RegTile {
-  int first_block[kMaxTensors + 1];
-  int tiles_x[kMaxTensors];
+
+struct RegPlane {
+  const float* t;
+  float* g;
+  int H, W, C4;
+  uint32_t terms;
+};
+struct RegTable {
+  RegPlane pl[kMaxTensors];
+  int first_block[kMaxTensors + 1];  // first tile (block) of each plane
+  int tiles_x[kMaxTensors];          // tiles across a row of each plane
+  int n;
 };
 
 // write_range (optional, DEVICE int64 [P,2]): gradients are written only for float4 elements [begin, end) of plane p (the
 // sums always cover the whole plane) -- the data-parallel step with the sparse gradient exchange lets every rank write
 // the regularisers' gradient for ITS shard of the bucket only.
 template <bool ACCUMULATE>
-__global__ void __launch_bounds__(256) plane_reg_fused_kernel(const __grid_constant__ RegTable T, const __grid_constant__ RegTile G,
-                                                              const float* __restrict__ coef, double* __restrict__ sums,
-                                                              const long long* __restrict__ write_range, int sums_in_range) {
-  const int p = find_tensor(G.first_block, T.n, blockIdx.x);
+__global__ void __launch_bounds__(256) plane_reg_fused_kernel(const __grid_constant__ RegTable T, const float* __restrict__ coef,
+                                                              double* __restrict__ sums, const long long* __restrict__ write_range,
+                                                              int sums_in_range) {
+  const int p = find_tensor(T.first_block, T.n, blockIdx.x);
   const RegPlane& P = T.pl[p];
   const float* __restrict__ t = P.t;
   const int H = P.H, W = P.W, C4 = P.C4;
   const uint32_t terms = P.terms;
-  const float k0 = (terms & 1u) ? coef[p * 4 + 0] : 0.f, k1 = (terms & 2u) ? coef[p * 4 + 1] : 0.f;
-  const float k2 = (terms & 4u) ? coef[p * 4 + 2] : 0.f, k3 = (terms & 8u) ? coef[p * 4 + 3] : 0.f;
-  const int local = blockIdx.x - G.first_block[p];
-  const int tx = local % G.tiles_x[p], ty = local / G.tiles_x[p];
+  const float4 coef4 = coef != nullptr ? reg_coef(coef, p, terms) : make_float4(0.f, 0.f, 0.f, 0.f);  // NULL: sums only
+  const int local = blockIdx.x - T.first_block[p];
+  const int tx = local % T.tiles_x[p], ty = local / T.tiles_x[p];
   const int row4 = W * C4;                      // float4 elements per row
   const int col = tx * 256 + threadIdx.x;       // float4 column of this thread
   const bool active = col < row4;
@@ -171,7 +134,7 @@ __global__ void __launch_bounds__(256) plane_reg_fused_kernel(const __grid_const
     const long long hi = (long long)(h1 - 1) * row4 + min(row4, tx * 256 + 256) - 1;
     if (hi < wr0 || lo >= wr1) return;
   }
-  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+  float4 s = zero;
   if (active) {
     const float* base = t + (size_t)col * 4;
     const size_t rstride = (size_t)row4 * 4;
@@ -181,33 +144,14 @@ __global__ void __launch_bounds__(256) plane_reg_fused_kernel(const __grid_const
     // one row: c = row h, b / a = rows h-1 / h-2, d / e = rows h+1 / h+2, l / r = W neighbours of row h
     auto do_row = [&](int h, const float4& a, const float4& b, const float4& c, const float4& d, const float4& e, const float4& l,
                       const float4& r) {
-      float4 g = zero;
       const long long e4 = (long long)h * row4 + col;
       const bool in_range = write_range == nullptr || (e4 >= wr0 && e4 < wr1);
       const bool cnt = !shard_sums || in_range;  // shard mode: every term is counted by the rank that owns its element
-      if (terms & 1u) {  // squared first difference along H
-        if (h + 1 < H) { const float4 df = sub4m(d, c); if (cnt) s0 += sq4m(df); g = fma4(df, -2.f * k0, g); }
-        if (h >= 1) g = fma4(sub4m(c, b), 2.f * k0, g);
-      }
-      if (needW) {  // squared first difference along W
-        if (hasR) { const float4 df = sub4m(r, c); if (cnt) s1 += sq4m(df); g = fma4(df, -2.f * k1, g); }
-        if (hasL) g = fma4(sub4m(c, l), 2.f * k1, g);
-      }
-      if (need2) {  // squared second difference along H
-        if (h + 2 < H) { const float4 dd = sub4m(sub4m(e, d), sub4m(d, c)); if (cnt) s2 += sq4m(dd); g = fma4(dd, 2.f * k2, g); }
-        if (h >= 1 && h + 1 < H) g = fma4(sub4m(sub4m(d, c), sub4m(c, b)), -4.f * k2, g);
-        if (h >= 2) g = fma4(sub4m(sub4m(c, b), sub4m(b, a)), 2.f * k2, g);
-      }
-      if (terms & 8u) {  // |1 - t|
-        if (cnt) s3 += fabsf(1.f - c.x) + fabsf(1.f - c.y) + fabsf(1.f - c.z) + fabsf(1.f - c.w);
-        g.x -= k3 * sgnm(1.f - c.x); g.y -= k3 * sgnm(1.f - c.y); g.z -= k3 * sgnm(1.f - c.z); g.w -= k3 * sgnm(1.f - c.w);
-      }
-      if (gbase != nullptr) {
-        if (in_range) {
-          float4* gp = reinterpret_cast<float4*>(gbase + (size_t)h * rstride + (size_t)col * 4);
-          if (ACCUMULATE) { const float4 cur = *gp; g.x += cur.x; g.y += cur.y; g.z += cur.z; g.w += cur.w; }
-          *gp = g;
-        }
+      float4 g = reg_stencil(terms, coef4, h, H, hasL, hasR, cnt, a, b, c, d, e, [&] { return l; }, [&] { return r; }, s);
+      if (gbase != nullptr && in_range) {
+        float4* gp = reinterpret_cast<float4*>(gbase + (size_t)h * rstride + (size_t)col * 4);
+        if (ACCUMULATE) { const float4 cur = *gp; g.x += cur.x; g.y += cur.y; g.z += cur.z; g.w += cur.w; }
+        *gp = g;
       }
     };
     float4 a = need2 ? row_at(h0 - 2) : zero, b = row_at(h0 - 1), c = row_at(h0), d = row_at(h0 + 1);
@@ -230,19 +174,7 @@ __global__ void __launch_bounds__(256) plane_reg_fused_kernel(const __grid_const
       a = nr[0]; b = nr[1]; c = nr[2]; d = nr[3];
     }
   }
-  if (sums != nullptr) {
-    __shared__ double red[4][8];
-    const double dd[4] = {warp_sum_d((double)s0), warp_sum_d((double)s1), warp_sum_d((double)s2), warp_sum_d((double)s3)};
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (lane == 0)
-      for (int k = 0; k < 4; ++k) red[k][warp] = dd[k];
-    __syncthreads();
-    if (threadIdx.x < 4 && ((terms >> threadIdx.x) & 1u)) {
-      double acc = 0.0;
-      for (int wv = 0; wv < 8; ++wv) acc += red[threadIdx.x][wv];
-      atomicAdd(&sums[p * 4 + threadIdx.x], acc);
-    }
-  }
+  if (sums != nullptr) add_reg_sums(sums + p * 4, terms, s);
 }
 
 struct AdamTensor {
@@ -376,8 +308,7 @@ __global__ void __launch_bounds__(256, 3) plane_reg_adam_kernel(const __grid_con
   const RegAdamPlane& P = T.pl[p];
   const int H = P.H, W = P.W, C4 = P.C4, row4 = W * C4;
   const uint32_t terms = P.terms;
-  const float k0 = (terms & 1u) ? coef[p * 4 + 0] : 0.f, k1 = (terms & 2u) ? coef[p * 4 + 1] : 0.f;
-  const float k2 = (terms & 4u) ? coef[p * 4 + 2] : 0.f, k3 = (terms & 8u) ? coef[p * 4 + 3] : 0.f;
+  const float4 coef4 = reg_coef(coef, p, terms);
   const int local = blockIdx.x - T.first_block[p];
   const int tx = local % T.tiles_x[p], ty = local / T.tiles_x[p];
   const int tid = threadIdx.x;
@@ -404,7 +335,7 @@ __global__ void __launch_bounds__(256, 3) plane_reg_adam_kernel(const __grid_con
     return pp[(size_t)h * row4 + col];
   };
   auto halo_side = [&](int h, int side) -> float4 { return hl[kFHaloRows + ((h - h0) * 2 + side) * kFMaxC4 + kc]; };
-  float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+  float4 s = zero;
   float4 a = need2 ? old_row(h0 - 2) : zero, b = old_row(h0 - 1), c = old_row(h0), d = old_row(h0 + 1);
   float4 gn = zero, mn = zero, vn = zero, hLn = zero, hRn = zero;
   if (active) {
@@ -426,24 +357,10 @@ __global__ void __launch_bounds__(256, 3) plane_reg_adam_kernel(const __grid_con
     x[tid] = c;
     __syncthreads();  // every thread's pre-update row h is visible before any thread overwrites row h in global memory
     if (active) {
-      float4 g = zero;
-      if (terms & 1u) {  // squared first difference along H
-        if (h + 1 < H) { const float4 df = sub4m(d, c); s0 += sq4m(df); g = fma4(df, -2.f * k0, g); }
-        if (h >= 1) g = fma4(sub4m(c, b), 2.f * k0, g);
-      }
-      if (terms & 2u) {  // squared first difference along W
-        if (hasR) { const float4 r = edgeR ? hR : x[tid + C4]; const float4 df = sub4m(r, c); s1 += sq4m(df); g = fma4(df, -2.f * k1, g); }
-        if (hasL) { const float4 l = edgeL ? hL : x[tid - C4]; g = fma4(sub4m(c, l), 2.f * k1, g); }
-      }
-      if (need2) {  // squared second difference along H
-        if (h + 2 < H) { const float4 dd = sub4m(sub4m(e, d), sub4m(d, c)); s2 += sq4m(dd); g = fma4(dd, 2.f * k2, g); }
-        if (h >= 1 && h + 1 < H) g = fma4(sub4m(sub4m(d, c), sub4m(c, b)), -4.f * k2, g);
-        if (h >= 2) g = fma4(sub4m(sub4m(c, b), sub4m(b, a)), 2.f * k2, g);
-      }
-      if (terms & 8u) {  // |1 - t|
-        s3 += fabsf(1.f - c.x) + fabsf(1.f - c.y) + fabsf(1.f - c.z) + fabsf(1.f - c.w);
-        g.x -= k3 * sgnm(1.f - c.x); g.y -= k3 * sgnm(1.f - c.y); g.z -= k3 * sgnm(1.f - c.z); g.w -= k3 * sgnm(1.f - c.w);
-      }
+      // W neighbours: the exchanged row inside the tile, the halo snapshot at its edges (where x[tid -/+ C4] would fall
+      // outside the exchanged row)
+      const float4 g = reg_stencil(terms, coef4, h, H, hasL, hasR, true, a, b, c, d, e,
+                                   [&] { return edgeL ? hL : x[tid - C4]; }, [&] { return edgeR ? hR : x[tid + C4]; }, s);
       float4 pn = c, mm = mm0, vv = vv0;
       float* pa = &pn.x; const float* ga = &gg.x; const float* ra = &g.x; float* ma = &mm.x; float* va = &vv.x;
 #pragma unroll
@@ -460,19 +377,7 @@ __global__ void __launch_bounds__(256, 3) plane_reg_adam_kernel(const __grid_con
     }
     a = b; b = c; c = d; d = e;
   }
-  if (sums != nullptr) {
-    __shared__ double red[4][8];
-    const double dd[4] = {warp_sum_d((double)s0), warp_sum_d((double)s1), warp_sum_d((double)s2), warp_sum_d((double)s3)};
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (lane == 0)
-      for (int k = 0; k < 4; ++k) red[k][warp] = dd[k];
-    __syncthreads();
-    if (threadIdx.x < 4 && ((terms >> threadIdx.x) & 1u)) {
-      double acc = 0.0;
-      for (int wv = 0; wv < 8; ++wv) acc += red[threadIdx.x][wv];
-      atomicAdd(&sums[p * 4 + threadIdx.x], acc);
-    }
-  }
+  if (sums != nullptr) add_reg_sums(sums + p * 4, terms, s);
 }
 
 // Per-step scalars of a graph-replayed training step, from the device-resident step counter: the proposal-weight
@@ -501,8 +406,9 @@ __global__ void step_scalars_kernel(long long* __restrict__ step_counter, const 
   *step_counter = s + 1;
 }
 
+// Planes [begin, end) of the fused sweep; a plane with a gradient target needs the coefficient table.
 static int fill_reg_table(RegTable& T, const float* const* planes, float* const* grads, const int32_t* hwc,
-                          const uint32_t* terms, int begin, int end, bool need_grad) {
+                          const uint32_t* terms, int begin, int end, bool have_coef) {
   int nb = 0, k = 0;
   for (int i = begin; i < end; ++i, ++k) {
     RegPlane& r = T.pl[k];
@@ -511,12 +417,13 @@ static int fill_reg_table(RegTable& T, const float* const* planes, float* const*
     r.H = hwc[i * 3 + 0];
     r.W = hwc[i * 3 + 1];
     const int C = hwc[i * 3 + 2];
-    KP_CHECK(r.t != nullptr && r.H >= 1 && r.W >= 1 && C >= 4 && C % 4 == 0, "plane_reg_multi: plane %d invalid (C %% 4 != 0?)", i);
-    KP_CHECK(!need_grad || r.g != nullptr, "plane_reg_multi: grad pointer %d is NULL", i);
+    KP_CHECK(r.t != nullptr && r.H >= 1 && r.W >= 1 && C >= 4 && C % 4 == 0, "plane_reg_fused: plane %d invalid (C %% 4 != 0?)", i);
+    KP_CHECK(have_coef || r.g == nullptr, "plane_reg_fused: plane %d has a gradient target but coef_dev is NULL", i);
     r.C4 = C / 4;
     r.terms = terms[i];
     T.first_block[k] = nb;
-    nb += (int)ceil_div((int64_t)r.H * r.W * r.C4, kChunk);
+    T.tiles_x[k] = (int)ceil_div((int64_t)r.W * r.C4, 256);
+    nb += T.tiles_x[k] * (int)ceil_div(r.H, kRegRows);
   }
   T.first_block[k] = nb;
   T.n = k;
@@ -526,36 +433,6 @@ static int fill_reg_table(RegTable& T, const float* const* planes, float* const*
 }  // namespace kp
 
 using namespace kp;
-
-extern "C" int kp_plane_reg_multi_fwd(const float* const* planes, const int32_t* hwc, const uint32_t* terms, int P,
-                                      double* sums, void* stream) {
-  KP_CHECK(planes && hwc && terms && sums && P >= 0, "plane_reg_multi_fwd: bad arguments");
-  for (int begin = 0; begin < P; begin += kMaxTensors) {
-    const int end = std::min(P, begin + kMaxTensors);
-    RegTable T;
-    if (fill_reg_table(T, planes, nullptr, hwc, terms, begin, end, false)) return 1;
-    const int nb = T.first_block[T.n];
-    if (nb == 0) continue;
-    plane_reg_multi_fwd_kernel<<<nb, 256, 0, as_stream(stream)>>>(T, sums + (size_t)begin * 4);
-    KP_LAUNCH_CHECK("plane_reg_multi_fwd");
-  }
-  return 0;
-}
-
-extern "C" int kp_plane_reg_multi_bwd(const float* const* planes, float* const* grads, const int32_t* hwc,
-                                      const uint32_t* terms, int P, const float* coef_dev, int accumulate, void* stream) {
-  KP_CHECK(planes && grads && hwc && terms && coef_dev && P >= 0, "plane_reg_multi_bwd: bad arguments");
-  for (int begin = 0; begin < P; begin += kMaxTensors) {
-    const int end = std::min(P, begin + kMaxTensors);
-    RegTable T;
-    if (fill_reg_table(T, planes, grads, hwc, terms, begin, end, true)) return 1;
-    const int nb = T.first_block[T.n];
-    if (nb == 0) continue;
-    plane_reg_multi_bwd_kernel<<<nb, 256, 0, as_stream(stream)>>>(T, coef_dev + (size_t)begin * 4, accumulate);
-    KP_LAUNCH_CHECK("plane_reg_multi_bwd");
-  }
-  return 0;
-}
 
 extern "C" int kp_step_scalars(int64_t* step_counter, const double* lr_table, const float* anneal_table, int64_t max_steps,
                                int n_groups, const float* betas_host, float grad_scale, float* anneal_out,
@@ -601,24 +478,18 @@ extern "C" int kp_plane_reg_fused_shard(const float* const* planes, float* const
 static int plane_reg_fused_impl(const float* const* planes, float* const* grads, const int32_t* hwc, const uint32_t* terms, int P,
                                 const float* coef_dev, int accumulate, double* sums, const int64_t* write_range_dev,
                                 int sums_in_range, void* stream) {
-  KP_CHECK(planes && hwc && terms && coef_dev && P >= 0, "plane_reg_fused: bad arguments");
+  KP_CHECK(planes && hwc && terms && P >= 0, "plane_reg_fused: bad arguments");
   for (int begin = 0; begin < P; begin += kMaxTensors) {
     const int end = std::min(P, begin + kMaxTensors);
     RegTable T;
-    if (fill_reg_table(T, planes, grads, hwc, terms, begin, end, false)) return 1;
-    RegTile G;
-    int nb = 0;
-    for (int k = 0; k < T.n; ++k) {
-      G.first_block[k] = nb;
-      G.tiles_x[k] = (int)ceil_div((int64_t)T.pl[k].W * T.pl[k].C4, 256);
-      nb += G.tiles_x[k] * (int)ceil_div(T.pl[k].H, kRegRows);
-    }
-    G.first_block[T.n] = nb;
+    if (fill_reg_table(T, planes, grads, hwc, terms, begin, end, coef_dev != nullptr)) return 1;
+    const int nb = T.first_block[T.n];
     if (nb == 0) continue;
+    const float* cf = coef_dev ? coef_dev + (size_t)begin * 4 : nullptr;
     double* s = sums ? sums + (size_t)begin * 4 : nullptr;
     const long long* wr = write_range_dev ? reinterpret_cast<const long long*>(write_range_dev) + (size_t)begin * 2 : nullptr;
-    if (accumulate) plane_reg_fused_kernel<true><<<nb, 256, 0, as_stream(stream)>>>(T, G, coef_dev + (size_t)begin * 4, s, wr, sums_in_range);
-    else plane_reg_fused_kernel<false><<<nb, 256, 0, as_stream(stream)>>>(T, G, coef_dev + (size_t)begin * 4, s, wr, sums_in_range);
+    if (accumulate) plane_reg_fused_kernel<true><<<nb, 256, 0, as_stream(stream)>>>(T, cf, s, wr, sums_in_range);
+    else plane_reg_fused_kernel<false><<<nb, 256, 0, as_stream(stream)>>>(T, cf, s, wr, sums_in_range);
     KP_LAUNCH_CHECK("plane_reg_fused");
   }
   return 0;

@@ -256,29 +256,8 @@ def kplanes_regularizers(ms_grids_nerf, ms_grids_prop):
     the planes: identical values to ``space_tv_loss`` / ``time_smoothness_loss`` / ``sparse_transients_loss`` called on
     the field grids and on the proposal grids, but each plane is streamed once forward and once backward and receives
     a single gradient contribution.  Returns a dict keyed like the reference's loss dict."""
-    names = ["space_tv_loss", "time_smoothness_loss", "sparse_transients_loss",
-             "space_tv_proposal_loss", "time_smoothness_proposal_loss", "sparse_transients_proposal_loss"]
-    planes, terms, rows = [], [], []
-    for group, ms in enumerate((_flatten_grids(ms_grids_nerf), _flatten_grids(ms_grids_prop))):
-        for grids in ms:
-            dynamic = len(grids) == 6
-            spatial = [0, 1, 3] if dynamic else [0, 1, 2]
-            for gid, g in enumerate(grids):
-                _, c, h, w = g.shape
-                row = [[0.0] * 4 for _ in range(6)]
-                if gid in spatial:
-                    t = T_H | T_W
-                    row[3 * group + 0][0] = 1.0 / (c * (h - 1) * w)
-                    row[3 * group + 0][1] = 1.0 / (c * h * (w - 1))
-                else:
-                    t = T_W | T_SMOOTH | T_L1
-                    row[3 * group + 0][1] = 1.0 / (c * h * (w - 1))
-                    row[3 * group + 1][2] = 1.0 / (c * (h - 2) * w)
-                    row[3 * group + 2][3] = 1.0 / g.numel()
-                planes.append(g)
-                terms.append(t)
-                rows.append(row)
+    planes, terms, rows = regularizer_plan(ms_grids_nerf, ms_grids_prop)
     sums = ops.plane_reg_sums(planes, terms)  # [P,4]
     norm = _const(rows, sums.device)  # [P,6,4]
     vals = (sums[:, None, :] * norm).sum(dim=(0, 2))  # [6]
-    return {name: vals[i] for i, name in enumerate(names)}
+    return {name: vals[i] for i, name in enumerate(REG_NAMES)}

@@ -22,6 +22,7 @@ from ..field_components.spatial_distortions import SceneContraction
 from ..fields.base_field import FieldHeadNames
 from ..fields.kplanes_field import KPlanesDensityField, KPlanesField
 from ..model_components.losses import (
+    REG_NAMES,
     DepthLossType,
     MSELoss,
     depth_loss,
@@ -352,13 +353,11 @@ class KPlanesModel(Model):
         out: Dict[str, torch.Tensor] = {}
         ms_grids_nerf = self.field.grids
         ms_grids_prop = [p.grids for p in self.proposal_networks]
-        dynamic = len(self.config.spacetime_resolution) > 3 and not self.config.freeze_time_planes
-        reg_keys = ("space_tv_loss", "space_tv_proposal_loss", "sparse_transients_loss", "sparse_transients_proposal_loss",
-                    "time_smoothness_loss", "time_smoothness_proposal_loss")
-        if dynamic and all(k in loss_coef for k in reg_keys):
+        if self._all_six_regularizers():
             # the six regularisers of kplanes.py:430-446 from one pass over the planes (same values)
             out.update(kplanes_regularizers(ms_grids_nerf, ms_grids_prop))
             return out
+        dynamic = self._dynamic()
         if "space_tv_loss" in loss_coef:
             out["space_tv_loss"] = space_tv_loss(ms_grids_nerf)
         if "space_tv_proposal_loss" in loss_coef:
@@ -374,13 +373,16 @@ class KPlanesModel(Model):
                 out["time_smoothness_proposal_loss"] = time_smoothness_loss(ms_grids_prop)
         return out
 
+    def _dynamic(self) -> bool:
+        return len(self.config.spacetime_resolution) > 3 and not self.config.freeze_time_planes
+
+    def _all_six_regularizers(self) -> bool:
+        """Dynamic scene with all six regulariser keys: they are evaluated together, in one pass over the planes."""
+        return self._dynamic() and all(k in self.config.loss_coefficients for k in REG_NAMES)
+
     def fused_regularizers_applicable(self) -> bool:
         """Whether ``regularizers_into_grads`` covers this configuration (dynamic scene, all six regulariser keys)."""
-        loss_coef = self.config.loss_coefficients
-        dynamic = len(self.config.spacetime_resolution) > 3 and not self.config.freeze_time_planes
-        reg_keys = ("space_tv_loss", "space_tv_proposal_loss", "sparse_transients_loss", "sparse_transients_proposal_loss",
-                    "time_smoothness_loss", "time_smoothness_proposal_loss")
-        return dynamic and all(k in loss_coef for k in reg_keys) and not self.config.freeze_space_planes
+        return self._all_six_regularizers() and not self.config.freeze_space_planes
 
     def regularized_planes(self) -> List[Parameter]:
         return [p for g in self.field.grids for p in g] + [p for net in self.proposal_networks for p in net.grids]

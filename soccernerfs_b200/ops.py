@@ -1016,19 +1016,13 @@ def loss_head(pred: torch.Tensor, image: torch.Tensor, dist_per_ray: Optional[to
 
 class _PlaneReg(torch.autograd.Function):
     """sums[p] = (sum dh^2, sum dw^2, sum (d2h)^2, sum |1-t|) for each plane p, masked by terms[p].
-    One kernel launch for the whole plane list in each direction."""
+    The forward is one sums-only ``plane_reg_fused`` sweep; the backward one gradient-only sweep per target kind."""
 
     @staticmethod
     def forward(ctx, terms: Tuple[int, ...], *planes):
         ctx.sinks = [grad_sink(p) for p in planes]
-        planes = [as_channel_last(p.detach()) for p in planes]
-        for p in planes:
-            ptr_cl(p)
-        sums = torch.zeros((len(planes), 4), dtype=torch.float64, device=planes[0].device)
-        hwc, tm = _reg_tables(planes, terms)
-        call("kp_plane_reg_multi_fwd", _plane_ptrs(planes), hwc, tm, len(planes), ptr(sums), stream_ptr())
-        ctx.planes, ctx.terms = planes, terms
-        return sums.float()
+        ctx.planes, ctx.terms = [as_channel_last(p.detach()) for p in planes], terms
+        return plane_reg_fused(ctx.planes, terms, None, [None] * len(planes), accumulate=False).float()
 
     @staticmethod
     def backward(ctx, gsums):
@@ -1041,15 +1035,14 @@ class _PlaneReg(torch.autograd.Function):
             return (None,) * (1 + len(planes))
         g = f32c(gsums)
         grads = [None] * len(planes)
-        for accumulate in (1, 0):  # sunk planes: accumulate into the sink; others: write a fresh gradient tensor
-            sub = [i for i in idx if (ctx.sinks[i] is not None) == bool(accumulate)]
+        for accumulate in (True, False):  # sunk planes: accumulate into the sink; others: write a fresh gradient tensor
+            sub = [i for i in idx if (ctx.sinks[i] is not None) == accumulate]
             if not sub:
                 continue
-            sel = [planes[i] for i in sub]
             if accumulate:
                 tgt = [ctx.sinks[i] for i in sub]
             else:
-                flat = torch.empty(sum(p.numel() for p in sel), dtype=torch.float32, device=g.device)
+                flat = torch.empty(sum(planes[i].numel() for i in sub), dtype=torch.float32, device=g.device)
                 tgt, off = [], 0
                 for i in sub:
                     _, c, h, w = planes[i].shape
@@ -1057,35 +1050,34 @@ class _PlaneReg(torch.autograd.Function):
                     tgt.append(grads[i])
                     off += planes[i].numel()
             coef = g if len(sub) == len(planes) else g[sub].contiguous()
-            hwc, tm = _reg_tables(sel, [ctx.terms[i] for i in sub])
-            call("kp_plane_reg_multi_bwd", _plane_ptrs(sel), _plane_ptrs(tgt), hwc, tm, len(sel), ptr(coef), accumulate,
-                 stream_ptr())
+            plane_reg_fused([planes[i] for i in sub], [ctx.terms[i] for i in sub], coef, tgt, accumulate, want_sums=False)
         return (None, *grads)
 
 
-def plane_reg_fused(planes: Sequence[torch.Tensor], terms: Sequence[int], coef_dev: torch.Tensor,
+def plane_reg_fused(planes: Sequence[torch.Tensor], terms: Sequence[int], coef_dev: Optional[torch.Tensor],
                     targets: Sequence[Optional[torch.Tensor]], accumulate: bool, want_sums: bool = True,
                     write_range: Optional[torch.Tensor] = None, sums_in_range: bool = False) -> Optional[torch.Tensor]:
     """One sweep per plane: -> sums [P,4] (float64) of the regulariser terms, and targets[p] (channel-last gradient
-    buffers, entries may be None) = / += sum_i coef_dev[p,i] * d(sums[p,i])/d(plane).  No autograd: this is the training
-    step's form, where the gradient goes straight into the parameter's bucket (and, with accumulate=False, replaces the
-    bucket's memset)."""
+    buffers, entries may be None) = / += sum_i coef_dev[p,i] * d(sums[p,i])/d(plane).  ``coef_dev`` may be None when
+    every target is None.  No autograd: the training step's gradient goes straight into the parameter's bucket (and,
+    with accumulate=False, replaces the bucket's memset); ``plane_reg_sums`` wraps it for autograd."""
     planes = [as_channel_last(p.detach()) for p in planes]
     for p, t in zip(planes, targets):
         ptr_cl(p)
         if t is not None and (t.shape != p.shape or t.stride() != p.stride() or t.dtype != torch.float32):
             raise RuntimeError("plane_reg_fused: a gradient target must have the plane's channel-last layout")
     sums = torch.zeros((len(planes), 4), dtype=torch.float64, device=planes[0].device) if want_sums else None
+    coef = None if coef_dev is None else f32c(coef_dev)
     hwc, tm = _reg_tables(planes, terms)
     if write_range is not None:  # int64 [P,2] on the device: float4 element range of each plane whose gradient is written
         if write_range.dtype != torch.int64 or tuple(write_range.shape) != (len(planes), 2):
             raise RuntimeError("plane_reg_fused: write_range must be int64 [P,2]")
         # sums_in_range: the shard form -- sums restricted to the range too, tiles outside it skipped
         call("kp_plane_reg_fused_shard" if sums_in_range else "kp_plane_reg_fused_range", _plane_ptrs(planes),
-             _plane_ptrs(list(targets)), hwc, tm, len(planes), ptr(f32c(coef_dev)), int(accumulate), ptr(sums), ptr(write_range),
+             _plane_ptrs(list(targets)), hwc, tm, len(planes), ptr(coef), int(accumulate), ptr(sums), ptr(write_range),
              stream_ptr())
         return sums
-    call("kp_plane_reg_fused", _plane_ptrs(planes), _plane_ptrs(list(targets)), hwc, tm, len(planes), ptr(f32c(coef_dev)),
+    call("kp_plane_reg_fused", _plane_ptrs(planes), _plane_ptrs(list(targets)), hwc, tm, len(planes), ptr(coef),
          int(accumulate), ptr(sums), stream_ptr())
     return sums
 

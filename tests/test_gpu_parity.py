@@ -909,8 +909,9 @@ def test_cfg4_piecewise_single_jitter_samplers_vs_reference_fixture():
 
 
 def test_fused_regularizer_sweep_matches_autograd_path():
-    """kp_plane_reg_fused (one sweep: values + gradient written into the sinks) vs the two-sweep autograd path
-    (kp_plane_reg_multi_fwd/bwd): same six scaled loss values, same plane gradients; accumulate mode adds on top."""
+    """kp_plane_reg_fused in the training step's form (one sweep: values + gradient written into the sinks) vs the
+    autograd path (ops.plane_reg_sums: a sums-only sweep forward, gradient-only sweeps backward): same six scaled loss
+    values, same plane gradients; accumulate mode adds on top."""
     from soccernerfs_b200.distributed import GradBucket
     from soccernerfs_b200.models.kplanes import scale_dict
     from tests.helpers import build_model
@@ -935,6 +936,46 @@ def test_fused_regularizer_sweep_matches_autograd_path():
     model.regularizers_into_grads(accumulate=True)
     for p, r in zip(planes, ref_grads):
         assert rel_err(p.grad, 2 * r) < 1e-6
+
+
+def test_plane_reg_sums_and_gradients_vs_oracle_across_tiles():
+    """ops.plane_reg_sums and its autograd gradients against the torch formulas of the oracle (compute_plane_tv,
+    compute_plane_smoothness, |1 - t|) in float64, for every term combination the model uses.  The planes cross the
+    sweep's 32-row and 256-float4 tile edges (C = 8, 16 and 32); half of them carry a gradient sink, so the accumulating
+    and the writing backward sweeps both run in one backward."""
+    from soccernerfs_b200 import ops
+
+    torch.manual_seed(11)
+    T_H, T_W, T_SMOOTH, T_L1 = 1, 2, 4, 8
+    shapes = [(1, 32, 150, 70), (1, 32, 100, 64), (1, 8, 130, 200), (1, 8, 67, 128), (1, 32, 5, 3), (1, 16, 64, 64)]
+    base = [0.3 + 0.4 * torch.rand(sh) for sh in shapes]  # 1 - t keeps its sign: |1 - t| is differentiable everywhere
+
+    def oracle_sums(t):  # [4] float64: the four sums whose means the reference's losses take
+        _, c, h, w = t.shape
+        w_tv = ko.compute_plane_tv(t, only_w=True)
+        return torch.stack([(ko.compute_plane_tv(t) - w_tv) * (c * (h - 1) * w), w_tv * (c * h * (w - 1)),
+                            ko.compute_plane_smoothness(t) * (c * (h - 2) * w), torch.abs(1 - t).sum()])
+
+    for combo in (T_H | T_W, T_W, T_SMOOTH, T_L1, T_W | T_SMOOTH | T_L1):
+        mask = torch.tensor([(combo >> i) & 1 for i in range(4)], dtype=torch.float64)
+        weights = torch.rand(len(shapes), 4, dtype=torch.float64) * mask
+        planes = [ops.as_channel_last(b.to(DEV)).requires_grad_(True) for b in base]
+        for p in planes[::2]:
+            p._kp_grad_sink = torch.full_like(p, 0.25, memory_format=torch.preserve_format)
+            p.grad = p._kp_grad_sink
+        sums = ops.plane_reg_sums(planes, [combo] * len(planes))
+        (sums * weights.float().to(DEV)).sum().backward()
+        ref_planes = [b.double().requires_grad_(True) for b in base]
+        ref = torch.stack([oracle_sums(t) for t in ref_planes]) * mask
+        (ref * weights).sum().backward()
+        got = sums.detach().cpu().double()
+        for i in range(len(planes)):
+            for k in range(4):
+                assert rel_err(got[i, k], ref[i, k].detach()) < TOL, (combo, i, k)
+            grad = planes[i].grad - 0.25 if i % 2 == 0 else planes[i].grad
+            assert rel_err(grad.cpu(), ref_planes[i].grad) < TOL, (combo, i)
+        for p in planes[::2]:
+            del p._kp_grad_sink
 
 
 def test_plane_reg_adam_matches_regulariser_sweep_plus_adam():
