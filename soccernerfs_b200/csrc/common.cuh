@@ -109,6 +109,29 @@ __device__ __forceinline__ double warp_excl_scan_d(double v, int lane) {
   return lane == 0 ? 0.0 : up;
 }
 
+// Spherical-harmonics basis (degree 4, 16 terms) of a view direction, the first half of the colour net's input:
+// get_normalized_directions (kplanes_field.py:39-44) then tcnn SH maps [0,1] -> [-1,1]; basis NS/utils/math.py:25-86.
+__device__ __forceinline__ void sh16(float dx, float dy, float dz, float* out) {
+  const float x = ((dx + 1.f) / 2.f) * 2.f - 1.f, y = ((dy + 1.f) / 2.f) * 2.f - 1.f, z = ((dz + 1.f) / 2.f) * 2.f - 1.f;
+  const float xx = x * x, yy = y * y, zz = z * z;
+  out[0] = 0.28209479177387814f;
+  out[1] = 0.4886025119029199f * y;
+  out[2] = 0.4886025119029199f * z;
+  out[3] = 0.4886025119029199f * x;
+  out[4] = 1.0925484305920792f * x * y;
+  out[5] = 1.0925484305920792f * y * z;
+  out[6] = 0.9461746957575601f * zz - 0.31539156525251999f;
+  out[7] = 1.0925484305920792f * x * z;
+  out[8] = 0.5462742152960396f * (xx - yy);
+  out[9] = 0.5900435899266435f * y * (3.f * xx - yy);
+  out[10] = 2.890611442640554f * x * y * z;
+  out[11] = 0.4570457994644658f * y * (5.f * zz - 1.f);
+  out[12] = 0.3731763325901154f * z * (5.f * zz - 3.f);
+  out[13] = 0.4570457994644658f * x * (5.f * zz - 1.f);
+  out[14] = 1.445305721320277f * z * (xx - yy);
+  out[15] = 0.5900435899266435f * x * (xx - 3.f * yy);
+}
+
 // torch.nan_to_num defaults: nan -> 0, +inf -> FLT_MAX, -inf -> -FLT_MAX
 __device__ __forceinline__ float nan_to_num(float x) {
   if (isnan(x)) return 0.f;

@@ -67,26 +67,129 @@ __device__ __forceinline__ void issue_layer(uint32_t tmem_d, const float* a_hi, 
   }
 }
 
-__device__ __forceinline__ void sh16(float dx, float dy, float dz, float* out) {
-  // get_normalized_directions (kplanes_field.py:39-44) then tcnn SH maps [0,1] -> [-1,1]; basis NS/utils/math.py:25-86
-  const float x = ((dx + 1.f) / 2.f) * 2.f - 1.f, y = ((dy + 1.f) / 2.f) * 2.f - 1.f, z = ((dz + 1.f) / 2.f) * 2.f - 1.f;
-  const float xx = x * x, yy = y * y, zz = z * z;
-  out[0] = 0.28209479177387814f;
-  out[1] = 0.4886025119029199f * y;
-  out[2] = 0.4886025119029199f * z;
-  out[3] = 0.4886025119029199f * x;
-  out[4] = 1.0925484305920792f * x * y;
-  out[5] = 1.0925484305920792f * y * z;
-  out[6] = 0.9461746957575601f * zz - 0.31539156525251999f;
-  out[7] = 1.0925484305920792f * x * z;
-  out[8] = 0.5462742152960396f * (xx - yy);
-  out[9] = 0.5900435899266435f * y * (3.f * xx - yy);
-  out[10] = 2.890611442640554f * x * y * z;
-  out[11] = 0.4570457994644658f * y * (5.f * zz - 1.f);
-  out[12] = 0.3731763325901154f * z * (5.f * zz - 3.f);
-  out[13] = 0.4570457994644658f * x * (5.f * zz - 1.f);
-  out[14] = 1.445305721320277f * z * (xx - yy);
-  out[15] = 0.5900435899266435f * x * (xx - 3.f * yy);
+// Shared-memory carve-up of the colour net's weights (layers 3-5) and the 128 x 64 activation region, behind the sigma
+// net's weights in decoder_fwd_fused_kernel and alone in color_fwd_fused_kernel.  All regions are multiples of 1 KB.
+struct ColorSmem {
+  float *w3_hi, *w3_lo;    // [64 x 32]
+  float *w4_hi, *w4_lo;    // [64 x 64]
+  float *w5_hi, *w5_lo;    // [16 x 64] (3 valid rows)
+  float *act_hi, *act_lo;  // [128 x 64]
+};
+constexpr int kColorSmemFloats = 2 * 64 * 32 + 2 * 64 * 64 + 2 * 16 * 64 + 2 * 128 * 64;
+// the sigma net's weights in front of it in decoder_fwd_fused_kernel: w1 [64 x K0P] and w2 [16 x 64], hi + lo
+__host__ __device__ constexpr int sigma_smem_floats(int K0P) { return 2 * 64 * K0P + 2 * 16 * 64; }
+// dynamic shared memory of a fused kernel whose colour-net region starts `lead_floats` in (+ 1 KB for align1024)
+constexpr size_t fused_smem_bytes(int lead_floats) { return (size_t)(lead_floats + kColorSmemFloats) * sizeof(float) + 1024; }
+
+__device__ __forceinline__ ColorSmem color_smem(float* p) {
+  ColorSmem s;
+  s.w3_hi = p;
+  s.w3_lo = s.w3_hi + 64 * 32;
+  s.w4_hi = s.w3_lo + 64 * 32;
+  s.w4_lo = s.w4_hi + 64 * 64;
+  s.w5_hi = s.w4_lo + 64 * 64;
+  s.w5_lo = s.w5_hi + 16 * 64;
+  s.act_hi = s.w5_lo + 16 * 64;
+  s.act_lo = s.act_hi + 128 * 64;
+  return s;
+}
+
+// w3 [64 x kin] (colour-input width kin = 31 or 15), w4 [64 x 64], w5 [3 x 64]
+__device__ __forceinline__ void stage_color_weights(const float* w3, const float* w4, const float* w5, int kin, const ColorSmem& s) {
+  stage_weight<64, 32>(w3, kin, 64, kin, s.w3_hi, s.w3_lo);
+  stage_weight<64, 64>(w4, 64, 64, 64, s.w4_hi, s.w4_lo);
+  stage_weight<16, 64>(w5, 64, 3, 64, s.w5_hi, s.w5_lo);
+}
+
+// The colour input is [SH(16) | geo(15) | 0] (view dependent, cin width 32) or [geo(15) | 0 | zeros(16)] (cin width 16,
+// the zero half only in the activation region).  Warps 0-3 write the geometry half from x (x[15] = 0) ...
+__device__ __forceinline__ void store_geo_input(const float* x, int row, bool valid, int64_t grow, bool view_dep, float* cin,
+                                                const ColorSmem& s) {
+  store_act16(x, row, view_dep ? 16 : 0, s.act_hi, s.act_lo);
+  if (cin != nullptr && valid) {
+#pragma unroll
+    for (int q = 0; q < 4; ++q)
+      *reinterpret_cast<float4*>(cin + grow * (view_dep ? 32 : 16) + (view_dep ? 16 : 0) + 4 * q) =
+          make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
+  }
+}
+// ... and warps 4-7 the SH basis of the sample's ray direction, or the zero half (x is scratch)
+__device__ __forceinline__ void store_sh_input(float* x, int row, bool valid, int64_t grow, const float* dirs, int S, float* cin,
+                                               const ColorSmem& s) {
+  if (dirs != nullptr) {
+    const int64_t ray = valid ? grow / S : 0;
+    sh16(dirs[ray * 3 + 0], dirs[ray * 3 + 1], dirs[ray * 3 + 2], x);
+    store_act16(x, row, 0, s.act_hi, s.act_lo);
+    if (cin != nullptr && valid) {
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        *reinterpret_cast<float4*>(cin + grow * 32 + 4 * q) = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 16; ++j) x[j] = 0.f;
+    store_act16(x, row, 16, s.act_hi, s.act_lo);  // zero the unused half of the 32-wide colour input
+  }
+}
+
+// Layers 3-5 on the colour input written to the activation region by every thread: h2 = relu(cin W3^T),
+// h3 = relu(h2 W4^T), rgb = sigmoid(h3 W5^T); h2 / h3 go to global memory only when given (training).  Ends with the
+// fences after which the next tile's MMAs may reuse the TMEM accumulator.  Every thread of the CTA calls it.
+__device__ __forceinline__ void color_layers(const ColorSmem& s, const uint32_t& tmem_slot, uint64_t* mma_bar, uint32_t& parity,
+                                             int quad, int half, int row, bool valid, int64_t grow, float* h2, float* h3,
+                                             float* rgb) {
+  publish_smem_and_sync();
+  // ---- layer 3: h2 = relu(cin W3^T) ------------------------------------------------------------------------------
+  if (threadIdx.x == 0) {
+    issue_layer<4>(tmem_slot, s.act_hi, s.act_lo, s.w3_hi, s.w3_lo, 64, 64, false);
+    umma_commit(mma_bar);
+  }
+  mbar_wait(mma_bar, parity);
+  parity ^= 1;
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  const uint32_t tbase = tmem_slot + ((uint32_t)(quad * 32) << 16);
+  float x[32];
+  uint32_t v[16];
+#pragma unroll 1
+  for (int layer = 0; layer < 2; ++layer) {  // epilogue of h2 then of h3
+#pragma unroll
+    for (int part = 0; part < 2; ++part) {
+      tmem_ld16(tbase + (uint32_t)(half * 32 + part * 16), v);
+      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+      for (int j = 0; j < 16; ++j) x[part * 16 + j] = fmaxf(__uint_as_float(v[j]), 0.f);
+    }
+    store_act16(x, row, half * 32, s.act_hi, s.act_lo);
+    store_act16(x + 16, row, half * 32 + 16, s.act_hi, s.act_lo);
+    float* hbuf = layer == 0 ? h2 : h3;
+    if (hbuf != nullptr && valid) {
+#pragma unroll
+      for (int q = 0; q < 8; ++q)
+        *reinterpret_cast<float4*>(hbuf + grow * 64 + half * 32 + 4 * q) = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
+    }
+    publish_smem_and_sync();
+    if (threadIdx.x == 0) {
+      if (layer == 0) issue_layer<8>(tmem_slot, s.act_hi, s.act_lo, s.w4_hi, s.w4_lo, 64, 64, false);  // h3 = relu(h2 W4^T)
+      else issue_layer<8>(tmem_slot, s.act_hi, s.act_lo, s.w5_hi, s.w5_lo, 16, 16, false);             // rgb = sigmoid(h3 W5^T)
+      umma_commit(mma_bar);
+    }
+    mbar_wait(mma_bar, parity);
+    parity ^= 1;
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  }
+  // epilogue 5: rgb
+  if (half == 0) {
+    tmem_ld16(tbase, v);
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    if (valid) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) rgb[grow * 3 + c] = 1.f / (1.f + expf(-__uint_as_float(v[c])));
+    }
+  }
+  // TMEM reads of this tile complete before the next tile's MMAs reuse the accumulator
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 }
 
 struct DecoderArgs {
@@ -106,19 +209,11 @@ __global__ void __launch_bounds__(256, 1) decoder_fwd_fused_kernel(const __grid_
   float* w1_lo = w1_hi + 64 * K0P;
   float* w2_hi = w1_lo + 64 * K0P;  // [16 x 64]
   float* w2_lo = w2_hi + 16 * 64;
-  float* w3_hi = w2_lo + 16 * 64;   // [64 x 32]
-  float* w3_lo = w3_hi + 64 * 32;
-  float* w4_hi = w3_lo + 64 * 32;   // [64 x 64]
-  float* w4_lo = w4_hi + 64 * 64;
-  float* w5_hi = w4_lo + 64 * 64;   // [16 x 64] (3 valid rows)
-  float* w5_lo = w5_hi + 16 * 64;
-  float* act_hi = w5_lo + 16 * 64;  // [128 x 64]
-  float* act_lo = act_hi + 128 * 64;
+  const ColorSmem cs = color_smem(w1_hi + sigma_smem_floats(K0P));
   __shared__ __align__(8) uint64_t mma_bar;
   __shared__ uint32_t tmem_slot;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const bool view_dep = A.dirs != nullptr;
-  const int kin = view_dep ? 31 : 15;
 
   if (threadIdx.x == 0) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&mma_bar)));
@@ -127,9 +222,7 @@ __global__ void __launch_bounds__(256, 1) decoder_fwd_fused_kernel(const __grid_
   tmem_alloc(&tmem_slot, warp);
   stage_weight<64, K0P>(A.w1, A.K0, 64, A.K0, w1_hi, w1_lo);
   stage_weight<16, 64>(A.w2, 64, 16, 64, w2_hi, w2_lo);
-  stage_weight<64, 32>(A.w3, kin, 64, kin, w3_hi, w3_lo);
-  stage_weight<64, 64>(A.w4, 64, 64, 64, w4_hi, w4_lo);
-  stage_weight<16, 64>(A.w5, 64, 3, 64, w5_hi, w5_lo);
+  stage_color_weights(A.w3, A.w4, A.w5, view_dep ? 31 : 15, cs);
 
   const int quad = warp & 3, half = warp >> 2;
   const int row = quad * 32 + lane;
@@ -151,10 +244,10 @@ __global__ void __launch_bounds__(256, 1) decoder_fwd_fused_kernel(const __grid_
     // ---- layer 1: h1 = relu(X W1^T), X staged in 64-column halves through the activation region -------------
 #pragma unroll
     for (int hh = 0; hh < HALVES; ++hh) {
-      tile_store<0, 64>(pre[hh], act_hi, act_lo);
+      tile_store<0, 64>(pre[hh], cs.act_hi, cs.act_lo);
       publish_smem_and_sync();
       if (threadIdx.x == 0) {
-        issue_layer<8>(tmem_slot, act_hi, act_lo, w1_hi + hh * (2 * 64 * 32), w1_lo + hh * (2 * 64 * 32), 64, 64, hh != 0);
+        issue_layer<8>(tmem_slot, cs.act_hi, cs.act_lo, w1_hi + hh * (2 * 64 * 32), w1_lo + hh * (2 * 64 * 32), 64, 64, hh != 0);
         umma_commit(&mma_bar);
       }
       mbar_wait(&mma_bar, parity);
@@ -183,8 +276,8 @@ __global__ void __launch_bounds__(256, 1) decoder_fwd_fused_kernel(const __grid_
     }
     // all TMEM reads done before layer 2 overwrites the accumulator; all MMAs of layer 1 have completed (waited), so
     // the activation region is free to take h1
-    store_act16(x, row, half * 32, act_hi, act_lo);
-    store_act16(x + 16, row, half * 32 + 16, act_hi, act_lo);
+    store_act16(x, row, half * 32, cs.act_hi, cs.act_lo);
+    store_act16(x + 16, row, half * 32 + 16, cs.act_hi, cs.act_lo);
     if (A.h1 != nullptr && valid) {
 #pragma unroll
       for (int q = 0; q < 8; ++q)
@@ -193,14 +286,13 @@ __global__ void __launch_bounds__(256, 1) decoder_fwd_fused_kernel(const __grid_
     publish_smem_and_sync();
     // ---- layer 2: o = h1 W2^T (16 outputs: 15 geometry features + sigma_raw) --------------------------------------
     if (threadIdx.x == 0) {
-      issue_layer<8>(tmem_slot, act_hi, act_lo, w2_hi, w2_lo, 16, 16, false);
+      issue_layer<8>(tmem_slot, cs.act_hi, cs.act_lo, w2_hi, w2_lo, 16, 16, false);
       umma_commit(&mma_bar);
     }
     mbar_wait(&mma_bar, parity);
     parity ^= 1;
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     // epilogue 2: warps 0-3 unload o (and write geo into the colour input), warps 4-7 evaluate the SH basis
-    const int cin_w = view_dep ? 32 : 16;
     if (half == 0) {
       tmem_ld16(tbase, v);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
@@ -213,78 +305,11 @@ __global__ void __launch_bounds__(256, 1) decoder_fwd_fused_kernel(const __grid_
         A.density[grow] = expf(x[15]);  // trunc_exp forward (activations.py:31-33)
       }
       x[15] = 0.f;  // colour input = [.. | geo(15) | 0]
-      store_act16(x, row, view_dep ? 16 : 0, act_hi, act_lo);
-      if (A.cin != nullptr && valid) {
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          *reinterpret_cast<float4*>(A.cin + grow * cin_w + (view_dep ? 16 : 0) + 4 * q) =
-              make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
-      }
+      store_geo_input(x, row, valid, grow, view_dep, A.cin, cs);
     } else {
-      if (view_dep) {
-        const int64_t ray = valid ? grow / A.S : 0;
-        sh16(A.dirs[ray * 3 + 0], A.dirs[ray * 3 + 1], A.dirs[ray * 3 + 2], x);
-        store_act16(x, row, 0, act_hi, act_lo);
-        if (A.cin != nullptr && valid) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q)
-            *reinterpret_cast<float4*>(A.cin + grow * 32 + 4 * q) = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
-        }
-      } else {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) x[j] = 0.f;
-        store_act16(x, row, 16, act_hi, act_lo);  // zero the unused half of the 32-wide colour input
-      }
+      store_sh_input(x, row, valid, grow, A.dirs, A.S, A.cin, cs);
     }
-    publish_smem_and_sync();
-    // ---- layer 3: h2 = relu(cin W3^T) ------------------------------------------------------------------------------
-    if (threadIdx.x == 0) {
-      issue_layer<4>(tmem_slot, act_hi, act_lo, w3_hi, w3_lo, 64, 64, false);
-      umma_commit(&mma_bar);
-    }
-    mbar_wait(&mma_bar, parity);
-    parity ^= 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll 1
-    for (int layer = 0; layer < 2; ++layer) {  // epilogue of h2 then of h3
-#pragma unroll
-      for (int part = 0; part < 2; ++part) {
-        tmem_ld16(tbase + (uint32_t)(half * 32 + part * 16), v);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-        for (int j = 0; j < 16; ++j) x[part * 16 + j] = fmaxf(__uint_as_float(v[j]), 0.f);
-      }
-      store_act16(x, row, half * 32, act_hi, act_lo);
-      store_act16(x + 16, row, half * 32 + 16, act_hi, act_lo);
-      float* hbuf = layer == 0 ? A.h2 : A.h3;
-      if (hbuf != nullptr && valid) {
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          *reinterpret_cast<float4*>(hbuf + grow * 64 + half * 32 + 4 * q) = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
-      }
-      publish_smem_and_sync();
-      if (threadIdx.x == 0) {
-        if (layer == 0) issue_layer<8>(tmem_slot, act_hi, act_lo, w4_hi, w4_lo, 64, 64, false);  // h3 = relu(h2 W4^T)
-        else issue_layer<8>(tmem_slot, act_hi, act_lo, w5_hi, w5_lo, 16, 16, false);             // rgb = sigmoid(h3 W5^T)
-        umma_commit(&mma_bar);
-      }
-      mbar_wait(&mma_bar, parity);
-      parity ^= 1;
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    }
-    // epilogue 5: rgb
-    if (half == 0) {
-      tmem_ld16(tbase, v);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (valid) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) A.rgb[grow * 3 + c] = 1.f / (1.f + expf(-__uint_as_float(v[c])));
-      }
-    }
-    // TMEM reads of this tile complete before the next tile's MMAs reuse the accumulator
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    color_layers(cs, tmem_slot, &mma_bar, parity, quad, half, row, valid, grow, A.h2, A.h3, A.rgb);
   }
   tmem_free(tmem_slot, warp);
 }
@@ -307,114 +332,35 @@ struct ColorArgs {
 
 __global__ void __launch_bounds__(256, 1) color_fwd_fused_kernel(const __grid_constant__ ColorArgs A) {
   extern __shared__ uint8_t smem_raw[];
-  float* w3_hi = align1024(smem_raw);  // [64 x 32]
-  float* w3_lo = w3_hi + 64 * 32;
-  float* w4_hi = w3_lo + 64 * 32;      // [64 x 64]
-  float* w4_lo = w4_hi + 64 * 64;
-  float* w5_hi = w4_lo + 64 * 64;      // [16 x 64] (3 valid rows)
-  float* w5_lo = w5_hi + 16 * 64;
-  float* act_hi = w5_lo + 16 * 64;     // [128 x 64]
-  float* act_lo = act_hi + 128 * 64;
+  const ColorSmem cs = color_smem(align1024(smem_raw));
   __shared__ __align__(8) uint64_t mma_bar;
   __shared__ uint32_t tmem_slot;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const bool view_dep = A.dirs != nullptr;
-  const int kin = view_dep ? 31 : 15;
   if (threadIdx.x == 0) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&mma_bar)));
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   tmem_alloc(&tmem_slot, warp);
-  stage_weight<64, 32>(A.w3, kin, 64, kin, w3_hi, w3_lo);
-  stage_weight<64, 64>(A.w4, 64, 64, 64, w4_hi, w4_lo);
-  stage_weight<16, 64>(A.w5, 64, 3, 64, w5_hi, w5_lo);
+  stage_color_weights(A.w3, A.w4, A.w5, view_dep ? 31 : 15, cs);
   const int quad = warp & 3, half = warp >> 2;
   const int row = quad * 32 + lane;
   const int64_t n_tiles = (A.M + 127) / 128;
-  const int cin_w = view_dep ? 32 : 16;
   uint32_t parity = 0;
   for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const int64_t row0 = tile * 128;
     const int rows_valid = (int)min((int64_t)128, A.M - row0);
     const bool valid = row < rows_valid;
     const int64_t grow = row0 + row;
-    const uint32_t tbase = tmem_slot + ((uint32_t)(quad * 32) << 16);
-    float x[32];
-    uint32_t v[16];
-    // colour input = [SH(16) | geo(15) | 0] (view dependent) or [geo(15) | 0 | zeros(16)]: warps 0-3 bring the geometry
-    // features, warps 4-7 the SH basis (or the zero half)
+    float x[16];
     if (half == 0) {
 #pragma unroll
       for (int j = 0; j < 16; ++j) x[j] = (valid && j < 15) ? __ldg(A.o + grow * A.ldo + j) : 0.f;
-      store_act16(x, row, view_dep ? 16 : 0, act_hi, act_lo);
-      if (A.cin != nullptr && valid) {
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          *reinterpret_cast<float4*>(A.cin + grow * cin_w + (view_dep ? 16 : 0) + 4 * q) =
-              make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
-      }
+      store_geo_input(x, row, valid, grow, view_dep, A.cin, cs);
     } else {
-      if (view_dep) {
-        const int64_t ray = valid ? grow / A.S : 0;
-        sh16(A.dirs[ray * 3 + 0], A.dirs[ray * 3 + 1], A.dirs[ray * 3 + 2], x);
-        store_act16(x, row, 0, act_hi, act_lo);
-        if (A.cin != nullptr && valid) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q)
-            *reinterpret_cast<float4*>(A.cin + grow * 32 + 4 * q) = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
-        }
-      } else {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) x[j] = 0.f;
-        store_act16(x, row, 16, act_hi, act_lo);
-      }
+      store_sh_input(x, row, valid, grow, A.dirs, A.S, A.cin, cs);
     }
-    publish_smem_and_sync();
-    if (threadIdx.x == 0) {  // h2 = relu(cin W3^T)
-      issue_layer<4>(tmem_slot, act_hi, act_lo, w3_hi, w3_lo, 64, 64, false);
-      umma_commit(&mma_bar);
-    }
-    mbar_wait(&mma_bar, parity);
-    parity ^= 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll 1
-    for (int layer = 0; layer < 2; ++layer) {  // epilogue of h2 then of h3
-#pragma unroll
-      for (int part = 0; part < 2; ++part) {
-        tmem_ld16(tbase + (uint32_t)(half * 32 + part * 16), v);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-        for (int j = 0; j < 16; ++j) x[part * 16 + j] = fmaxf(__uint_as_float(v[j]), 0.f);
-      }
-      store_act16(x, row, half * 32, act_hi, act_lo);
-      store_act16(x + 16, row, half * 32 + 16, act_hi, act_lo);
-      float* hbuf = layer == 0 ? A.h2 : A.h3;
-      if (hbuf != nullptr && valid) {
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          *reinterpret_cast<float4*>(hbuf + grow * 64 + half * 32 + 4 * q) = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);
-      }
-      publish_smem_and_sync();
-      if (threadIdx.x == 0) {
-        if (layer == 0) issue_layer<8>(tmem_slot, act_hi, act_lo, w4_hi, w4_lo, 64, 64, false);  // h3 = relu(h2 W4^T)
-        else issue_layer<8>(tmem_slot, act_hi, act_lo, w5_hi, w5_lo, 16, 16, false);             // rgb = sigmoid(h3 W5^T)
-        umma_commit(&mma_bar);
-      }
-      mbar_wait(&mma_bar, parity);
-      parity ^= 1;
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    }
-    if (half == 0) {
-      tmem_ld16(tbase, v);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (valid) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) A.rgb[grow * 3 + c] = 1.f / (1.f + expf(-__uint_as_float(v[c])));
-      }
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    color_layers(cs, tmem_slot, &mma_bar, parity, quad, half, row, valid, grow, A.h2, A.h3, A.rgb);
   }
   tmem_free(tmem_slot, warp);
 }
@@ -445,11 +391,11 @@ extern "C" int kp_decoder_fwd_fused(const float* feats, int K0, const float* dir
   const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(M, 128), sms);
   cudaStream_t st = as_stream(stream);
   if (K0 <= 64) {
-    const size_t smem = (size_t)(2 * 64 * 64 + 2 * 16 * 64 + 2 * 64 * 32 + 2 * 64 * 64 + 2 * 16 * 64 + 2 * 128 * 64) * 4 + 1024;
+    const size_t smem = fused_smem_bytes(sigma_smem_floats(64));
     cudaFuncSetAttribute(decoder_fwd_fused_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     decoder_fwd_fused_kernel<64><<<grid, 256, smem, st>>>(a);
   } else {
-    const size_t smem = (size_t)(2 * 64 * 128 + 2 * 16 * 64 + 2 * 64 * 32 + 2 * 64 * 64 + 2 * 16 * 64 + 2 * 128 * 64) * 4 + 1024;
+    const size_t smem = fused_smem_bytes(sigma_smem_floats(128));
     cudaFuncSetAttribute(decoder_fwd_fused_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     decoder_fwd_fused_kernel<128><<<grid, 256, smem, st>>>(a);
   }
@@ -467,7 +413,7 @@ int kp_color_fwd_fused_launch(const float* directions, int S, const float* o, in
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(M, 128), sms);
-  const size_t smem = (size_t)(2 * 64 * 32 + 2 * 64 * 64 + 2 * 16 * 64 + 2 * 128 * 64) * 4 + 1024;
+  const size_t smem = fused_smem_bytes(0);
   cudaFuncSetAttribute(color_fwd_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   color_fwd_fused_kernel<<<grid, 256, smem, st>>>(a);
   kp::g_launches += 1;

@@ -12,9 +12,6 @@
 //     6*K [M,C] tensors, and scatter-adds with red.global.add.v4.f32 (16-byte L2 reductions).
 // Also here: the fused proposal density field (kplanes_field.py:434-460): gather (C=8) -> Hadamard ->
 // 8->64->1 MLP -> trunc_exp in one kernel, and its backward.
-#include <stdlib.h>
-#include <string.h>
-
 #include <algorithm>
 
 #include "common.cuh"
@@ -35,7 +32,6 @@ struct FieldRef {
   int n_scales, n_planes;
   uint32_t use_mask;
   int concat;
-  uint32_t agg_mask;  // scatter: bit k = merge equal texels of neighbouring samples of scale k inside the warp first
 };
 
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
@@ -102,31 +98,16 @@ static int fill_field(FieldRef& F, const float* const* plane_ptrs, float* const*
   F.n_planes = n_planes;
   F.use_mask = use_mask;
   F.concat = concat;
-  // Warp aggregation pays where consecutive samples of a ray share texels: the coarse scales.  A ray crosses at most
-  // ~R texels of an R^2 plane with S samples, so neighbours coincide often when R <= ~4 S; finer scales skip the
-  // extra shuffles.
-  F.agg_mask = 0;
-  const char* agg = getenv("KP_SCATTER_AGG");
-  for (int k = 0; k < n_scales; ++k) {
-    const int r = std::max(F.reso[k][0], std::max(F.reso[k][1], F.reso[k][2]));
-    // measured on B200 (gpurun_out r2_bench_agg_*: scatter 0.477 ms without, 0.511 ms with the coarse scales merged): the
-    // shuffle work costs more than the reds it removes, so merging is opt-in (KP_SCATTER_AGG=auto: coarse scales, =all)
-    bool on = false;
-    if (agg != nullptr && strcmp(agg, "auto") == 0) on = r <= 256;
-    if (agg != nullptr && strcmp(agg, "all") == 0) on = true;
-    if (on) F.agg_mask |= 1u << k;
-  }
   // L2 policy (ncu, 32x preset: the gather read 1.74 GB and the scatter moved 6.1 GB of DRAM for ~0.5 / ~1.4 GB of distinct
   // lines -- the once-per-step lines of the big space planes kept evicting the re-used coarse scales): planes of at least
-  // stream_bytes are streamed with evict_first.  KP_L2_STREAM_MB overrides the threshold (0 = never).
-  long long stream_bytes = 16ll << 20;  // (sweep on B200, 32x preset: off 1.35 ms, 96 MB 1.28, 32 MB 1.25, 16 MB 1.19, 4 MB 1.22 ms scatter)
-  if (getenv("KP_L2_STREAM_MB") != nullptr) stream_bytes = atoll(getenv("KP_L2_STREAM_MB")) << 20;
+  // stream_bytes are streamed with evict_first.
+  constexpr long long stream_bytes = 16ll << 20;  // (sweep on B200, 32x preset: off 1.35 ms, 96 MB 1.28, 32 MB 1.25, 16 MB 1.19, 4 MB 1.22 ms scatter)
   // only when the field as a whole is far beyond L2 (>= 512 MB): a 152 MB field keeps a 75 % L2 hit rate without any
   // policy, and streaming its largest scale costs more misses than it saves (ncu: gather DRAM reads 193 -> 269 MB)
   long long total_bytes = 0;
   for (int k = 0; k < n_scales; ++k)
     for (int p = 0; p < n_planes; ++p) total_bytes += (long long)F.pl[k * KP_MAX_PLANES + p].H * F.pl[k * KP_MAX_PLANES + p].W * feature_dim * 4;
-  if (stream_bytes > 0 && total_bytes >= (512ll << 20))
+  if (total_bytes >= (512ll << 20))
     for (int k = 0; k < n_scales; ++k)
       for (int p = 0; p < n_planes; ++p) {
         PlaneRef& r = F.pl[k * KP_MAX_PLANES + p];
@@ -381,47 +362,15 @@ __global__ void __launch_bounds__(128, 3) hexplane_fwd_wide_kernel(const __grid_
 // ---------------------------------------------------------------------------------------------------
 // Backward scatter: d plane_p[corner] += w_corner * g * prod_{q != p} interp_q.
 // ---------------------------------------------------------------------------------------------------
-// Warp-aggregated reduction: the 32 / LPS samples a warp owns are consecutive samples of a ray, so at the coarse scales
-// neighbouring samples often update the SAME texel corner.  Before the red, every run of neighbouring samples with an
-// equal texel index is summed with a segmented shuffle reduction (lane l talks to lanes l + LPS, l + 2 LPS, ... which
-// hold the same 16-byte channel slice of the next samples) and only the first sample of the run issues one red.v4 with
-// the run's total.  Runs are maximal CONTIGUOUS sequences of equal keys (from a ballot of the run heads), so any key
-// pattern is handled correctly -- non-adjacent duplicates are simply not merged.  `key` < 0 = nothing to add.
-// A warp-uniform test skips the value shuffles when no two neighbours coincide.
-template <int LPS>
-__device__ __forceinline__ void red_add_v4_aggregated(float* __restrict__ plane_grad, int key, float4 v, int lane) {
-  const unsigned full = 0xffffffffu;
-  const int prev = __shfl_up_sync(full, key, LPS);
-  const bool head = (lane < LPS) || (prev != key);
-  const unsigned heads = __ballot_sync(full, head);
-  if (heads != full) {  // some sample continues its neighbour's run
-    // first lane of the next run after my sample's lanes (32 if none): additions may only reach below it
-    const int my_end = (lane / LPS + 1) * LPS;
-    const unsigned later = my_end < 32 ? (heads >> my_end) : 0u;
-    const int run_end = later ? my_end + __ffs(later) - 1 : 32;
-#pragma unroll
-    for (int d = LPS; d < 32; d <<= 1) {
-      const float x = __shfl_down_sync(full, v.x, d), y = __shfl_down_sync(full, v.y, d);
-      const float z = __shfl_down_sync(full, v.z, d), w = __shfl_down_sync(full, v.w, d);
-      if (lane + d < run_end) { v.x += x; v.y += y; v.z += z; v.w += w; }
-    }
-  }
-  if (head && key >= 0) red_add_v4(plane_grad + (int64_t)key * (LPS * 4), v);
-}
-
 template <int C, int NP, bool STREAM>
 __global__ void __launch_bounds__(128, 4) hexplane_bwd_kernel(const __grid_constant__ FieldRef F,
                                                             const __grid_constant__ KpPoints P, int64_t M,
                                                             const float* __restrict__ grad_out) {
   constexpr int LPS = C / 4;
   const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t m_raw = gt / LPS;
+  const int64_t m = gt / LPS;
   const int c4 = (int)(gt % LPS) * 4;
-  const int lane = threadIdx.x & 31;
-  // lanes past the last sample stay alive (the aggregation shuffles are warp-wide) on a clamped sample, adding nothing
-  const bool live = m_raw < M;
-  if (__all_sync(0xffffffffu, !live)) return;
-  const int64_t m = live ? m_raw : M - 1;
+  if (m >= M) return;
   float pt[4];
   load_point(P, m, pt);
   const int out_stride = F.concat ? F.n_scales * C : C;
@@ -467,17 +416,12 @@ __global__ void __launch_bounds__(128, 4) hexplane_bwd_kernel(const __grid_const
       if (!((F.use_mask >> p) & 1u) || pr.g == nullptr) continue;
       const float4 gp = mul4(g, mul4(pre[p], suf[p]));
       float* gb = pr.g + c4;
-      if ((F.agg_mask >> k) & 1u) {  // (warp-uniform: F is a kernel parameter)
-        red_add_v4_aggregated<LPS>(gb, (live && b[p].w00 != 0.f) ? b[p].o00 : -1, scale4(gp, b[p].w00), lane);
-        red_add_v4_aggregated<LPS>(gb, (live && b[p].w01 != 0.f) ? b[p].o01 : -1, scale4(gp, b[p].w01), lane);
-        red_add_v4_aggregated<LPS>(gb, (live && b[p].w10 != 0.f) ? b[p].o10 : -1, scale4(gp, b[p].w10), lane);
-        red_add_v4_aggregated<LPS>(gb, (live && b[p].w11 != 0.f) ? b[p].o11 : -1, scale4(gp, b[p].w11), lane);
-      } else if (STREAM && live && pr.stream) {
+      if (STREAM && pr.stream) {
         if (b[p].w00 != 0.f) red_add_v4_stream(gb + (int64_t)b[p].o00 * C, scale4(gp, b[p].w00), pol);
         if (b[p].w01 != 0.f) red_add_v4_stream(gb + (int64_t)b[p].o01 * C, scale4(gp, b[p].w01), pol);
         if (b[p].w10 != 0.f) red_add_v4_stream(gb + (int64_t)b[p].o10 * C, scale4(gp, b[p].w10), pol);
         if (b[p].w11 != 0.f) red_add_v4_stream(gb + (int64_t)b[p].o11 * C, scale4(gp, b[p].w11), pol);
-      } else if (live) {
+      } else {
         if (b[p].w00 != 0.f) red_add_v4(gb + (int64_t)b[p].o00 * C, scale4(gp, b[p].w00));
         if (b[p].w01 != 0.f) red_add_v4(gb + (int64_t)b[p].o01 * C, scale4(gp, b[p].w01));
         if (b[p].w10 != 0.f) red_add_v4(gb + (int64_t)b[p].o10 * C, scale4(gp, b[p].w10));
@@ -485,7 +429,7 @@ __global__ void __launch_bounds__(128, 4) hexplane_bwd_kernel(const __grid_const
       }
       // sparse gradient exchange: mark the texels this sample reduced into (one lane of the sample's C/4; plain byte
       // stores of the same value, so no ordering between writers is needed)
-      if (pr.f != nullptr && live && c4 == 0) {
+      if (pr.f != nullptr && c4 == 0) {
         if (b[p].w00 != 0.f) pr.f[b[p].o00] = 1;
         if (b[p].w01 != 0.f) pr.f[b[p].o01] = 1;
         if (b[p].w10 != 0.f) pr.f[b[p].o10] = 1;
@@ -818,11 +762,9 @@ static int launch_hexplane(bool bwd, const FieldRef& F, const KpPoints& P, int64
     // wide mapping (4 lanes x 8 channels per sample).  Measured on B200 (gpurun_out/s3k_bench*): L2-resident field (cfg2
     // training) 0.165 -> 0.150 ms; coherent rays of full-frame inference 361.9 -> 352.3 ms per frame; HBM-resident field with
     // random rays (cfg3 training) 0.359 -> 0.405 ms -- there the float4 kernel keeps more requests in flight.  Hence: wide
-    // unless the field streams from HBM (any_stream) with incoherent rays.  KP_GATHER_WIDE=0/1 overrides.  Needs 32-byte
-    // aligned planes and output rows.
-    static const int wide_env = getenv("KP_GATHER_WIDE") != nullptr ? atoi(getenv("KP_GATHER_WIDE")) : -1;
+    // unless the field streams from HBM (any_stream) with incoherent rays.  Needs 32-byte aligned planes and output rows.
     const bool coherent = P.ray_tile > 1 && P.pts == nullptr;
-    bool wide = !bwd && (wide_env == 1 || (wide_env != 0 && (coherent || !any_stream))) && P.ray_tile >= 0;  // (< 0: float4 kernel, tests)
+    bool wide = !bwd && (coherent || !any_stream) && P.ray_tile >= 0;  // (< 0: float4 kernel, tests)
     wide = wide && (reinterpret_cast<uintptr_t>(out) & 31) == 0;
     for (int k = 0; k < F.n_scales && wide; ++k)
       for (int p = 0; p < F.n_planes; ++p) wide = wide && (reinterpret_cast<uintptr_t>(F.pl[k * KP_MAX_PLANES + p].p) & 31) == 0;

@@ -6,8 +6,6 @@
 // staged reduction-major so both micro-tile operands are 16-byte LDS) instantiated for the three products a
 // dense layer needs -- Y = X W^T, dX = dY W, dW += dY^T X (split over the M reduction, atomically
 // accumulated) -- with the activations / masks fused in the epilogues.
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "common.cuh"
@@ -175,28 +173,11 @@ __global__ void color_input_kernel(const float* __restrict__ dirs, int S, const 
     return;
   }
   const int64_t n = m / S;
-  // get_normalized_directions (kplanes_field.py:39-44) then tcnn SH maps [0,1] -> [-1,1]
-  const float x = ((dirs[n * 3 + 0] + 1.f) / 2.f) * 2.f - 1.f;
-  const float y = ((dirs[n * 3 + 1] + 1.f) / 2.f) * 2.f - 1.f;
-  const float z = ((dirs[n * 3 + 2] + 1.f) / 2.f) * 2.f - 1.f;
-  const float xx = x * x, yy = y * y, zz = z * z;
   float* dst = cin + m * 32;
-  dst[0] = 0.28209479177387814f;
-  dst[1] = 0.4886025119029199f * y;
-  dst[2] = 0.4886025119029199f * z;
-  dst[3] = 0.4886025119029199f * x;
-  dst[4] = 1.0925484305920792f * x * y;
-  dst[5] = 1.0925484305920792f * y * z;
-  dst[6] = 0.9461746957575601f * zz - 0.31539156525251999f;
-  dst[7] = 1.0925484305920792f * x * z;
-  dst[8] = 0.5462742152960396f * (xx - yy);
-  dst[9] = 0.5900435899266435f * y * (3.f * xx - yy);
-  dst[10] = 2.890611442640554f * x * y * z;
-  dst[11] = 0.4570457994644658f * y * (5.f * zz - 1.f);
-  dst[12] = 0.3731763325901154f * z * (5.f * zz - 3.f);
-  dst[13] = 0.4570457994644658f * x * (5.f * zz - 1.f);
-  dst[14] = 1.445305721320277f * z * (xx - yy);
-  dst[15] = 0.5900435899266435f * x * (xx - 3.f * yy);
+  float sh[16];
+  sh16(dirs[n * 3 + 0], dirs[n * 3 + 1], dirs[n * 3 + 2], sh);
+#pragma unroll
+  for (int c = 0; c < 16; ++c) dst[c] = sh[c];
 #pragma unroll
   for (int c = 0; c < 15; ++c) dst[16 + c] = geo[c];
   dst[31] = 0.f;
@@ -219,23 +200,21 @@ __global__ void sigmoid_grad_kernel(const float* __restrict__ rgb, const float* 
 
 
 // ---------------------------------------------------------------------------------------------------------------
-// Backward of a NARROW output layer (sigma net: 16 outputs, colour net: 3) in plain fp32 SIMT, one pass:
-//   dOut[M,NO] is formed on the fly from the upstream gradients (never written),
+// Backward of the colour net's output layer (rgb = sigmoid(h3 W5^T), 3 outputs) in plain fp32 SIMT, one pass:
+//   dOut[M,3] = grad_rgb * rgb * (1 - rgb) is formed on the fly (never written),
 //   dH[M,K] = (dOut . W) * (H > 0)            (the hidden layer's ReLU mask)
-//   dW[NO,K] += dOut^T . H
-// With NO <= 16 the two products are 8*NO FMAs per 16 bytes of H: far below the memory time of streaming H in and dH
+//   dW[3,K] += dOut^T . H
+// With 3 outputs the two products are 24 FMAs per 16 bytes of H: far below the memory time of streaming H in and dH
 // out, so the tensor-core route (two GEMM launches that each stream H again, plus a kernel that materialises dOut)
-// only added launches and passes over memory.  K/4 lanes own one row (coalesced 16-byte accesses); every lane keeps its
+// only adds launches and passes over memory.  K/4 lanes own one row (coalesced 16-byte accesses); every lane keeps its
 // four columns of W and of the dW accumulator in registers; block-level reduction of dW in shared memory, one red per
 // weight per block.
-//   MODE 0: dOut[:, 0:15] = grad_geo (or 0), dOut[:,15] += grad_density * exp(clamp(o[:,15], -15, 15))   (_TruncExp backward)
-//   MODE 1: dOut[:, j] = grad_rgb * rgb * (1 - rgb)                                                       (sigmoid backward)
 // ---------------------------------------------------------------------------------------------------------------
-template <int NO, int K, int MODE>
+template <int K>
 __global__ void __launch_bounds__(128) narrow_layer_bwd_kernel(const float* __restrict__ H, float* __restrict__ dH,
                                                                const float* __restrict__ W, float* __restrict__ dW, int64_t M,
-                                                               const float* __restrict__ a0, const float* __restrict__ a1,
-                                                               const float* __restrict__ a2) {
+                                                               const float* __restrict__ rgb, const float* __restrict__ grad_rgb) {
+  constexpr int NO = 3;
   constexpr int LPR = K / 4;      // lanes per row
   constexpr int RPW = 32 / LPR;   // rows per warp pass
   static_assert(LPR == 16 || LPR == 32, "K must be 64 or 128");
@@ -252,7 +231,7 @@ __global__ void __launch_bounds__(128) narrow_layer_bwd_kernel(const float* __re
   }
   const int64_t warps_total = (int64_t)gridDim.x * (blockDim.x >> 5);
   const int64_t gw = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
-  constexpr int U = NO <= 4 ? 4 : 1;  // rows in flight per lane: all loads of U rows are issued before the arithmetic
+  constexpr int U = 4;  // rows in flight per lane: all loads of U rows are issued before the arithmetic
   for (int64_t base = gw * RPW * U; base < M; base += warps_total * RPW * U) {
     float d[U][NO];
     float4 h[U];
@@ -263,19 +242,10 @@ __global__ void __launch_bounds__(128) narrow_layer_bwd_kernel(const float* __re
 #pragma unroll
       for (int j = 0; j < NO; ++j) d[u][j] = 0.f;
       if (s < M) {
-        if (MODE == 0) {
 #pragma unroll
-          for (int j4 = 0; j4 < NO / 4; ++j4) {
-            const float4 g = a2 != nullptr ? ldg4(a2 + s * NO + 4 * j4) : make_float4(0.f, 0.f, 0.f, 0.f);
-            d[u][4 * j4] = g.x; d[u][4 * j4 + 1] = g.y; d[u][4 * j4 + 2] = g.z; d[u][4 * j4 + 3] = g.w;
-          }
-          if (a1 != nullptr) d[u][NO - 1] += __ldg(a1 + s) * expf(fminf(fmaxf(__ldg(a0 + s * NO + NO - 1), -15.f), 15.f));
-        } else {
-#pragma unroll
-          for (int j = 0; j < NO; ++j) {
-            const float sg = __ldg(a0 + s * NO + j);
-            d[u][j] = __ldg(a1 + s * NO + j) * sg * (1.f - sg);
-          }
+        for (int j = 0; j < NO; ++j) {
+          const float sg = __ldg(rgb + s * NO + j);
+          d[u][j] = __ldg(grad_rgb + s * NO + j) * sg * (1.f - sg);
         }
         h[u] = ldg4(H + s * K + 4 * q);
       }
@@ -308,19 +278,18 @@ __global__ void __launch_bounds__(128) narrow_layer_bwd_kernel(const float* __re
   for (int i = threadIdx.x; i < NO * K; i += blockDim.x) red_add_f32(dW + i, s_acc[i]);
 }
 
-template <int NO, int MODE>
-static bool launch_narrow_bwd(int K, const float* H, float* dH, const float* W, float* dW, int64_t M, const float* a0,
-                              const float* a1, const float* a2, cudaStream_t st) {
-  if (getenv("KP_NARROW_BWD") != nullptr && atoi(getenv("KP_NARROW_BWD")) == 0) return false;
+// false when the shape or the alignment does not fit narrow_layer_bwd_kernel (the caller then takes the GEMM route)
+static bool launch_narrow_bwd(int K, const float* H, float* dH, const float* W, float* dW, int64_t M, const float* rgb,
+                              const float* grad_rgb, cudaStream_t st) {
   if (K != 64 && K != 128) return false;
-  if ((((uintptr_t)H | (uintptr_t)dH | (uintptr_t)W) & 15) != 0 || (a2 != nullptr && ((uintptr_t)a2 & 15) != 0)) return false;
+  if ((((uintptr_t)H | (uintptr_t)dH | (uintptr_t)W) & 15) != 0) return false;
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int rpw = 32 / (K / 4);
   const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(M, 4 * rpw), (int64_t)sms * 4));
-  if (K == 64) narrow_layer_bwd_kernel<NO, 64, MODE><<<grid, 128, 0, st>>>(H, dH, W, dW, M, a0, a1, a2);
-  else narrow_layer_bwd_kernel<NO, 128, MODE><<<grid, 128, 0, st>>>(H, dH, W, dW, M, a0, a1, a2);
+  if (K == 64) narrow_layer_bwd_kernel<64><<<grid, 128, 0, st>>>(H, dH, W, dW, M, rgb, grad_rgb);
+  else narrow_layer_bwd_kernel<128><<<grid, 128, 0, st>>>(H, dH, W, dW, M, rgb, grad_rgb);
   kp::g_launches += 1;
   return true;
 }
@@ -348,19 +317,13 @@ extern "C" int kp_sigma_net_bwd(const float* feats, const float* w1, const float
   if (M == 0) return 0;
   KP_CHECK(feats && w1 && w2 && h1 && o && grad_w1 && grad_w2 && scratch, "sigma_net_bwd: bad arguments");
   cudaStream_t st = as_stream(stream);
-  // d_o lives in the first [M,16] floats of a dedicated region at the end of scratch? No: scratch is [M,H] with
-  // H >= 16, and d_o is consumed (dW2, d_h1) before d_h1 overwrites scratch -- so d_o needs its own storage.
-  // We therefore keep d_o in grad_feats' first M*16 floats (K >= 16), which is only written by the last GEMM.
+  // d_o = dL/do [M,16] cannot share scratch [M,H], which receives d_h1 while d_o is read; it is kept in grad_feats' first
+  // M*16 floats (K >= 16), which only the last GEMM writes.
   KP_CHECK(K >= 16 && grad_feats != nullptr, "sigma_net_bwd: needs grad_feats with K >= 16");
-  // (the 16-output version of the narrow SIMT kernel needs 64 dW accumulator registers per lane and measured slower than
-  //  the tensor-core route: 0.221 vs 0.158 ms for the whole sigma backward at cfg2 -- opt-in with KP_NARROW_BWD=2)
-  const bool narrow16 = getenv("KP_NARROW_BWD") != nullptr && atoi(getenv("KP_NARROW_BWD")) == 2;
-  if (!narrow16 || !launch_narrow_bwd<16, 0>(H, h1, scratch, w2, grad_w2, M, o, grad_density, grad_geo, st)) {
-    float* d_o = grad_feats;
-    sigma_dout_kernel<<<(unsigned)ceil_div(M * 16, 256), 256, 0, st>>>(o, grad_density, grad_geo, M, d_o);
-    gemm_dw(d_o, 16, h1, H, grad_w2, H, M, 16, H, st);
-    gemm_dx<EPI_RELU_MASK>(d_o, 16, w2, H, scratch, H, M, 16, H, h1, H, st);   // d_h1
-  }
+  float* d_o = grad_feats;
+  sigma_dout_kernel<<<(unsigned)ceil_div(M * 16, 256), 256, 0, st>>>(o, grad_density, grad_geo, M, d_o);
+  gemm_dw(d_o, 16, h1, H, grad_w2, H, M, 16, H, st);
+  gemm_dx<EPI_RELU_MASK>(d_o, 16, w2, H, scratch, H, M, 16, H, h1, H, st);   // d_h1
   gemm_dw(scratch, H, feats, K, grad_w1, K, M, H, K, st);
   gemm_dx<EPI_NONE>(scratch, H, w1, K, grad_feats, K, M, H, K, nullptr, 0, st);
   KP_LAUNCH_CHECK("sigma_net_bwd");
@@ -375,7 +338,7 @@ extern "C" int kp_color_net_fwd(const float* directions, int S, const float* o, 
   KP_CHECK(o && w3 && w4 && w5 && cin && h2 && h3 && rgb && H2 >= 1 && ldgeo >= 15, "color_net_fwd: bad arguments");
   KP_CHECK(directions == nullptr || (S >= 1 && M % S == 0), "color_net_fwd: M must be a multiple of S");
   cudaStream_t st = as_stream(stream);
-  if (H2 == 64 && !(getenv("KP_COLOR_FUSED") != nullptr && atoi(getenv("KP_COLOR_FUSED")) == 0)) {
+  if (H2 == 64) {
     // the whole colour net in one tcgen05 launch (decoder_fused.cu): weights resident, activations chained on chip
     kp_color_fwd_fused_launch(directions, S, o, ldgeo, w3, w4, w5, M, cin, h2, h3, rgb, st);
     KP_LAUNCH_CHECK("color_net_fwd");
@@ -401,7 +364,7 @@ extern "C" int kp_color_net_bwd(int view_dependent, const float* cin, const floa
            "color_net_bwd: bad arguments");
   cudaStream_t st = as_stream(stream);
   const int ldc = view_dependent ? 32 : 16, kin = view_dependent ? 31 : 15, geo_off = view_dependent ? 16 : 0;
-  if (!launch_narrow_bwd<3, 1>(H2, h3, scratch_a, w5, grad_w5, M, rgb, grad_rgb, nullptr, st)) {  // d_h3 -> a, dW5, one pass
+  if (!launch_narrow_bwd(H2, h3, scratch_a, w5, grad_w5, M, rgb, grad_rgb, st)) {  // d_h3 -> a, dW5, one pass
     float* dpre = scratch_b;  // [M,4]
     sigmoid_grad_kernel<<<(unsigned)ceil_div(M * 4, 256), 256, 0, st>>>(rgb, grad_rgb, M, dpre);
     gemm_dw(dpre, 4, h3, H2, grad_w5, H2, M, 3, H2, st);

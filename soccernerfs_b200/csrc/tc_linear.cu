@@ -23,7 +23,6 @@
 // For 32-bit operands the tensor core only accepts the 32-byte-base swizzle in the MN-major view (atoms of 4 rows x
 // 128 bytes, 32-byte chunk q of row r at chunk q ^ (r & 3)), so a tile is staged in the swizzle of the view it is
 // consumed in.
-#include <stdlib.h>
 #include <string.h>
 
 #include "tc_common.cuh"
@@ -596,10 +595,7 @@ static unsigned persistent_grid(Kern kern, int64_t n_tiles, size_t smem) {
     per_sm = std::min<int>(65536 / std::max(1, regs_cta), (int)((size_t)smem_sm / smem_cta));
   }
   if (per_sm < 1) per_sm = 1;
-  if (getenv("KP_TC_MAX_CTAS") != nullptr) per_sm = std::min(per_sm, atoi(getenv("KP_TC_MAX_CTAS")));
   if (per_sm > 4) per_sm = 4;  // 4 x 128 TMEM columns
-  if (getenv("KP_TC_DEBUG") != nullptr)
-    fprintf(stderr, "[kp tc] smem=%zu B -> %d CTA/SM, grid %lld\n", smem, per_sm, (long long)std::min<int64_t>(n_tiles, (int64_t)sms * per_sm));
   return (unsigned)std::min<int64_t>(n_tiles, (int64_t)sms * per_sm);
 }
 
@@ -669,13 +665,10 @@ static bool launch_ws(const float* A, int64_t lda, const float* W, int64_t ldw, 
   const int64_t n_tiles = ceil_div(M, 128);
   const unsigned gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>(n_tiles, (int64_t)sms / gy));
   const dim3 grid(gx, gy);
-  if (getenv("KP_TC_DEBUG") != nullptr)
-    fprintf(stderr, "[kp tc ws] B_MN=%d R=%d N=%d: KS=%d slices=%d N_slice=%d stages=%d smem=%zu grid=(%u,%u)\n", B_MN, R, N_total, KS,
-            n_slices, N_slice, n_stages, smem, gx, gy);
   const bool mask = aux != nullptr;
   // activation tiles through the TMA engine when the matrix can be described by a tensor map (16-byte aligned rows)
   CUtensorMap tmA;
-  const bool use_tma = !(getenv("KP_TC_TMA") != nullptr && atoi(getenv("KP_TC_TMA")) == 0) && make_tmap_2d(&tmA, A, M, R, lda, 128, false);
+  const bool use_tma = make_tmap_2d(&tmA, A, M, R, lda, 128, false);
   const CUtensorMap* tm = use_tma ? &tmA : nullptr;
   if (B_MN) {
     if (KS == 64) { if (mask) launch_ws_inst<1, 64, 0, true>(P, tm, n_stages, grid, smem, st); else launch_ws_inst<1, 64, 0, false>(P, tm, n_stages, grid, smem, st); }
@@ -710,8 +703,7 @@ static bool launch_ws_wgrad(const float* X, int64_t ldx, const float* dY, int64_
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div(M, ROWS), sms));
   CUtensorMap tmX, tmY;
-  const bool use_tma = !(getenv("KP_TC_TMA") != nullptr && atoi(getenv("KP_TC_TMA")) == 0) &&
-                       make_tmap_2d(&tmX, X, M, K, ldx, ROWS, true) && make_tmap_2d(&tmY, dY, M, N, lddy, ROWS, true);
+  const bool use_tma = make_tmap_2d(&tmX, X, M, K, ldx, ROWS, true) && make_tmap_2d(&tmY, dY, M, N, lddy, ROWS, true);
   if (use_tma) {
     auto kern = tc_ws_wgrad_kernel<K_PAD, N_PAD, ROWS, true>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
