@@ -355,6 +355,23 @@ int64_t kp_compose_frame_scratch_bytes(int H, int W, int P);
 int kp_compose_frame(const float* const* panels, const int* kinds, int P, int H, int W, const float* accumulation,
                      const float* turbo, const float* viridis, void* scratch, uint8_t* out, void* stream);
 
+/* ---- baseline JPEG encoding of a composed frame (the image files and Motion-JPEG video of a rendered camera path):
+ *      image uint8 [H, W, 3] RGB, 1 <= H, W <= 65535 -> out: one baseline JFIF file (SOF0, YCbCr 4:2:0, the Annex K.1
+ *      quantisation tables at the IJG quality scaling, the Annex K.3 Huffman tables, RSTm every KP_JPEG_RESTART_MCUS
+ *      MCUs), SOI ... EOI, and *length = its byte count (int64, device).  header: the KP_JPEG_HEADER_BYTES bytes
+ *      kp_jpeg_header(H, W, quality) writes (on the HOST; the caller copies them to the device once per key), SOI to SOS;
+ *      the kernel quantises with the header's DQT tables.  out: kp_jpeg_encode_capacity(H, W) device bytes, the worst
+ *      case (bytes past *length are not written).  scratch: kp_jpeg_encode_scratch_bytes(H, W) device bytes, 256-byte
+ *      aligned.  Colour conversion, edge padding and chroma downsampling are libjpeg's integer formulas; the DCT is fp32.
+ *      3 launches, no host synchronisation, graph-capturable. ---- */
+#define KP_JPEG_RESTART_MCUS 4
+#define KP_JPEG_HEADER_BYTES 613
+int64_t kp_jpeg_encode_capacity(int H, int W);
+int64_t kp_jpeg_encode_scratch_bytes(int H, int W);
+int kp_jpeg_header(int H, int W, int quality, uint8_t* header);
+int kp_jpeg_encode(const uint8_t* image, int H, int W, const uint8_t* header, void* scratch, uint8_t* out, int64_t* length,
+                   void* stream);
+
 /* ---- (e) data-parallel gradient all-reduce over NVLink peer memory (replaces the NCCL all-reduce torch DDP issues
  *      around NS/engine/trainer.py:382-412).  Every rank allocates one ARENA = [KP_PEER_SIGNAL_BYTES of flag words |
  *      data], exports its CUDA-IPC handle, and opens the arenas of the other ranks of the node.  kp_peer_allreduce

@@ -82,6 +82,10 @@ SIGNATURES = {
     "kp_image_metrics": ([_P, _P, c_int, c_int, c_int, _P, _P, _P], c_int),
     "kp_compose_frame_scratch_bytes": ([c_int, c_int, c_int], c_int64),
     "kp_compose_frame": ([_P, POINTER(c_int), c_int, c_int, c_int, _P, _P, _P, _P, _P, _P], c_int),
+    "kp_jpeg_encode_capacity": ([c_int, c_int], c_int64),
+    "kp_jpeg_encode_scratch_bytes": ([c_int, c_int], c_int64),
+    "kp_jpeg_header": ([c_int, c_int, c_int, _P], c_int),
+    "kp_jpeg_encode": ([_P, c_int, c_int, _P, _P, _P, _P, _P], c_int),
     "kp_loss_head_fwd": ([_P, _P, c_int64, _P, _P, _P, c_int, c_float, c_float, c_float, _P, c_int, _P, _P, _P, _P, _P], c_int),
     "kp_loss_head_bwd": ([_P, _P, c_int64, _P, c_int, c_float, c_float, c_float, _P, _P, _P, _P, _P, _P], c_int),
     "kp_peer_alloc": ([c_int64, POINTER(c_void_p), _P], c_int),

@@ -61,6 +61,16 @@ def get_path_from_json(camera_path: Dict[str, Any]) -> Cameras:
                    camera_type=camera_type, times=times)
 
 
+def get_seconds_from_json(camera_path: Dict[str, Any]) -> float:
+    """The path's ``seconds``: how long its video plays (``len(camera_path) / seconds`` frames per second)."""
+    if "seconds" not in camera_path:
+        raise ValueError("camera path: no 'seconds' entry; a video needs the path's length in seconds")
+    seconds = float(camera_path["seconds"])
+    if not seconds > 0 or not math.isfinite(seconds):
+        raise ValueError(f"camera path: seconds must be positive and finite (got {camera_path['seconds']!r})")
+    return seconds
+
+
 @dataclass
 class CropData:
     """A crop of the render (scripts/render.py ``CropData``): outside the box the background colour shows."""

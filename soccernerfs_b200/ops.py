@@ -955,6 +955,51 @@ def compose_frame(frames: Dict[str, torch.Tensor], names: Sequence[str]) -> torc
     return out
 
 
+_JPEG_HEADERS: Dict = {}
+JPEG_HEADER_BYTES = 613  # KP_JPEG_HEADER_BYTES
+
+
+def _jpeg_header(device, h: int, w: int, quality: int) -> torch.Tensor:
+    key = (str(device), h, w, quality)
+    if key not in _JPEG_HEADERS:  # built on the host and copied once per (device, size, quality): no copy per frame
+        host = torch.empty(JPEG_HEADER_BYTES, dtype=torch.uint8)
+        call("kp_jpeg_header", h, w, quality, c_void_p(host.data_ptr()))
+        _JPEG_HEADERS[key] = host.to(device)
+    return _JPEG_HEADERS[key]
+
+
+def jpeg_capacity(h: int, w: int) -> int:
+    """Bytes ``encode_jpeg`` reserves for an h x w image: the worst-case file size (kp_jpeg_encode_capacity)."""
+    return int(_lib.load().kp_jpeg_encode_capacity(h, w))
+
+
+def encode_jpeg(image: torch.Tensor, quality: int = 95) -> Tuple[torch.Tensor, torch.Tensor]:
+    """A uint8 RGB CUDA image [H, W, 3] -> one baseline JPEG (JFIF, YCbCr 4:2:0, IJG ``quality`` 1..100) encoded on the
+    device (kp_jpeg_encode): ``(bytes uint8 [jpeg_capacity(H, W)], length int64 [1])``, both on the image's device; the
+    file is ``bytes[:length]``.  On the current stream, no host synchronisation (graph-capturable once the header for
+    this size and quality has been built by an earlier call)."""
+    if not isinstance(quality, int) or isinstance(quality, bool) or not 1 <= quality <= 100:
+        raise ValueError(f"encode_jpeg: quality {quality!r} is not an integer in 1..100")
+    if image.dim() != 3 or image.shape[2] != 3:
+        raise ValueError(f"encode_jpeg: image is {tuple(image.shape)}; expected [H, W, 3]")
+    h, w = int(image.shape[0]), int(image.shape[1])
+    if not (1 <= h <= 65535 and 1 <= w <= 65535):
+        raise ValueError(f"encode_jpeg: a {h}x{w} image; JPEG needs 1..65535 rows and columns")
+    if image.dtype != torch.uint8:
+        raise TypeError(f"encode_jpeg: image must be uint8 (got {image.dtype})")
+    if not image.is_cuda:
+        raise RuntimeError("encode_jpeg: image must be a CUDA tensor (there is no CPU path)")
+    image = image.contiguous()
+    dev = image.device
+    header = _jpeg_header(dev, h, w, quality)
+    out = torch.empty(jpeg_capacity(h, w), dtype=torch.uint8, device=dev)
+    length = torch.empty(1, dtype=torch.int64, device=dev)
+    scratch = torch.empty(int(_lib.load().kp_jpeg_encode_scratch_bytes(h, w)), dtype=torch.uint8, device=dev)
+    call("kp_jpeg_encode", c_void_p(image.data_ptr()), h, w, c_void_p(header.data_ptr()), c_void_p(scratch.data_ptr()),
+         c_void_p(out.data_ptr()), ptr(length), stream_ptr())
+    return out, length
+
+
 _HEAD_WS: Dict = {}
 
 
