@@ -250,12 +250,6 @@ int kp_step_scalars(int64_t* step_counter, const double* lr_table, const float* 
                     const float* betas_host, float grad_scale, float* anneal_out /* device, or NULL */,
                     float* const* hyper_out_host, void* stream);
 
-/* ---- (f1) Adam over a flat fp32 buffer (torch.optim.Adam math; NS/engine/optimizers.py:74-160,
- *      method_configs.py:546-557: lr 1e-2, eps 1e-12).  step is 1-based. ---------------------------- */
-int kp_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
-                 float beta1, float beta2, float eps, float weight_decay, int64_t step, float grad_scale,
-                 void* stream);
-
 /* Repack between the reference's NCHW [1,C,H,W] checkpoint layout and channel-last [H,W,C]. */
 int kp_repack_nchw_to_hwc(const float* src, float* dst, int C, int H, int W, void* stream);
 int kp_repack_hwc_to_nchw(const float* src, float* dst, int C, int H, int W, void* stream);

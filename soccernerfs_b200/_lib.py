@@ -72,7 +72,6 @@ SIGNATURES = {
                           _P, c_int64, c_int, _P], c_int),
     "kp_step_scalars": ([_P, _P, _P, c_int64, c_int, POINTER(c_float), c_float, _P, _P, _P], c_int),
     "kp_adam_multi": ([_P, _P, _P, _P, _P, c_int, c_float, c_float, c_float, c_float, c_float, c_int64, c_float, _P, _P], c_int),
-    "kp_adam_step": ([_P, _P, _P, _P, c_int64, c_float, c_float, c_float, c_float, c_float, c_int64, c_float, _P], c_int),
     "kp_generate_rays": ([_P, _P, _P, _P, _P, c_int, _P, c_int, c_int, c_int64, c_int64, c_float, _P, _P, _P, _P, _P, _P], c_int),
     "kp_ist_map": ([_P, c_int, c_int64, _P, _P, c_float, _P, _P], c_int),
     "kp_isg_map": ([_P, c_int, c_int64, _P, _P, _P, c_int, c_int, c_float, _P, _P, _P], c_int),

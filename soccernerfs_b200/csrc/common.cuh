@@ -1,6 +1,7 @@
 // Shared device/host helpers for libkplanes_b200 (sm_100a only).
 #pragma once
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -137,6 +138,46 @@ __device__ __forceinline__ float nan_to_num(float x) {
   if (isnan(x)) return 0.f;
   if (isinf(x)) return x > 0 ? 3.4028234663852886e38f : -3.4028234663852886e38f;
   return x;
+}
+
+// ---- torch.optim.Adam (NS/engine/optimizers.py:74-160), the one update rule of every optimizer kernel ----------------
+struct AdamScalars {
+  float lr_over_bc1, inv_sqrt_bc2, beta1, beta2, eps, wd, grad_scale;
+};
+
+// Bias corrections of a 1-based step, in double as torch computes them.
+static inline AdamScalars adam_scalars(float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,
+                                       float grad_scale) {
+  const double bc1 = 1.0 - pow((double)beta1, (double)step);
+  const double bc2 = 1.0 - pow((double)beta2, (double)step);
+  return AdamScalars{(float)(lr / bc1), (float)(1.0 / sqrt(bc2)), beta1, beta2, eps, weight_decay, grad_scale};
+}
+
+// hyper_dev (optional, DEVICE float[3] = lr/bias_corr1, 1/sqrt(bias_corr2), grad_scale) overrides the host scalars, so a
+// captured CUDA graph can be replayed with fresh per-step values (kp_step_scalars writes them).
+__device__ __forceinline__ AdamScalars with_hyper_dev(AdamScalars s, const float* hyper_dev) {
+  if (hyper_dev != nullptr) {
+    s.lr_over_bc1 = hyper_dev[0];
+    s.inv_sqrt_bc2 = hyper_dev[1];
+    s.grad_scale = hyper_dev[2];
+  }
+  return s;
+}
+
+// One element; g is the gradient with grad_scale already applied.  Every rounding is spelled out (fmaf, __fmul_rn) so
+// that all callers compute the same bits: left to the compiler, `v * beta2 + (1 - beta2) * gr * gr` was contracted one way
+// in one kernel and the other way in another.
+__device__ __forceinline__ void adam_update(float g, float& p, float& m, float& v, const AdamScalars& s) {
+  const float gr = fmaf(s.wd, p, g);
+  m = fmaf(gr - m, 1.f - s.beta1, m);
+  v = fmaf(v, s.beta2, __fmul_rn(__fmul_rn((1.f - s.beta2), gr), gr));
+  p -= s.lr_over_bc1 * m / fmaf(sqrtf(v), s.inv_sqrt_bc2, s.eps);
+}
+__device__ __forceinline__ void adam_update4(float4 g, float4& p, float4& m, float4& v, const AdamScalars& s) {
+  adam_update(g.x, p.x, m.x, v.x, s);
+  adam_update(g.y, p.y, m.y, v.y, s);
+  adam_update(g.z, p.z, m.z, v.z, s);
+  adam_update(g.w, p.w, m.w, v.w, s);
 }
 
 }  // namespace kp

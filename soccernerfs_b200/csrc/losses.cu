@@ -1,7 +1,6 @@
 // Loss kernels (sm_100a).
 //   kp_distortion_*  : lossfun_distortion, NS/model_components/losses.py:125-136 (O(S^2) per ray, one warp per ray)
 //   kp_interlevel_*  : outer / lossfun_outer, losses.py:46-95 (two searchsorted(side="right") + cumsum differences)
-//   kp_adam_step     : torch.optim.Adam update over a flat buffer (NS/engine/optimizers.py:74-160).
 #include "common.cuh"
 
 namespace kp {
@@ -113,37 +112,6 @@ __global__ void __launch_bounds__(32 * kRaysPerBlock) interlevel_kernel(const fl
   }
 }
 
-__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g,
-                                                   float* __restrict__ m, float* __restrict__ v, int64_t n, float lr_over_bc1,
-                                                   float beta1, float beta2, float eps, float wd, float inv_sqrt_bc2,
-                                                   float grad_scale) {
-  const int64_t i4 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
-  if (i4 >= n) return;
-  if (i4 + 4 <= n) {
-    float4 pp = *reinterpret_cast<float4*>(p + i4);
-    const float4 gg = *reinterpret_cast<const float4*>(g + i4);
-    float4 mm = *reinterpret_cast<float4*>(m + i4), vv = *reinterpret_cast<float4*>(v + i4);
-    float* pa = &pp.x; const float* ga = &gg.x; float* ma = &mm.x; float* va = &vv.x;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      float gr = ga[k] * grad_scale + wd * pa[k];
-      ma[k] = ma[k] + (gr - ma[k]) * (1.f - beta1);
-      va[k] = va[k] * beta2 + (1.f - beta2) * gr * gr;
-      pa[k] -= lr_over_bc1 * ma[k] / (sqrtf(va[k]) * inv_sqrt_bc2 + eps);
-    }
-    *reinterpret_cast<float4*>(p + i4) = pp;
-    *reinterpret_cast<float4*>(m + i4) = mm;
-    *reinterpret_cast<float4*>(v + i4) = vv;
-  } else {
-    for (int64_t i = i4; i < n; ++i) {
-      float gr = g[i] * grad_scale + wd * p[i];
-      m[i] = m[i] + (gr - m[i]) * (1.f - beta1);
-      v[i] = v[i] * beta2 + (1.f - beta2) * gr * gr;
-      p[i] -= lr_over_bc1 * m[i] / (sqrtf(v[i]) * inv_sqrt_bc2 + eps);
-    }
-  }
-}
-
 __global__ void repack_kernel(const float* __restrict__ src, float* __restrict__ dst, int C, int H, int W, int to_hwc) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t total = (int64_t)C * H * W;
@@ -208,22 +176,6 @@ extern "C" int kp_interlevel_bwd(const float* c, const float* w, const float* cp
   interlevel_kernel<true><<<(unsigned)ceil_div(N, kRaysPerBlock), 32 * kRaysPerBlock, smem, as_stream(stream)>>>(
       c, w, cp, wp, grad_loss, N, S, Sp, nullptr, grad_wp);
   KP_LAUNCH_CHECK("interlevel_bwd");
-  return 0;
-}
-
-extern "C" int kp_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
-                            float beta1, float beta2, float eps, float weight_decay, int64_t step, float grad_scale,
-                            void* stream) {
-  if (n == 0) return 0;
-  KP_CHECK(param && grad && exp_avg && exp_avg_sq && step >= 1, "adam_step: bad arguments");
-  KP_CHECK((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0,
-           "adam_step: buffers must be 16-byte aligned");
-  const double bc1 = 1.0 - pow((double)beta1, (double)step);
-  const double bc2 = 1.0 - pow((double)beta2, (double)step);
-  adam_kernel<<<(unsigned)ceil_div(ceil_div(n, 4), 256), 256, 0, as_stream(stream)>>>(
-      param, grad, exp_avg, exp_avg_sq, n, (float)(lr / bc1), beta1, beta2, eps, weight_decay, (float)(1.0 / sqrt(bc2)),
-      grad_scale);
-  KP_LAUNCH_CHECK("adam_step");
   return 0;
 }
 

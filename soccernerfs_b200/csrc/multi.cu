@@ -4,9 +4,10 @@
 //                                        one sweep (the default model has 36 planes; per-plane launches were
 //                                        launch-latency bound).
 //   kp_plane_reg_adam                  : the same regulariser stencil fused with an in-place Adam step.
-//   kp_adam_multi                      : torch.optim.Adam over a list of dense fp32 tensors (NS/engine/optimizers.py:74-160,
-//                                        method_configs.py:546-557); hyper-parameters may come from device memory so
-//                                        the step can be replayed from a CUDA graph.
+//   kp_adam_multi                      : torch.optim.Adam over a list of dense fp32 tensors that share one step count
+//                                        (NS/engine/optimizers.py:74-160, method_configs.py:546-557); hyper-parameters
+//                                        may come from device memory so the step can be replayed from a CUDA graph.
+// Both Adam passes apply the update rule of common.cuh (adam_update).
 // Work is split into fixed-size chunks or tiles; a block finds its (tensor, chunk) by a short scan of a prefix table
 // that travels in the kernel parameters.
 #include "common.cuh"
@@ -191,14 +192,8 @@ struct AdamTable {
 };
 
 __global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__ AdamTable T,
-                                                         const float* __restrict__ hyper_dev, float lr_over_bc1,
-                                                         float inv_sqrt_bc2, float beta1, float beta2, float eps, float wd,
-                                                         float grad_scale) {
-  if (hyper_dev != nullptr) {  // graph-replayable path: per-step scalars live in device memory
-    lr_over_bc1 = hyper_dev[0];
-    inv_sqrt_bc2 = hyper_dev[1];
-    grad_scale = hyper_dev[2];
-  }
+                                                         const float* __restrict__ hyper_dev, AdamScalars s) {
+  s = with_hyper_dev(s, hyper_dev);
   const int ti = find_tensor(T.first_block, T.n, blockIdx.x);
   const AdamTensor& A = T.t[ti];
   const int64_t base = (int64_t)(blockIdx.x - T.first_block[ti]) * kChunk * 4;
@@ -211,24 +206,12 @@ __global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__
       float4 pp = *reinterpret_cast<float4*>(A.p + i4);
       const float4 gg = *reinterpret_cast<const float4*>(A.g + i4);
       float4 mm = *reinterpret_cast<float4*>(A.m + i4), vv = *reinterpret_cast<float4*>(A.v + i4);
-      float* pa = &pp.x; const float* ga = &gg.x; float* ma = &mm.x; float* va = &vv.x;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const float gr = ga[k] * grad_scale + wd * pa[k];
-        ma[k] = ma[k] + (gr - ma[k]) * (1.f - beta1);
-        va[k] = va[k] * beta2 + (1.f - beta2) * gr * gr;
-        pa[k] -= lr_over_bc1 * ma[k] / (sqrtf(va[k]) * inv_sqrt_bc2 + eps);
-      }
+      adam_update4(scale4(gg, s.grad_scale), pp, mm, vv, s);
       *reinterpret_cast<float4*>(A.p + i4) = pp;
       *reinterpret_cast<float4*>(A.m + i4) = mm;
       *reinterpret_cast<float4*>(A.v + i4) = vv;
     } else {
-      for (int64_t i = i4; i < A.n && i < i4 + 4; ++i) {
-        const float gr = A.g[i] * grad_scale + wd * A.p[i];
-        A.m[i] = A.m[i] + (gr - A.m[i]) * (1.f - beta1);
-        A.v[i] = A.v[i] * beta2 + (1.f - beta2) * gr * gr;
-        A.p[i] -= lr_over_bc1 * A.m[i] / (sqrtf(A.v[i]) * inv_sqrt_bc2 + eps);
-      }
+      for (int64_t i = i4; i < A.n && i < i4 + 4; ++i) adam_update(A.g[i] * s.grad_scale, A.p[i], A.m[i], A.v[i], s);
     }
   }
 }
@@ -295,14 +278,8 @@ __global__ void __launch_bounds__(256) plane_halo_snapshot_kernel(const __grid_c
 template <bool ZERO_GRAD>
 __global__ void __launch_bounds__(256, 3) plane_reg_adam_kernel(const __grid_constant__ RegAdamTable T, const float4* __restrict__ halo,
                                                              const float* __restrict__ coef, double* __restrict__ sums,
-                                                             const float* __restrict__ hyper_dev, float lr_over_bc1,
-                                                             float inv_sqrt_bc2, float beta1, float beta2, float eps, float wd,
-                                                             float grad_scale) {
-  if (hyper_dev != nullptr) {
-    lr_over_bc1 = hyper_dev[0];
-    inv_sqrt_bc2 = hyper_dev[1];
-    grad_scale = hyper_dev[2];
-  }
+                                                             const float* __restrict__ hyper_dev, AdamScalars adam) {
+  adam = with_hyper_dev(adam, hyper_dev);
   __shared__ float4 xch[2][256];
   const int p = find_tensor(T.first_block, T.n, blockIdx.x);
   const RegAdamPlane& P = T.pl[p];
@@ -362,14 +339,9 @@ __global__ void __launch_bounds__(256, 3) plane_reg_adam_kernel(const __grid_con
       const float4 g = reg_stencil(terms, coef4, h, H, hasL, hasR, true, a, b, c, d, e,
                                    [&] { return edgeL ? hL : x[tid - C4]; }, [&] { return edgeR ? hR : x[tid + C4]; }, s);
       float4 pn = c, mm = mm0, vv = vv0;
-      float* pa = &pn.x; const float* ga = &gg.x; const float* ra = &g.x; float* ma = &mm.x; float* va = &vv.x;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {  // torch.optim.Adam, same operation order as adam_multi_kernel
-        const float gr = (ga[k] * grad_scale + ra[k]) + wd * pa[k];
-        ma[k] = ma[k] + (gr - ma[k]) * (1.f - beta1);
-        va[k] = va[k] * beta2 + (1.f - beta2) * gr * gr;
-        pa[k] -= lr_over_bc1 * ma[k] / (sqrtf(va[k]) * inv_sqrt_bc2 + eps);
-      }
+      const float gs = adam.grad_scale;
+      adam_update4(make_float4(fmaf(gg.x, gs, g.x), fmaf(gg.y, gs, g.y), fmaf(gg.z, gs, g.z), fmaf(gg.w, gs, g.w)), pn, mm, vv,
+                   adam);
       const size_t i = (size_t)h * row4 + col;
       pp[i] = pn; mp[i] = mm; vp[i] = vv;
       // untouched lines (85 % of the 32x scale per step) are still zero: skip the store (same value, less HBM write traffic)
@@ -500,8 +472,7 @@ extern "C" int kp_adam_multi(float* const* params, const float* const* grads, fl
                              float eps, float weight_decay, int64_t step, float grad_scale, const float* hyper_dev,
                              void* stream) {
   KP_CHECK(params && grads && exp_avg && exp_avg_sq && sizes && P >= 0 && step >= 1, "adam_multi: bad arguments");
-  const double bc1 = 1.0 - pow((double)beta1, (double)step);
-  const double bc2 = 1.0 - pow((double)beta2, (double)step);
+  const AdamScalars adam = adam_scalars(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
   for (int begin = 0; begin < P; begin += kMaxTensors) {
     const int end = std::min(P, begin + kMaxTensors);
     AdamTable T;
@@ -515,8 +486,7 @@ extern "C" int kp_adam_multi(float* const* params, const float* const* grads, fl
     T.first_block[k] = nb;
     T.n = k;
     if (nb == 0) continue;
-    adam_multi_kernel<<<nb, 256, 0, as_stream(stream)>>>(T, hyper_dev, (float)(lr / bc1), (float)(1.0 / sqrt(bc2)), beta1,
-                                                         beta2, eps, weight_decay, grad_scale);
+    adam_multi_kernel<<<nb, 256, 0, as_stream(stream)>>>(T, hyper_dev, adam);
     KP_LAUNCH_CHECK("adam_multi");
   }
   return 0;
@@ -543,8 +513,7 @@ extern "C" int kp_plane_reg_adam(float* const* planes, float* const* grads, floa
            "plane_reg_adam: bad arguments");
   KP_CHECK(scratch_bytes >= kp_plane_reg_adam_scratch_bytes(hwc, P), "plane_reg_adam: scratch too small (%lld bytes)",
            (long long)scratch_bytes);
-  const double bc1 = 1.0 - pow((double)beta1, (double)step);
-  const double bc2 = 1.0 - pow((double)beta2, (double)step);
+  const AdamScalars adam = adam_scalars(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
   float4* halo = reinterpret_cast<float4*>(scratch);
   for (int begin = 0; begin < P; begin += kFMaxTensors) {
     const int end = std::min(P, begin + kFMaxTensors);
@@ -571,12 +540,8 @@ extern "C" int kp_plane_reg_adam(float* const* planes, float* const* grads, floa
     kp::g_launches += 1;
     double* s = sums ? sums + (size_t)begin * 4 : nullptr;
     const float* cf = coef_dev + (size_t)begin * 4;
-    if (zero_grads)
-      plane_reg_adam_kernel<true><<<nb, 256, 0, st>>>(T, halo, cf, s, hyper_dev, (float)(lr / bc1), (float)(1.0 / sqrt(bc2)), beta1,
-                                                      beta2, eps, weight_decay, grad_scale);
-    else
-      plane_reg_adam_kernel<false><<<nb, 256, 0, st>>>(T, halo, cf, s, hyper_dev, (float)(lr / bc1), (float)(1.0 / sqrt(bc2)), beta1,
-                                                       beta2, eps, weight_decay, grad_scale);
+    if (zero_grads) plane_reg_adam_kernel<true><<<nb, 256, 0, st>>>(T, halo, cf, s, hyper_dev, adam);
+    else plane_reg_adam_kernel<false><<<nb, 256, 0, st>>>(T, halo, cf, s, hyper_dev, adam);
     KP_LAUNCH_CHECK("plane_reg_adam");
     halo += (size_t)nb * kFHaloF4;
   }

@@ -147,8 +147,8 @@ struct ShardedAdamArgs {
   float* v;
   int rank, world;
   int64_t n4;                    // group size in float4 units
-  const float* hyper_dev;        // optional DEVICE {lr / bias_corr1, 1 / sqrt(bias_corr2), grad_scale}
-  float lr_over_bc1, inv_sqrt_bc2, beta1, beta2, eps, wd, grad_scale;
+  const float* hyper_dev;        // optional, see with_hyper_dev
+  AdamScalars adam;
   uint8_t* touched[kPeerMaxWorld];  // sparse variant: one byte per 128-byte line of every rank's gradient region
 };
 
@@ -165,12 +165,7 @@ __global__ void __launch_bounds__(kPeerThreads) peer_sharded_adam_kernel(const _
   __syncthreads();
   const uint32_t flag = s_flag;
   peer_barrier(b, 0, flag);
-  float lr_over_bc1 = a.lr_over_bc1, inv_sqrt_bc2 = a.inv_sqrt_bc2, grad_scale = a.grad_scale;
-  if (a.hyper_dev != nullptr) {
-    lr_over_bc1 = a.hyper_dev[0];
-    inv_sqrt_bc2 = a.hyper_dev[1];
-    grad_scale = a.hyper_dev[2];
-  }
+  const AdamScalars adam = with_hyper_dev(a.adam, a.hyper_dev);
   const int64_t lo = a.n4 * a.rank / N, hi = a.n4 * (a.rank + 1) / N;
   const int64_t stride = (int64_t)gridDim.x * kPeerThreads;
   constexpr int U = 2;
@@ -194,14 +189,7 @@ __global__ void __launch_bounds__(kPeerThreads) peer_sharded_adam_kernel(const _
         float4 s = g[u][0];
 #pragma unroll
         for (int p = 1; p < N; ++p) { s.x += g[u][p].x; s.y += g[u][p].y; s.z += g[u][p].z; s.w += g[u][p].w; }
-        float* ga = &s.x; float* pa = &pp[u].x; float* ma = &mm[u].x; float* va = &vv[u].x;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {  // torch.optim.Adam (same arithmetic as adam_multi_kernel)
-          const float gr = ga[k] * grad_scale + a.wd * pa[k];
-          ma[k] = ma[k] + (gr - ma[k]) * (1.f - a.beta1);
-          va[k] = va[k] * a.beta2 + (1.f - a.beta2) * gr * gr;
-          pa[k] -= lr_over_bc1 * ma[k] / (sqrtf(va[k]) * inv_sqrt_bc2 + a.eps);
-        }
+        adam_update4(scale4(s, adam.grad_scale), pp[u], mm[u], vv[u], adam);
         *reinterpret_cast<float4*>(a.m + 4 * (i - lo)) = mm[u];
         *reinterpret_cast<float4*>(a.v + 4 * (i - lo)) = vv[u];
 #pragma unroll
@@ -243,12 +231,7 @@ __global__ void __launch_bounds__(kPeerThreads) peer_sharded_adam_sparse_kernel(
   __syncthreads();
   const uint32_t flag = s_flag;
   peer_barrier(b, 0, flag);
-  float lr_over_bc1 = a.lr_over_bc1, inv_sqrt_bc2 = a.inv_sqrt_bc2, grad_scale = a.grad_scale;
-  if (a.hyper_dev != nullptr) {
-    lr_over_bc1 = a.hyper_dev[0];
-    inv_sqrt_bc2 = a.hyper_dev[1];
-    grad_scale = a.hyper_dev[2];
-  }
+  const AdamScalars adam = with_hyper_dev(a.adam, a.hyper_dev);
   const int64_t lo = a.n4 * a.rank / N, hi = a.n4 * (a.rank + 1) / N;
   const int64_t stride = (int64_t)gridDim.x * kPeerThreads;
   constexpr int U = N <= 4 ? 4 : 2;  // elements in flight per thread (U*N 16-byte peer loads)
@@ -288,14 +271,7 @@ __global__ void __launch_bounds__(kPeerThreads) peer_sharded_adam_sparse_kernel(
         float4 sum = s[u];
 #pragma unroll
         for (int p = 0; p < N; ++p) { sum.x += g[u][p].x; sum.y += g[u][p].y; sum.z += g[u][p].z; sum.w += g[u][p].w; }
-        float* ga = &sum.x; float* pa = &pp[u].x; float* ma = &mm[u].x; float* va = &vv[u].x;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {  // torch.optim.Adam (same arithmetic as adam_multi_kernel)
-          const float gr = ga[k] * grad_scale + a.wd * pa[k];
-          ma[k] = ma[k] + (gr - ma[k]) * (1.f - a.beta1);
-          va[k] = va[k] * a.beta2 + (1.f - a.beta2) * gr * gr;
-          pa[k] -= lr_over_bc1 * ma[k] / (sqrtf(va[k]) * inv_sqrt_bc2 + a.eps);
-        }
+        adam_update4(scale4(sum, adam.grad_scale), pp[u], mm[u], vv[u], adam);
         *reinterpret_cast<float4*>(a.m + 4 * (i - lo)) = mm[u];
         *reinterpret_cast<float4*>(a.v + 4 * (i - lo)) = vv[u];
 #pragma unroll
@@ -342,75 +318,33 @@ __global__ void __launch_bounds__(kPeerThreads) peer_touched_cleanup_kernel(floa
 
 using namespace kp;
 
-extern "C" int kp_peer_sharded_adam(void* const* arenas, int rank, int world, int64_t grad_begin, int64_t param_begin,
-                                    int64_t count, float* exp_avg_shard, float* exp_avg_sq_shard, float lr, float beta1,
-                                    float beta2, float eps, float weight_decay, int64_t step, float grad_scale,
-                                    const float* hyper_dev, int blocks, void* stream) {
-  KP_CHECK(arenas != nullptr && exp_avg_shard != nullptr && exp_avg_sq_shard != nullptr, "peer_sharded_adam: NULL argument");
-  KP_CHECK(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "peer_sharded_adam: rank %d / world %d", rank, world);
-  KP_CHECK(grad_begin >= 0 && param_begin >= 0 && count >= 0 && grad_begin % 4 == 0 && param_begin % 4 == 0 && count % 4 == 0,
-           "peer_sharded_adam: offsets / count must be multiples of 4 floats");
-  KP_CHECK(step >= 1, "peer_sharded_adam: step is 1-based");
-  if (count == 0) return 0;
-  if (blocks <= 0) blocks = 64;
-  KP_CHECK(blocks <= kPeerMaxBlocks, "peer_sharded_adam: blocks=%d > %d", blocks, kPeerMaxBlocks);
-  ShardedAdamArgs a;
-  for (int p = 0; p < kPeerMaxWorld; ++p) { a.grad[p] = nullptr; a.param[p] = nullptr; a.sig[p] = nullptr; }
-  for (int p = 0; p < world; ++p) {
-    KP_CHECK(arenas[p] != nullptr, "peer_sharded_adam: arena %d is NULL", p);
-    a.sig[p] = reinterpret_cast<uint32_t*>(arenas[p]);
-    float* data = reinterpret_cast<float*>(reinterpret_cast<char*>(arenas[p]) + KP_PEER_SIGNAL_BYTES);
-    a.grad[p] = data + grad_begin;
-    a.param[p] = data + param_begin;
-  }
-  a.m = exp_avg_shard;
-  a.v = exp_avg_sq_shard;
-  a.rank = rank;
-  a.world = world;
-  a.n4 = count / 4;
-  a.hyper_dev = hyper_dev;
-  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-  a.lr_over_bc1 = (float)(lr / bc1);
-  a.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
-  a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.wd = weight_decay; a.grad_scale = grad_scale;
-  cudaStream_t st = as_stream(stream);
-  switch (world) {
-    case 1: peer_sharded_adam_kernel<1><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 2: peer_sharded_adam_kernel<2><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 3: peer_sharded_adam_kernel<3><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 4: peer_sharded_adam_kernel<4><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 5: peer_sharded_adam_kernel<5><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 6: peer_sharded_adam_kernel<6><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 7: peer_sharded_adam_kernel<7><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 8: peer_sharded_adam_kernel<8><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    default: set_error("peer_sharded_adam: world=%d unsupported", world); return 1;
-  }
-  KP_LAUNCH_CHECK("peer_sharded_adam");
-  return 0;
+template <int N>
+static void launch_sharded_adam(bool sparse, int blocks, cudaStream_t st, const ShardedAdamArgs& a) {
+  if (sparse) peer_sharded_adam_sparse_kernel<N><<<blocks, kPeerThreads, 0, st>>>(a);
+  else peer_sharded_adam_kernel<N><<<blocks, kPeerThreads, 0, st>>>(a);
 }
 
-extern "C" int kp_peer_sharded_adam_sparse(void* const* arenas, int rank, int world, int64_t grad_begin, int64_t param_begin,
-                                           int64_t touched_begin, int64_t count, float* exp_avg_shard, float* exp_avg_sq_shard,
-                                           float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,
-                                           float grad_scale, const float* hyper_dev, int blocks, void* stream) {
-  KP_CHECK(arenas != nullptr && exp_avg_shard != nullptr && exp_avg_sq_shard != nullptr, "peer_sharded_adam_sparse: NULL argument");
-  KP_CHECK(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "peer_sharded_adam_sparse: rank %d / world %d", rank, world);
-  KP_CHECK(grad_begin >= 0 && param_begin >= 0 && touched_begin >= 0 && count >= 0 && grad_begin % 32 == 0 && param_begin % 4 == 0 &&
-               touched_begin % 4 == 0 && count % 32 == 0,
-           "peer_sharded_adam_sparse: the gradient region must start and end on a 128-byte line");
-  KP_CHECK(step >= 1, "peer_sharded_adam_sparse: step is 1-based");
+// The part both sharded launchers share: checks, kernel arguments, the launch for world 1..8 and, for the sparse variant,
+// the clean-up.  touched_begin is read by the sparse variant only.
+static int peer_sharded_adam_impl(bool sparse, void* const* arenas, int rank, int world, int64_t grad_begin, int64_t param_begin,
+                                  int64_t touched_begin, int64_t count, float* exp_avg_shard, float* exp_avg_sq_shard, float lr,
+                                  float beta1, float beta2, float eps, float weight_decay, int64_t step, float grad_scale,
+                                  const float* hyper_dev, int blocks, void* stream) {
+  const char* name = sparse ? "peer_sharded_adam_sparse" : "peer_sharded_adam";
+  KP_CHECK(arenas != nullptr && exp_avg_shard != nullptr && exp_avg_sq_shard != nullptr, "%s: NULL argument", name);
+  KP_CHECK(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "%s: rank %d / world %d", name, rank, world);
+  KP_CHECK(step >= 1, "%s: step is 1-based", name);
   if (count == 0) return 0;
   if (blocks <= 0) blocks = 64;
-  KP_CHECK(blocks <= kPeerMaxBlocks, "peer_sharded_adam_sparse: blocks=%d > %d", blocks, kPeerMaxBlocks);
-  ShardedAdamArgs a;
-  for (int p = 0; p < kPeerMaxWorld; ++p) { a.grad[p] = nullptr; a.param[p] = nullptr; a.sig[p] = nullptr; a.touched[p] = nullptr; }
+  KP_CHECK(blocks <= kPeerMaxBlocks, "%s: blocks=%d > %d", name, blocks, kPeerMaxBlocks);
+  ShardedAdamArgs a = {};
   for (int p = 0; p < world; ++p) {
-    KP_CHECK(arenas[p] != nullptr, "peer_sharded_adam_sparse: arena %d is NULL", p);
+    KP_CHECK(arenas[p] != nullptr, "%s: arena %d is NULL", name, p);
     a.sig[p] = reinterpret_cast<uint32_t*>(arenas[p]);
     float* data = reinterpret_cast<float*>(reinterpret_cast<char*>(arenas[p]) + KP_PEER_SIGNAL_BYTES);
     a.grad[p] = data + grad_begin;
     a.param[p] = data + param_begin;
-    a.touched[p] = reinterpret_cast<uint8_t*>(data + touched_begin);
+    if (sparse) a.touched[p] = reinterpret_cast<uint8_t*>(data + touched_begin);
   }
   a.m = exp_avg_shard;
   a.v = exp_avg_sq_shard;
@@ -418,32 +352,49 @@ extern "C" int kp_peer_sharded_adam_sparse(void* const* arenas, int rank, int wo
   a.world = world;
   a.n4 = count / 4;
   a.hyper_dev = hyper_dev;
-  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-  a.lr_over_bc1 = (float)(lr / bc1);
-  a.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
-  a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.wd = weight_decay; a.grad_scale = grad_scale;
+  a.adam = adam_scalars(lr, beta1, beta2, eps, weight_decay, step, grad_scale);
   cudaStream_t st = as_stream(stream);
-  switch (world) {
-    case 1: peer_sharded_adam_sparse_kernel<1><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 2: peer_sharded_adam_sparse_kernel<2><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 3: peer_sharded_adam_sparse_kernel<3><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 4: peer_sharded_adam_sparse_kernel<4><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 5: peer_sharded_adam_sparse_kernel<5><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 6: peer_sharded_adam_sparse_kernel<6><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 7: peer_sharded_adam_sparse_kernel<7><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    case 8: peer_sharded_adam_sparse_kernel<8><<<blocks, kPeerThreads, 0, st>>>(a); break;
-    default: set_error("peer_sharded_adam_sparse: world=%d unsupported", world); return 1;
+  switch (world) {  // 1..kPeerMaxWorld, checked above
+    case 1: launch_sharded_adam<1>(sparse, blocks, st, a); break;
+    case 2: launch_sharded_adam<2>(sparse, blocks, st, a); break;
+    case 3: launch_sharded_adam<3>(sparse, blocks, st, a); break;
+    case 4: launch_sharded_adam<4>(sparse, blocks, st, a); break;
+    case 5: launch_sharded_adam<5>(sparse, blocks, st, a); break;
+    case 6: launch_sharded_adam<6>(sparse, blocks, st, a); break;
+    case 7: launch_sharded_adam<7>(sparse, blocks, st, a); break;
+    case 8: launch_sharded_adam<8>(sparse, blocks, st, a); break;
   }
-  kp::g_launches += 1;
-  {
+  if (sparse) {
+    kp::g_launches += 1;
     const int64_t lo = a.n4 * rank / world, hi = a.n4 * (rank + 1) / world;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     peer_touched_cleanup_kernel<<<sms * 8, kPeerThreads, 0, st>>>(a.grad[rank], a.touched[rank], a.n4, lo, hi);
   }
-  KP_LAUNCH_CHECK("peer_sharded_adam_sparse");
+  KP_LAUNCH_CHECK(name);
   return 0;
+}
+
+extern "C" int kp_peer_sharded_adam(void* const* arenas, int rank, int world, int64_t grad_begin, int64_t param_begin,
+                                    int64_t count, float* exp_avg_shard, float* exp_avg_sq_shard, float lr, float beta1,
+                                    float beta2, float eps, float weight_decay, int64_t step, float grad_scale,
+                                    const float* hyper_dev, int blocks, void* stream) {
+  KP_CHECK(grad_begin >= 0 && param_begin >= 0 && count >= 0 && grad_begin % 4 == 0 && param_begin % 4 == 0 && count % 4 == 0,
+           "peer_sharded_adam: offsets / count must be multiples of 4 floats");
+  return peer_sharded_adam_impl(false, arenas, rank, world, grad_begin, param_begin, 0, count, exp_avg_shard, exp_avg_sq_shard,
+                                lr, beta1, beta2, eps, weight_decay, step, grad_scale, hyper_dev, blocks, stream);
+}
+
+extern "C" int kp_peer_sharded_adam_sparse(void* const* arenas, int rank, int world, int64_t grad_begin, int64_t param_begin,
+                                           int64_t touched_begin, int64_t count, float* exp_avg_shard, float* exp_avg_sq_shard,
+                                           float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,
+                                           float grad_scale, const float* hyper_dev, int blocks, void* stream) {
+  KP_CHECK(grad_begin >= 0 && param_begin >= 0 && touched_begin >= 0 && count >= 0 && grad_begin % 32 == 0 && param_begin % 4 == 0 &&
+               touched_begin % 4 == 0 && count % 32 == 0,
+           "peer_sharded_adam_sparse: the gradient region must start and end on a 128-byte line");
+  return peer_sharded_adam_impl(true, arenas, rank, world, grad_begin, param_begin, touched_begin, count, exp_avg_shard,
+                                exp_avg_sq_shard, lr, beta1, beta2, eps, weight_decay, step, grad_scale, hyper_dev, blocks, stream);
 }
 
 extern "C" int kp_peer_alloc(int64_t data_bytes, void** arena, void* ipc_handle64) {

@@ -1,9 +1,9 @@
 """Optimizer / scheduler pieces the K-Planes training step needs (SURVEY.md 8f rank 1).
 
 ``FusedAdam`` has torch.optim.Adam's math (the reference uses ``AdamOptimizerConfig(lr=1e-2, eps=1e-12)``,
-NS/configs/method_configs.py:546-557, NS/engine/optimizers.py:74-160) executed by ``kp_adam_step``: one
-vectorised pass per parameter over param / grad / exp_avg / exp_avg_sq.  ``cosine_decay_factor`` is the
-reference's ``CosineDecayScheduler`` lambda (NS/engine/schedulers.py:126-142).
+NS/configs/method_configs.py:546-557, NS/engine/optimizers.py:74-160) executed by ``kp_adam_multi``: one
+vectorised pass over param / grad / exp_avg / exp_avg_sq of every parameter of a group that shares a step count.
+``cosine_decay_factor`` is the reference's ``CosineDecayScheduler`` lambda (NS/engine/schedulers.py:126-142).
 """
 from __future__ import annotations
 
@@ -32,7 +32,7 @@ class FusedAdam(torch.optim.Optimizer):
                 loss = closure()
         for group in self.param_groups:
             b1, b2 = group["betas"]
-            ps, gs, ms, vs = [], [], [], []
+            launches = {}  # step count -> (params, grads, exp_avgs, exp_avg_sqs)
             rp = []  # planes of this group routed through the fused regulariser + Adam pass
             for p in group["params"]:
                 if p.grad is None or p.numel() == 0:
@@ -51,6 +51,7 @@ class FusedAdam(torch.optim.Optimizer):
                         raise RuntimeError("fused regulariser + Adam pass: a plane's gradient must share the plane's layout")
                     rp.append(p)
                     continue
+                ps, gs, ms, vs = launches.setdefault(st["step"], ([], [], [], []))
                 ps.append(p), gs.append(g), ms.append(st["exp_avg"]), vs.append(st["exp_avg_sq"])
             if rp:
                 steps = {self.state[p]["step"] for p in rp}
@@ -60,15 +61,12 @@ class FusedAdam(torch.optim.Optimizer):
                                      [self.state[p]["exp_avg_sq"] for p in rp], group["lr"], b1, b2, group["eps"],
                                      group["weight_decay"], steps.pop(), grad_scale,
                                      hyper_dev=group.get("hyper_dev") if use_device_hyper else None)
-            if ps:
-                steps = {self.state[p]["step"] for p in ps}
-                if len(steps) != 1:  # parameters joined the optimizer at different times: per-tensor launches
-                    for p, g, m, v in zip(ps, gs, ms, vs):
-                        ops.adam_step_(p, g, m, v, group["lr"], b1, b2, group["eps"], group["weight_decay"],
-                                       self.state[p]["step"], grad_scale)
-                else:
-                    ops.adam_multi_(ps, gs, ms, vs, group["lr"], b1, b2, group["eps"], group["weight_decay"], steps.pop(),
-                                    grad_scale, hyper_dev=group.get("hyper_dev") if use_device_hyper else None)
+            # parameters that joined the optimizer at different times have different step counts: one launch per count,
+            # with the host's scalars (the device triple holds the bias corrections of one step count)
+            hyper_dev = group.get("hyper_dev") if use_device_hyper and len(launches) == 1 else None
+            for step, (ps, gs, ms, vs) in launches.items():
+                ops.adam_multi_(ps, gs, ms, vs, group["lr"], b1, b2, group["eps"], group["weight_decay"], step, grad_scale,
+                                hyper_dev=hyper_dev)
         return loss
 
 

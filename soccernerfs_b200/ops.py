@@ -1150,17 +1150,6 @@ def plane_reg_sums(planes: Sequence[torch.Tensor], terms: Sequence[int]) -> torc
 # ------------------------------------------------------------------------------------------------
 # (f1) Adam
 # ------------------------------------------------------------------------------------------------
-def adam_step_(param, grad, exp_avg, exp_avg_sq, lr, beta1, beta2, eps, weight_decay, step, grad_scale=1.0) -> None:
-    """In-place torch.optim.Adam update on (possibly channel-last) dense fp32 tensors sharing one memory layout."""
-    n = param.numel()
-    for t in (grad, exp_avg, exp_avg_sq):
-        if t.stride() != param.stride() or t.numel() != n:
-            raise RuntimeError("adam_step_: param/grad/state must share one dense layout")
-    call("kp_adam_step", c_void_p(param.data_ptr()), c_void_p(grad.data_ptr()), c_void_p(exp_avg.data_ptr()),
-         c_void_p(exp_avg_sq.data_ptr()), n, float(lr), float(beta1), float(beta2), float(eps), float(weight_decay), int(step),
-         float(grad_scale), stream_ptr())
-
-
 def plane_reg_adam_supported(c: int) -> bool:
     return bool(_lib.load().kp_plane_reg_adam_supported(int(c)))
 

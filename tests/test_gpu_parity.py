@@ -428,6 +428,88 @@ def test_fused_adam_matches_torch_adam():
         assert rel_err(m.detach().cpu(), r.detach()) < 1e-5
 
 
+def test_fused_adam_mixed_step_counts_matches_torch_adam():
+    """A parameter without a gradient for the first two steps lags two steps behind the others: FusedAdam then launches
+    kp_adam_multi once per step count.  Its size is not a multiple of 4, so the kernel's scalar tail runs too."""
+    from soccernerfs_b200 import ops
+    from soccernerfs_b200.engine.optimizers import FusedAdam
+
+    gen = torch.Generator().manual_seed(4)
+    shapes = [(1, 8, 13, 9), (64, 31), (37,), (1, 32, 16, 16)]
+    late = 2
+    ps = [torch.randn(s, generator=gen) for s in shapes]
+    mine = [torch.nn.Parameter(ops.as_channel_last(p.to(DEV)) if p.dim() == 4 else p.to(DEV)) for p in ps]
+    ref = [torch.nn.Parameter(p.clone()) for p in ps]
+    a, b = FusedAdam(mine, lr=1e-2, eps=1e-12), torch.optim.Adam(ref, lr=1e-2, eps=1e-12)
+    for it in range(5):
+        for i, (m, r) in enumerate(zip(mine, ref)):
+            if i == late and it < 2:
+                continue
+            gr = torch.randn(r.shape, generator=gen)
+            r.grad = gr.clone()
+            m.grad = torch.empty_like(m).copy_(gr.to(DEV))
+        a.step()
+        b.step()
+    assert [a.state[p]["step"] for p in mine] == [5, 5, 3, 5]
+    for m, r in zip(mine, ref):
+        assert rel_err(m.detach().cpu(), r.detach()) < 1e-5
+
+
+def test_adam_kernels_share_one_update_rule():
+    """kp_adam_multi, kp_plane_reg_adam with no regulariser term and both sharded kernels at world 1 (kp_peer_sharded_adam,
+    and kp_peer_sharded_adam_sparse with every line marked) give the same bits for the same p, g, m, v and grad_scale
+    (weight_decay 0, as in the presets)."""
+    from ctypes import byref, c_void_p, create_string_buffer
+
+    from soccernerfs_b200 import _lib, ops
+    from soccernerfs_b200.distributed import PeerArena, _RawCudaMemory
+
+    C, H, W = 32, 37, 29
+    n = C * H * W  # a multiple of 32 floats: the sparse kernel exchanges whole 128-byte lines
+    gen = torch.Generator().manual_seed(9)
+    p0, g0 = torch.randn(n, generator=gen).to(DEV), torch.randn(n, generator=gen).to(DEV)
+    m0, v0 = (0.1 * torch.randn(n, generator=gen)).to(DEV), (0.01 * torch.rand(n, generator=gen)).to(DEV)
+    lr, b1, b2, eps, wd, step, gs = 1e-2, 0.9, 0.999, 1e-12, 0.0, 7, 0.5
+
+    p, m, v = p0.clone(), m0.clone(), v0.clone()
+    ops.adam_multi_([p], [g0.clone()], [m], [v], lr, b1, b2, eps, wd, step, gs)
+    ref = (p, m, v)
+    assert not torch.equal(p, p0)
+    got = {}
+
+    def plane(t):  # channel-last [1,C,H,W] view of a flat buffer
+        return t.view(1, H, W, C).permute(0, 3, 1, 2)
+
+    p, m, v = p0.clone(), m0.clone(), v0.clone()
+    scratch = torch.empty(ops.plane_reg_adam_scratch_bytes([plane(p)]), dtype=torch.uint8, device=DEV)
+    coef = torch.rand(1, 4, generator=gen).to(DEV)  # unused: terms = 0 selects no regulariser
+    ops.plane_reg_adam_([plane(p)], [plane(g0.clone())], [plane(m)], [plane(v)], [0], coef, lr, b1, b2, eps, wd, step, gs,
+                        scratch, zero_grads=False)
+    got["plane_reg_adam"] = (p, m, v)
+
+    # one arena, data region = [gradients | parameters | touched marks]; at world 1 the barriers wait on the own flags only
+    own, handle = c_void_p(), create_string_buffer(64)
+    _lib.call("kp_peer_alloc", 3 * n * 4, byref(own), handle)
+    try:
+        data = torch.as_tensor(_RawCudaMemory(own.value + PeerArena.SIGNAL_BYTES, 3 * n), device=DEV)
+        arenas = (c_void_p * 1)(own.value)
+        for sparse in (False, True):
+            data[:n].copy_(g0)
+            data[n:2 * n].copy_(p0)
+            data[2 * n:].view(torch.uint8)[: n // 32].fill_(1)
+            m, v = m0.clone(), v0.clone()
+            name = "kp_peer_sharded_adam_sparse" if sparse else "kp_peer_sharded_adam"
+            offsets = (0, n, 2 * n) if sparse else (0, n)
+            _lib.call(name, arenas, 0, 1, *offsets, n, c_void_p(m.data_ptr()), c_void_p(v.data_ptr()), lr, b1, b2, eps, wd, step,
+                      gs, c_void_p(0), 0, _lib.stream_ptr())
+            got[name] = (data[n:2 * n].clone(), m, v)
+        torch.cuda.synchronize()
+    finally:
+        _lib.call("kp_peer_free", own)
+    for name, (p, m, v) in got.items():
+        assert torch.equal(p, ref[0]) and torch.equal(m, ref[1]) and torch.equal(v, ref[2]), name
+
+
 def test_eval_mode_and_chunked_full_frame():
     """Eval path: deterministic samplers, last_sample background, chunked get_outputs_for_camera_ray_bundle."""
     from soccernerfs_b200.cameras.rays import RayBundle
