@@ -63,6 +63,15 @@ typedef struct KpPoints {
 int kp_hexplane_fwd(const float* const* plane_ptrs, const int32_t* plane_hw, int n_scales, int n_planes,
                     int C, const KpPoints* points, int64_t M, int concat, uint32_t use_mask,
                     float* out /* [M, n_scales*C] (concat) or [M, C] */, void* stream);
+/* Forward only, dynamic fields (n_planes = 6; 3 is an error): out exactly as kp_hexplane_fwd writes it, bit for bit, from
+ * the same texel reads, and the dynamics score of every sample
+ *   T[k,c] = prod over the time planes XT, YT, ZT kept by use_mask of their bilinear interpolants (scale k, channel c),
+ *   delta  = 1/(n_scales*C) * sum_k sum_c |1 - T[k,c]|                                              (fp32 [M]),
+ * the per-sample form of sparse_transients_loss (NS/model_components/losses.py, kplanes_field.py:97-100 for the time
+ * planes' place in the Hadamard product of interpolate_kplanes, :77-126): 0 where the time planes are the identity. */
+int kp_hexplane_fwd_dyn(const float* const* plane_ptrs, const int32_t* plane_hw, int n_scales, int n_planes, int C,
+                        const KpPoints* points, int64_t M, int concat, uint32_t use_mask, float* out, float* delta /* [M] */,
+                        void* stream);
 /* grad_plane_ptrs: HOST array of device pointers (same order); entries may be NULL (frozen plane,
  * kplanes_field.py:102-110).  Gradients are ACCUMULATED (red.global.add) into the buffers. */
 int kp_hexplane_bwd(const float* const* plane_ptrs, float* const* grad_plane_ptrs, const int32_t* plane_hw,
@@ -348,6 +357,11 @@ int kp_image_metrics(const float* pred, const float* target, int B, int H, int W
 int64_t kp_compose_frame_scratch_bytes(int H, int W, int P);
 int kp_compose_frame(const float* const* panels, const int* kinds, int P, int H, int W, const float* accumulation,
                      const float* turbo, const float* viridis, void* scratch, uint8_t* out, void* stream);
+/* Same, each depth panel blended with its own accumulation: accumulations is a HOST array [P] of device pointers, entry p
+ * read only when kinds[p] is KP_PANEL_DEPTH (e.g. depth_static with accumulation_static beside depth with accumulation).
+ * kp_compose_frame is this call with its accumulation in every entry. */
+int kp_compose_frame_accs(const float* const* panels, const int* kinds, const float* const* accumulations, int P, int H,
+                          int W, const float* turbo, const float* viridis, void* scratch, uint8_t* out, void* stream);
 
 /* ---- baseline JPEG encoding of a composed frame (the image files and Motion-JPEG video of a rendered camera path):
  *      image uint8 [H, W, 3] RGB, 1 <= H, W <= 65535 -> out: one baseline JFIF file (SOF0, YCbCr 4:2:0, the Annex K.1

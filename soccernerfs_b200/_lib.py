@@ -36,6 +36,7 @@ SIGNATURES = {
     "kp_last_error": ([], c_char_p),
     "kp_launch_count": ([], ctypes.c_longlong),
     "kp_hexplane_fwd": ([_P, _P, c_int, c_int, c_int, POINTER(KpPoints), c_int64, c_int, c_uint32, _P, _P], c_int),
+    "kp_hexplane_fwd_dyn": ([_P, _P, c_int, c_int, c_int, POINTER(KpPoints), c_int64, c_int, c_uint32, _P, _P, _P], c_int),
     "kp_hexplane_bwd": ([_P, _P, _P, c_int, c_int, c_int, POINTER(KpPoints), c_int64, c_int, c_uint32, _P, _P], c_int),
     "kp_hexplane_bwd_flags": ([_P, _P, _P, _P, c_int, c_int, c_int, POINTER(KpPoints), c_int64, c_int, c_uint32, _P, _P], c_int),
     "kp_density_field_fwd": ([_P, _P, c_int, c_int, _P, _P, c_int, c_int, POINTER(KpPoints), c_int64, c_uint32, _P, _P], c_int),
@@ -81,6 +82,7 @@ SIGNATURES = {
     "kp_image_metrics": ([_P, _P, c_int, c_int, c_int, _P, _P, _P], c_int),
     "kp_compose_frame_scratch_bytes": ([c_int, c_int, c_int], c_int64),
     "kp_compose_frame": ([_P, POINTER(c_int), c_int, c_int, c_int, _P, _P, _P, _P, _P, _P], c_int),
+    "kp_compose_frame_accs": ([_P, POINTER(c_int), _P, c_int, c_int, c_int, _P, _P, _P, _P, _P], c_int),
     "kp_jpeg_encode_capacity": ([c_int, c_int], c_int64),
     "kp_jpeg_encode_scratch_bytes": ([c_int, c_int], c_int64),
     "kp_jpeg_header": ([c_int, c_int, c_int, _P], c_int),

@@ -33,6 +33,7 @@ constexpr int kMinMaxPerThread = 16;
 
 struct ComposeArgs {
   const float* panel[KP_COMPOSE_MAX_PANELS];
+  const float* acc[KP_COMPOSE_MAX_PANELS];  // the accumulation a depth panel is blended with, NULL for other kinds
   int kind[KP_COMPOSE_MAX_PANELS];
   int depth_slot[KP_COMPOSE_MAX_PANELS];  // index into the min / max partials, -1 for other kinds
 };
@@ -94,7 +95,7 @@ __device__ __forceinline__ int cmap_index(float v) {  // (int64)(v * 255), clamp
   return (int)fminf(fmaxf(s, 0.f), 255.f);
 }
 
-__global__ void __launch_bounds__(kComposeThreads) compose_frame_kernel(const __grid_constant__ ComposeArgs args, const float* __restrict__ acc, int H, int W,
+__global__ void __launch_bounds__(kComposeThreads) compose_frame_kernel(const __grid_constant__ ComposeArgs args, int H, int W,
                                                                         int P, int vec, const float* __restrict__ turbo,
                                                                         const float* __restrict__ viridis, const float2* __restrict__ part,
                                                                         int part_blocks, uint8_t* __restrict__ out) {
@@ -103,6 +104,7 @@ __global__ void __launch_bounds__(kComposeThreads) compose_frame_kernel(const __
   const int p = blockIdx.y;
   const int kind = args.kind[p];
   const float* src = args.panel[p];
+  const float* __restrict__ acc = args.acc[p];
   if (kind != KP_PANEL_COLOR) {
     const float* tab = kind == KP_PANEL_DEPTH ? turbo : viridis;
     for (int i = threadIdx.x; i < 256 * 3; i += kComposeThreads) s_tab[i] = __ldg(tab + i);
@@ -196,6 +198,46 @@ __global__ void __launch_bounds__(kComposeThreads) compose_frame_kernel(const __
   }
 }
 
+// accumulations: HOST array [P]; entry p is read for a depth panel p only
+static int compose_frame(const float* const* panels, const int* kinds, const float* const* accumulations, int P, int H, int W,
+                         const float* turbo, const float* viridis, void* scratch, uint8_t* out, void* stream) {
+  KP_CHECK(panels && kinds && accumulations && turbo && viridis && scratch && out, "compose_frame: NULL argument");
+  KP_CHECK(P >= 1 && P <= KP_COMPOSE_MAX_PANELS, "compose_frame: P=%d panels (1..%d)", P, KP_COMPOSE_MAX_PANELS);
+  KP_CHECK(H > 0 && W > 0, "compose_frame: H=%d W=%d", H, W);
+  const int64_t n = (int64_t)H * W;
+  KP_CHECK(ceil_div(n, 4 * (int64_t)kComposeThreads) <= 0x7fffffff, "compose_frame: %dx%d frame is too large", H, W);
+  ComposeArgs args;
+  int n_depth = 0;
+  bool vec = ((uintptr_t)out & 3) == 0;
+  for (int p = 0; p < KP_COMPOSE_MAX_PANELS; ++p) {
+    args.panel[p] = nullptr, args.acc[p] = nullptr, args.kind[p] = KP_PANEL_COLOR, args.depth_slot[p] = -1;
+    if (p >= P) continue;
+    KP_CHECK(panels[p], "compose_frame: panel %d is NULL", p);
+    KP_CHECK(kinds[p] == KP_PANEL_COLOR || kinds[p] == KP_PANEL_ACCUMULATION || kinds[p] == KP_PANEL_DEPTH,
+             "compose_frame: panel %d has kind %d (0 colour, 1 accumulation, 2 depth)", p, kinds[p]);
+    args.panel[p] = panels[p], args.kind[p] = kinds[p];
+    if (kinds[p] == KP_PANEL_DEPTH) {
+      KP_CHECK(accumulations[p], "compose_frame: depth panel %d needs an accumulation", p);
+      args.depth_slot[p] = n_depth++;
+      args.acc[p] = accumulations[p];
+      vec = vec && ((uintptr_t)accumulations[p] & 15) == 0;
+    }
+    vec = vec && ((uintptr_t)panels[p] & 15) == 0;
+  }
+  const int mm_blocks = minmax_blocks(n);
+  float2* part = static_cast<float2*>(scratch);
+  cudaStream_t st = as_stream(stream);
+  if (n_depth > 0) {
+    compose_minmax_kernel<<<dim3(mm_blocks, P), kComposeThreads, 0, st>>>(args, n, vec ? 1 : 0, part);
+    KP_LAUNCH_CHECK("compose_frame(minmax)");
+  }
+  const int blocks = (int)ceil_div(n, 4 * (int64_t)kComposeThreads);
+  compose_frame_kernel<<<dim3(blocks, P), kComposeThreads, 0, st>>>(args, H, W, P, vec ? 1 : 0, turbo, viridis, part, mm_blocks,
+                                                                     out);
+  KP_LAUNCH_CHECK("compose_frame");
+  return 0;
+}
+
 }  // namespace kp
 
 using namespace kp;
@@ -207,35 +249,13 @@ extern "C" int64_t kp_compose_frame_scratch_bytes(int H, int W, int P) {
 
 extern "C" int kp_compose_frame(const float* const* panels, const int* kinds, int P, int H, int W, const float* accumulation,
                                 const float* turbo, const float* viridis, void* scratch, uint8_t* out, void* stream) {
-  KP_CHECK(panels && kinds && turbo && viridis && scratch && out, "compose_frame: NULL argument");
-  KP_CHECK(P >= 1 && P <= KP_COMPOSE_MAX_PANELS, "compose_frame: P=%d panels (1..%d)", P, KP_COMPOSE_MAX_PANELS);
-  KP_CHECK(H > 0 && W > 0, "compose_frame: H=%d W=%d", H, W);
-  const int64_t n = (int64_t)H * W;
-  KP_CHECK(ceil_div(n, 4 * (int64_t)kComposeThreads) <= 0x7fffffff, "compose_frame: %dx%d frame is too large", H, W);
-  ComposeArgs args;
-  int n_depth = 0;
-  bool vec = ((uintptr_t)accumulation & 15) == 0 && ((uintptr_t)out & 3) == 0;
-  for (int p = 0; p < KP_COMPOSE_MAX_PANELS; ++p) {
-    args.panel[p] = nullptr, args.kind[p] = KP_PANEL_COLOR, args.depth_slot[p] = -1;
-    if (p >= P) continue;
-    KP_CHECK(panels[p], "compose_frame: panel %d is NULL", p);
-    KP_CHECK(kinds[p] == KP_PANEL_COLOR || kinds[p] == KP_PANEL_ACCUMULATION || kinds[p] == KP_PANEL_DEPTH,
-             "compose_frame: panel %d has kind %d (0 colour, 1 accumulation, 2 depth)", p, kinds[p]);
-    args.panel[p] = panels[p], args.kind[p] = kinds[p];
-    if (kinds[p] == KP_PANEL_DEPTH) args.depth_slot[p] = n_depth++;
-    vec = vec && ((uintptr_t)panels[p] & 15) == 0;
-  }
-  KP_CHECK(n_depth == 0 || accumulation, "compose_frame: a depth panel needs the accumulation");
-  const int mm_blocks = minmax_blocks(n);
-  float2* part = static_cast<float2*>(scratch);
-  cudaStream_t st = as_stream(stream);
-  if (n_depth > 0) {
-    compose_minmax_kernel<<<dim3(mm_blocks, P), kComposeThreads, 0, st>>>(args, n, vec ? 1 : 0, part);
-    KP_LAUNCH_CHECK("compose_frame(minmax)");
-  }
-  const int blocks = (int)ceil_div(n, 4 * (int64_t)kComposeThreads);
-  compose_frame_kernel<<<dim3(blocks, P), kComposeThreads, 0, st>>>(args, accumulation, H, W, P, vec ? 1 : 0, turbo, viridis, part,
-                                                                     mm_blocks, out);
-  KP_LAUNCH_CHECK("compose_frame");
-  return 0;
+  const float* accs[KP_COMPOSE_MAX_PANELS];
+  for (int p = 0; p < KP_COMPOSE_MAX_PANELS; ++p) accs[p] = accumulation;
+  return compose_frame(panels, kinds, accs, P, H, W, turbo, viridis, scratch, out, stream);
+}
+
+extern "C" int kp_compose_frame_accs(const float* const* panels, const int* kinds, const float* const* accumulations, int P,
+                                     int H, int W, const float* turbo, const float* viridis, void* scratch, uint8_t* out,
+                                     void* stream) {
+  return compose_frame(panels, kinds, accumulations, P, H, W, turbo, viridis, scratch, out, stream);
 }

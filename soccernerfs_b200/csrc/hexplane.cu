@@ -360,6 +360,179 @@ __global__ void __launch_bounds__(128, 3) hexplane_fwd_wide_kernel(const __grid_
 }
 
 // ---------------------------------------------------------------------------------------------------
+// Forward gather with the dynamics score (kp_hexplane_fwd_dyn), six planes: the two kernels above with, beside the feature
+// product, T = the product of the time planes' interpolants (the same values, multiplied in the same plane order; the
+// feature product's operations and bits are unchanged) and delta[m] = mean over scales and channels of |1 - T|.  Kept
+// apart from the kernels above so that their code stays exactly what it was.
+// ---------------------------------------------------------------------------------------------------
+__host__ __device__ constexpr bool is_time_plane(int p) { return p == 2 || p == 4 || p == 5; }  // XT, YT, ZT
+
+// delta = (sum of the LPS lanes' partial sums) / (K * C), written by the sample's first lane.  The lanes of a sample are
+// adjacent and leave the kernel together, so the shuffle's group is complete.
+template <int LPS>
+__device__ __forceinline__ void store_delta(float part, int lane_in_sample, int64_t m, int n_scales, int C, float* delta) {
+  static_assert(LPS >= 1 && LPS <= 16 && (LPS & (LPS - 1)) == 0, "lanes per sample: a power of two below the warp");
+  const unsigned group = ((1u << LPS) - 1u) << ((threadIdx.x & 31) & ~(LPS - 1));
+#pragma unroll
+  for (int o = LPS / 2; o > 0; o >>= 1) part += __shfl_xor_sync(group, part, o, LPS);
+  if (lane_in_sample == 0) delta[m] = __fdiv_rn(part, (float)(n_scales * C));
+}
+
+template <int C, bool STREAM>
+__global__ void __launch_bounds__(128, 4) hexplane_fwd_dyn_kernel(const __grid_constant__ FieldRef F,
+                                                                const __grid_constant__ KpPoints P, int64_t M,
+                                                                float* __restrict__ out, float* __restrict__ delta) {
+  constexpr int NP = 6, LPS = C / 4;
+  const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int64_t m = gt / LPS;
+  const int c4 = (int)(gt % LPS) * 4;
+  if (m >= M) return;
+  if (P.ray_tile > 1 && P.pts == nullptr) {
+    const int64_t n_rays = M / P.S, tile_sz = (int64_t)P.ray_tile * P.S;
+    const int64_t tile = m / tile_sz;
+    const int r = (int)(m - tile * tile_sz);
+    const int t_here = (int)min((int64_t)P.ray_tile, n_rays - tile * P.ray_tile);
+    m = (tile * P.ray_tile + r % t_here) * P.S + r / t_here;
+  }
+  float pt[4];
+  load_point(P, m, pt);
+  const int out_stride = F.concat ? F.n_scales * C : C;
+  const uint64_t pol = STREAM ? l2_policy_evict_first() : 0ull;
+  float4 total = make_float4(0.f, 0.f, 0.f, 0.f);
+  float dsum = 0.f;  // this lane's sum of |1 - T| over its channels and the scales
+  for (int k = 0; k < F.n_scales; ++k) {
+    Axis ax[4];
+    axes_setup(F, k, pt, ax);
+    Bilerp b[NP];
+    float4 v[NP][4];
+#pragma unroll
+    for (int p = 0; p < NP; ++p) {
+      const PlaneRef& pr = F.pl[k * KP_MAX_PLANES + p];
+      b[p] = bilerp_from_axes(ax[plane_ca<NP>(p)], ax[plane_cb<NP>(p)], pr.W);
+      if ((F.use_mask >> p) & 1u) {
+        const float* base = pr.p + c4;
+        if (STREAM && pr.stream) {
+          v[p][0] = ldg4_stream(base + (int64_t)b[p].o00 * C, pol);
+          v[p][1] = ldg4_stream(base + (int64_t)b[p].o01 * C, pol);
+          v[p][2] = ldg4_stream(base + (int64_t)b[p].o10 * C, pol);
+          v[p][3] = ldg4_stream(base + (int64_t)b[p].o11 * C, pol);
+        } else {
+          v[p][0] = ldg4(base + (int64_t)b[p].o00 * C);
+          v[p][1] = ldg4(base + (int64_t)b[p].o01 * C);
+          v[p][2] = ldg4(base + (int64_t)b[p].o10 * C);
+          v[p][3] = ldg4(base + (int64_t)b[p].o11 * C);
+        }
+      }
+    }
+    float4 acc = make_float4(1.f, 1.f, 1.f, 1.f), tp = acc;
+#pragma unroll
+    for (int p = 0; p < NP; ++p)
+      if ((F.use_mask >> p) & 1u) {
+        const float4 f = bilerp_combine(b[p], v[p][0], v[p][1], v[p][2], v[p][3]);
+        acc = mul4(acc, f);
+        if (is_time_plane(p)) tp = mul4(tp, f);
+      }
+    dsum += fabsf(1.f - tp.x) + fabsf(1.f - tp.y) + fabsf(1.f - tp.z) + fabsf(1.f - tp.w);
+    if (F.concat) {
+      *reinterpret_cast<float4*>(out + m * out_stride + k * C + c4) = acc;
+    } else {
+      total.x += acc.x; total.y += acc.y; total.z += acc.z; total.w += acc.w;
+    }
+  }
+  if (!F.concat) *reinterpret_cast<float4*>(out + m * out_stride + c4) = total;
+  store_delta<LPS>(dsum, c4 / 4, m, F.n_scales, C, delta);
+}
+
+template <bool STREAM>
+__global__ void __launch_bounds__(128, 3) hexplane_fwd_wide_dyn_kernel(const __grid_constant__ FieldRef F,
+                                                                     const __grid_constant__ KpPoints P, int64_t M,
+                                                                     float* __restrict__ out, float* __restrict__ delta) {
+  constexpr int NP = 6, C = 32, LPS = 4, G = 3;
+  const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int64_t m = gt / LPS;
+  const int c8 = (int)(gt % LPS) * 8;
+  if (m >= M) return;
+  if (P.ray_tile > 1 && P.pts == nullptr) {
+    const int64_t n_rays = M / P.S, tile_sz = (int64_t)P.ray_tile * P.S;
+    const int64_t tile = m / tile_sz;
+    const int r = (int)(m - tile * tile_sz);
+    const int t_here = (int)min((int64_t)P.ray_tile, n_rays - tile * P.ray_tile);
+    m = (tile * P.ray_tile + r % t_here) * P.S + r / t_here;
+  }
+  float pt[4];
+  load_point(P, m, pt);
+  const int out_stride = F.concat ? F.n_scales * C : C;
+  const uint64_t pol = STREAM ? l2_policy_evict_first() : 0ull;
+  float2 total[4] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
+  float dsum = 0.f;
+  for (int k = 0; k < F.n_scales; ++k) {
+    Axis ax[4];
+    axes_setup(F, k, pt, ax);
+    float2 acc[4] = {make_float2(1.f, 1.f), make_float2(1.f, 1.f), make_float2(1.f, 1.f), make_float2(1.f, 1.f)};
+    float2 tp[4] = {make_float2(1.f, 1.f), make_float2(1.f, 1.f), make_float2(1.f, 1.f), make_float2(1.f, 1.f)};
+#pragma unroll
+    for (int g0 = 0; g0 < NP; g0 += G) {
+      Bilerp b[G];
+      float8 v[G][4];
+#pragma unroll
+      for (int i = 0; i < G; ++i) {
+        const int p = g0 + i;
+        const PlaneRef& pr = F.pl[k * KP_MAX_PLANES + p];
+        b[i] = bilerp_from_axes(ax[plane_ca<NP>(p)], ax[plane_cb<NP>(p)], pr.W);
+        if ((F.use_mask >> p) & 1u) {
+          const float* base = pr.p + c8;
+          if (STREAM && pr.stream) {
+            v[i][0] = ldg8_stream(base + (int64_t)b[i].o00 * C, pol);
+            v[i][1] = ldg8_stream(base + (int64_t)b[i].o01 * C, pol);
+            v[i][2] = ldg8_stream(base + (int64_t)b[i].o10 * C, pol);
+            v[i][3] = ldg8_stream(base + (int64_t)b[i].o11 * C, pol);
+          } else {
+            v[i][0] = ldg8(base + (int64_t)b[i].o00 * C);
+            v[i][1] = ldg8(base + (int64_t)b[i].o01 * C);
+            v[i][2] = ldg8(base + (int64_t)b[i].o10 * C);
+            v[i][3] = ldg8(base + (int64_t)b[i].o11 * C);
+          }
+        }
+      }
+#pragma unroll
+      for (int i = 0; i < G; ++i) {
+        const int p = g0 + i;
+        if (!((F.use_mask >> p) & 1u)) continue;
+        const float2 w00 = dup2(b[i].w00), w01 = dup2(b[i].w01), w10 = dup2(b[i].w10), w11 = dup2(b[i].w11);
+        auto pair = [&](float2 x00, float2 x01, float2 x10, float2 x11) {  // bilerp_combine per channel pair
+          float2 r = __fmul2_rn(x00, w00);
+          r = __ffma2_rn(x01, w01, r);
+          r = __ffma2_rn(x10, w10, r);
+          return __ffma2_rn(x11, w11, r);
+        };
+        const float2 f[4] = {pair(lo2(v[i][0].a), lo2(v[i][1].a), lo2(v[i][2].a), lo2(v[i][3].a)),
+                             pair(hi2(v[i][0].a), hi2(v[i][1].a), hi2(v[i][2].a), hi2(v[i][3].a)),
+                             pair(lo2(v[i][0].b), lo2(v[i][1].b), lo2(v[i][2].b), lo2(v[i][3].b)),
+                             pair(hi2(v[i][0].b), hi2(v[i][1].b), hi2(v[i][2].b), hi2(v[i][3].b))};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          acc[q] = __fmul2_rn(acc[q], f[q]);
+          if (is_time_plane(p)) tp[q] = __fmul2_rn(tp[q], f[q]);
+        }
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < 4; ++q) dsum += fabsf(1.f - tp[q].x) + fabsf(1.f - tp[q].y);
+    if (F.concat) {
+      stg8(out + m * out_stride + k * C + c8, make_float4(acc[0].x, acc[0].y, acc[1].x, acc[1].y),
+           make_float4(acc[2].x, acc[2].y, acc[3].x, acc[3].y));
+    } else {
+#pragma unroll
+      for (int q = 0; q < 4; ++q) total[q] = __fadd2_rn(total[q], acc[q]);
+    }
+  }
+  if (!F.concat)
+    stg8(out + m * out_stride + c8, make_float4(total[0].x, total[0].y, total[1].x, total[1].y),
+         make_float4(total[2].x, total[2].y, total[3].x, total[3].y));
+  store_delta<LPS>(dsum, c8 / 8, m, F.n_scales, C, delta);
+}
+
+// ---------------------------------------------------------------------------------------------------
 // Backward scatter: d plane_p[corner] += w_corner * g * prod_{q != p} interp_q.
 // ---------------------------------------------------------------------------------------------------
 template <int C, int NP, bool STREAM>
@@ -748,9 +921,10 @@ __global__ void __launch_bounds__(128, 4) density_field_bwd_kernel(const __grid_
   for (int i = threadIdx.x; i < HIDDEN; i += blockDim.x) red_add_f32(grad_w2 + i, s_acc[HIDDEN * C + i]);
 }
 
+// delta != NULL (forward of a six-plane field): the dynamics-score kernels, chosen exactly as the plain forward kernels are
 template <int C>
 static int launch_hexplane(bool bwd, const FieldRef& F, const KpPoints& P, int64_t M, const float* grad_out, float* out,
-                           cudaStream_t st) {
+                           float* delta, cudaStream_t st) {
   constexpr int LPS = C / 4;
   const int64_t blocks = ceil_div(M * LPS, 128);
   if (blocks == 0) return 0;
@@ -770,7 +944,10 @@ static int launch_hexplane(bool bwd, const FieldRef& F, const KpPoints& P, int64
       for (int p = 0; p < F.n_planes; ++p) wide = wide && (reinterpret_cast<uintptr_t>(F.pl[k * KP_MAX_PLANES + p].p) & 31) == 0;
     if (wide) {
       const int64_t wb = ceil_div(M * 4, 128);
-      if (F.n_planes == 6) {
+      if (delta != nullptr) {
+        if (any_stream) hexplane_fwd_wide_dyn_kernel<true><<<(unsigned)wb, 128, 0, st>>>(F, P, M, out, delta);
+        else hexplane_fwd_wide_dyn_kernel<false><<<(unsigned)wb, 128, 0, st>>>(F, P, M, out, delta);
+      } else if (F.n_planes == 6) {
         if (any_stream) hexplane_fwd_wide_kernel<6, true><<<(unsigned)wb, 128, 0, st>>>(F, P, M, out);
         else hexplane_fwd_wide_kernel<6, false><<<(unsigned)wb, 128, 0, st>>>(F, P, M, out);
       } else {
@@ -780,7 +957,10 @@ static int launch_hexplane(bool bwd, const FieldRef& F, const KpPoints& P, int64
       return 0;
     }
   }
-  if (F.n_planes == 6) {
+  if (delta != nullptr) {
+    if (any_stream) hexplane_fwd_dyn_kernel<C, true><<<(unsigned)blocks, 128, 0, st>>>(F, P, M, out, delta);
+    else hexplane_fwd_dyn_kernel<C, false><<<(unsigned)blocks, 128, 0, st>>>(F, P, M, out, delta);
+  } else if (F.n_planes == 6) {
     if (any_stream) {
       if (!bwd) hexplane_fwd_kernel<C, 6, true><<<(unsigned)blocks, 128, 0, st>>>(F, P, M, out);
       else hexplane_bwd_kernel<C, 6, true><<<(unsigned)blocks, 128, 0, st>>>(F, P, M, grad_out);
@@ -797,13 +977,13 @@ static int launch_hexplane(bool bwd, const FieldRef& F, const KpPoints& P, int64
 }
 
 static int dispatch_hexplane(bool bwd, int C, const FieldRef& F, const KpPoints& P, int64_t M, const float* grad_out,
-                             float* out, cudaStream_t st) {
+                             float* out, float* delta, cudaStream_t st) {
   switch (C) {
-    case 4: return launch_hexplane<4>(bwd, F, P, M, grad_out, out, st);
-    case 8: return launch_hexplane<8>(bwd, F, P, M, grad_out, out, st);
-    case 16: return launch_hexplane<16>(bwd, F, P, M, grad_out, out, st);
-    case 32: return launch_hexplane<32>(bwd, F, P, M, grad_out, out, st);
-    case 64: return launch_hexplane<64>(bwd, F, P, M, grad_out, out, st);
+    case 4: return launch_hexplane<4>(bwd, F, P, M, grad_out, out, delta, st);
+    case 8: return launch_hexplane<8>(bwd, F, P, M, grad_out, out, delta, st);
+    case 16: return launch_hexplane<16>(bwd, F, P, M, grad_out, out, delta, st);
+    case 32: return launch_hexplane<32>(bwd, F, P, M, grad_out, out, delta, st);
+    case 64: return launch_hexplane<64>(bwd, F, P, M, grad_out, out, delta, st);
     default: set_error("hexplane: feature dim C=%d unsupported (4,8,16,32,64)", C); return 1;
   }
 }
@@ -831,7 +1011,18 @@ extern "C" int kp_hexplane_fwd(const float* const* plane_ptrs, const int32_t* pl
   KP_CHECK(out != nullptr || M == 0, "hexplane_fwd: out is NULL");
   FieldRef F;
   if (fill_field(F, plane_ptrs, nullptr, plane_hw, n_scales, n_planes, points->D, use_mask, concat, C)) return 1;
-  return dispatch_hexplane(false, C, F, *points, M, nullptr, out, as_stream(stream));
+  return dispatch_hexplane(false, C, F, *points, M, nullptr, out, nullptr, as_stream(stream));
+}
+
+extern "C" int kp_hexplane_fwd_dyn(const float* const* plane_ptrs, const int32_t* plane_hw, int n_scales, int n_planes,
+                                   int C, const KpPoints* points, int64_t M, int concat, uint32_t use_mask, float* out,
+                                   float* delta, void* stream) {
+  KP_CHECK(n_planes == 6, "hexplane_fwd_dyn: a static field (n_planes=%d) has no time planes", n_planes);
+  if (check_points(points, M)) return 1;
+  KP_CHECK((out != nullptr && delta != nullptr) || M == 0, "hexplane_fwd_dyn: out or delta is NULL");
+  FieldRef F;
+  if (fill_field(F, plane_ptrs, nullptr, plane_hw, n_scales, n_planes, points->D, use_mask, concat, C)) return 1;
+  return dispatch_hexplane(false, C, F, *points, M, nullptr, out, delta, as_stream(stream));
 }
 
 extern "C" int kp_hexplane_bwd_flags(const float* const* plane_ptrs, float* const* grad_plane_ptrs, uint8_t* const* touched_ptrs,
@@ -845,7 +1036,7 @@ extern "C" int kp_hexplane_bwd_flags(const float* const* plane_ptrs, float* cons
   if (touched_ptrs != nullptr)
     for (int k = 0; k < n_scales; ++k)
       for (int p = 0; p < n_planes; ++p) F.pl[k * KP_MAX_PLANES + p].f = touched_ptrs[k * n_planes + p];
-  return dispatch_hexplane(true, C, F, *points, M, grad_out, nullptr, as_stream(stream));
+  return dispatch_hexplane(true, C, F, *points, M, grad_out, nullptr, nullptr, as_stream(stream));
 }
 
 extern "C" int kp_hexplane_bwd(const float* const* plane_ptrs, float* const* grad_plane_ptrs, const int32_t* plane_hw,

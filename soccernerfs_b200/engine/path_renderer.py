@@ -31,7 +31,7 @@ from ..cameras.camera_paths import CropData, get_crop_from_json, get_path_from_j
 from ..cameras.cameras import Cameras
 from ..model_components.renderers import background_color_override_context
 from .evaluator import images_of_rank
-from .frame_renderer import FrameRenderer
+from .frame_renderer import STATIC_OUTPUTS, FrameRenderer
 
 RING_SLOTS = 3  # pinned host images in flight: one being filled by the copy, the others being encoded
 IMAGE_FORMATS = ("png", "jpeg")
@@ -48,9 +48,15 @@ def load_camera_path(path_or_dict: Union[str, os.PathLike, Dict]) -> Tuple[Camer
 
 
 def available_outputs(model) -> List[str]:
-    """The per-pixel outputs of the model that can be written as images."""
+    """The per-pixel outputs of the model that can be written as images.  A dynamic model (its field has time planes) also
+    has its space-time decomposition: the static scene (``rgb_static``, ``depth_static``, ``accumulation_static``: the
+    render with the time planes left out, models.base_model.static_scene) and ``dynamic``, how far the time planes move
+    the scene from it (models.base_model.dynamics_output)."""
     names = ["rgb", "depth", "accumulation", "median_rgb"]
-    return names + [f"prop_depth_{i}" for i in range(getattr(model.config, "num_proposal_iterations", 0))]
+    names += [f"prop_depth_{i}" for i in range(getattr(model.config, "num_proposal_iterations", 0))]
+    if getattr(model.field, "has_time_planes", False):
+        names += list(STATIC_OUTPUTS) + ["dynamic"]
+    return names
 
 
 def check_render_inputs(model, cameras: Cameras, rendered_output_names: Sequence[str]) -> None:
@@ -64,9 +70,10 @@ def check_render_inputs(model, cameras: Cameras, rendered_output_names: Sequence
         raise ValueError(f"unknown rendered output(s) {unknown}; available outputs: {available}")
     if len(names) > ops.COMPOSE_MAX_PANELS:
         raise ValueError(f"at most {ops.COMPOSE_MAX_PANELS} rendered outputs per frame (got {len(names)})")
-    if getattr(model.field, "has_time_planes", False) and cameras.times is None:
-        raise ValueError("the model is dynamic (its field has time planes) but the cameras have no times: every camera of "
-                         "the path needs a render_time")
+    timed = [n for n in names if n not in STATIC_OUTPUTS]  # the static render reads no time
+    if getattr(model.field, "has_time_planes", False) and cameras.times is None and timed:
+        raise ValueError(f"the model is dynamic (its field has time planes) but the cameras have no times: every camera of "
+                         f"the path needs a render_time for the outputs {timed}")
     sizes = sorted(set(zip(cameras._height_host, cameras._width_host)))
     if len(sizes) > 1:
         raise ValueError(f"the cameras' frames differ in size (H, W): {sizes}; one image size per path")
@@ -108,7 +115,10 @@ def _frame_loop(model, cameras: Cameras, names: List[str], rank: int, world: int
     dev = model.device
     if cameras.device != dev:
         cameras = cameras.to(dev)
-    outputs = names + (["accumulation"] if "accumulation" not in names and any(ops.panel_kind(n) == 2 for n in names) else [])
+    outputs = list(names)
+    for n in names:  # each depth panel is blended with its own accumulation
+        if ops.panel_kind(n) == 2 and ops.accumulation_of(n) not in outputs:
+            outputs.append(ops.accumulation_of(n))
     mine = images_of_rank(len(cameras), rank, world)
     aabb_box = None
     bg = None

@@ -88,6 +88,13 @@ class FusedMLP(nn.Module):
         self.activation, self.output_activation = activation, output_activation
 
 
+def _static_time(like: torch.Tensor) -> torch.Tensor:
+    """The time coordinate of every point of a static render (models.base_model.static_scene): a constant, 0, that the
+    masked-out time planes never read -- it only lets a dynamic field's points keep their four coordinates, with or
+    without the cameras' times."""
+    return torch.zeros(like.shape[:-1] + (1,), dtype=torch.float32, device=like.device)
+
+
 def _ray_form(ray_samples: RaySamples):
     """(origins [N,3], directions [N,3], starts [N,S], ends [N,S], times [N]|None) if the samples are the usual
     per-ray broadcast of a RayBundle (RayBundle.get_ray_samples), else None."""
@@ -129,7 +136,15 @@ class _AabbHostMixin:
 
 
 class KPlanesField(Field, _AabbHostMixin):
-    """Multiscale hexplane radiance field (kplanes_field.py:129-370)."""
+    """Multiscale hexplane radiance field (kplanes_field.py:129-370).
+
+    Inference modes, set by context managers of models.base_model: ``static_scene`` (the time planes are left out of
+    every feature product, as ``freeze_time_planes`` leaves them out, and the points carry a constant time) and
+    ``dynamics_output`` (``forward`` also returns "dynamic" [..., 1]: per sample the dynamics score of
+    ops.hexplane_features_dyn)."""
+
+    static_scene = False
+    dynamic_output = False
 
     def __init__(
         self,
@@ -198,9 +213,12 @@ class KPlanesField(Field, _AabbHostMixin):
 
     # -- helpers ---------------------------------------------------------------------------------------
     def _points(self, ray_samples: RaySamples) -> ops.Points:
+        static = self.static_scene and self.has_time_planes
         rf = _ray_form(ray_samples)
         if rf is not None:
             o, d, st, en, t = rf
+            if static:
+                t = _static_time(o)[:, 0]
             return ops.points_from_rays(o, d, st, en, t, self._aabb6(), norm_mode=2 if self._contract else 1,
                                         dynamic=self.has_time_planes and t is not None,
                                         ray_tile=0 if torch.is_grad_enabled() else int(getattr(self, "coherent_ray_tile", 0)))
@@ -209,7 +227,9 @@ class KPlanesField(Field, _AabbHostMixin):
             positions = self.spatial_distortion(positions) / 2.0  # from [-2, 2] to [-1, 1]
         else:
             positions = SceneBox.get_normalized_positions(positions, self.aabb) * 2.0 - 1.0
-        if self.has_time_planes and ray_samples.times is not None:
+        if static:
+            positions = torch.cat((positions, _static_time(positions)), dim=-1)
+        elif self.has_time_planes and ray_samples.times is not None:
             positions = torch.cat((positions, ray_samples.times * 2 - 1), dim=-1)
         return ops.points_from_pts(positions.reshape(-1, positions.shape[-1]))
 
@@ -219,18 +239,25 @@ class KPlanesField(Field, _AabbHostMixin):
             ms = [[p.detach() for p in g] for g in ms]
         return ms
 
-    # -- Field surface ---------------------------------------------------------------------------------
-    def get_density(self, ray_samples: RaySamples):
-        """-> (density [N,S,1], geometry features [M,15]).  kplanes_field.py:275-312."""
-        batch = ray_samples.frustums.shape
-        points = self._points(ray_samples)
+    def _features(self, points: ops.Points) -> torch.Tensor:
+        """The gather of get_density / _forward_fused; in dynamics_output mode also keeps the samples' dynamics scores
+        for ``forward`` (``_last_dynamic``)."""
         ms = self._planes()
         if points.D != (4 if len(ms[0]) == 6 else 3):
             raise RuntimeError("dynamic K-Planes field needs ray_samples.times")
         self._last_points = points  # (bench.py's per-scale probe re-runs the gather / scatter on the step's own samples)
-        feats = ops.hexplane_features(ms, points, self.concat_features_across_scales,
-                                      _use_mask(len(ms[0]), self.freeze_time_planes),
-                                      post_backward=getattr(self, "_kp_post_backward", None))
+        mask = _use_mask(len(ms[0]), self.freeze_time_planes or self.static_scene)
+        if self.dynamic_output and len(ms[0]) == 6 and not torch.is_grad_enabled():
+            feats, self._last_dynamic = ops.hexplane_features_dyn(ms, points, self.concat_features_across_scales, mask)
+            return feats
+        return ops.hexplane_features(ms, points, self.concat_features_across_scales, mask,
+                                     post_backward=getattr(self, "_kp_post_backward", None))
+
+    # -- Field surface ---------------------------------------------------------------------------------
+    def get_density(self, ray_samples: RaySamples):
+        """-> (density [N,S,1], geometry features [M,15]).  kplanes_field.py:275-312."""
+        batch = ray_samples.frustums.shape
+        feats = self._features(self._points(ray_samples))
         if self.linear_decoder:  # density = trunc_exp(linear(features)); the features themselves feed the colour basis
             density = ops.trunc_exp(ops.linear(feats, self.sigma_net.weights[0]))
             return density.view(*batch, 1), feats
@@ -315,12 +342,15 @@ class KPlanesField(Field, _AabbHostMixin):
         return rgb.view(*batch, 3)
 
     def forward(self, ray_samples: RaySamples, compute_normals: bool = False, mask=None, bg_color=None):
-        fused = self._forward_fused(ray_samples)
-        if fused is not None:
-            return fused
-        density, density_features = self.get_density(ray_samples)
-        rgb = self.get_outputs(ray_samples, density_features)
-        return {FieldHeadNames.DENSITY: density, FieldHeadNames.RGB: rgb}
+        self._last_dynamic = None
+        out = self._forward_fused(ray_samples)
+        if out is None:
+            density, density_features = self.get_density(ray_samples)
+            out = {FieldHeadNames.DENSITY: density, FieldHeadNames.RGB: self.get_outputs(ray_samples, density_features)}
+        if self._last_dynamic is not None:
+            out["dynamic"] = self._last_dynamic.view(*ray_samples.frustums.shape, 1)
+            self._last_dynamic = None
+        return out
 
     def _forward_fused(self, ray_samples: RaySamples):
         """get_density + get_outputs with both decoders in ONE tensor-core kernel (same numbers as the two-call path);
@@ -339,20 +369,16 @@ class KPlanesField(Field, _AabbHostMixin):
             if not (n_samples > 1 and d.stride(-2) == 0):
                 return None
             dirs = d[..., 0, :].reshape(-1, 3)
-        points = self._points(ray_samples)
-        ms = self._planes()
-        if points.D != (4 if len(ms[0]) == 6 else 3):
-            raise RuntimeError("dynamic K-Planes field needs ray_samples.times")
-        self._last_points = points  # (bench.py's per-scale probe re-runs the gather / scatter on the step's own samples)
-        feats = ops.hexplane_features(ms, points, self.concat_features_across_scales,
-                                      _use_mask(len(ms[0]), self.freeze_time_planes),
-                                      post_backward=getattr(self, "_kp_post_backward", None))
+        feats = self._features(self._points(ray_samples))
         _, density, rgb = ops.decoder_fused(feats, dirs, n_samples, w1, w2, w3, w4, w5)
         return {FieldHeadNames.DENSITY: density.view(*batch, 1), FieldHeadNames.RGB: rgb.view(*batch, 3)}
 
 
 class KPlanesDensityField(Field, _AabbHostMixin):
-    """Proposal density field (kplanes_field.py:373-463): one fused gather + 8->64->1 MLP + trunc_exp kernel."""
+    """Proposal density field (kplanes_field.py:373-463): one fused gather + 8->64->1 MLP + trunc_exp kernel.
+    ``static_scene``: as KPlanesField's (models.base_model.static_scene sets it on every proposal network too)."""
+
+    static_scene = False
 
     def __init__(self, aabb, resolution, feature_dim, spatial_distortion=None, linear_decoder: bool = True,
                  freeze_time_planes: bool = False, freeze_space_planes: bool = False) -> None:
@@ -388,9 +414,12 @@ class KPlanesDensityField(Field, _AabbHostMixin):
         """-> (density [N,S,1], None).  NOTE: positions are normalised to [0,1] only, not [-1,1], exactly like
         the reference (kplanes_field.py:439-440; SURVEY.md finding 3)."""
         batch = ray_samples.frustums.shape
+        static = self.static_scene and self.has_time_planes
         rf = _ray_form(ray_samples)
         if rf is not None:
             o, d, st, en, t = rf
+            if static:
+                t = _static_time(o)[:, 0]
             points = ops.points_from_rays(o, d, st, en, t, self._aabb6(), norm_mode=2 if self._contract else 0,
                                           dynamic=self.has_time_planes and t is not None)
         else:
@@ -399,7 +428,9 @@ class KPlanesDensityField(Field, _AabbHostMixin):
                 positions = self.spatial_distortion(positions) / 2.0  # from [-2, 2] to [-1, 1] (kplanes_field.py:436-438)
             else:
                 positions = SceneBox.get_normalized_positions(positions, self.aabb)
-            if self.has_time_planes and ray_samples.times is not None:
+            if static:
+                positions = torch.cat((positions, _static_time(positions)), dim=-1)
+            elif self.has_time_planes and ray_samples.times is not None:
                 positions = torch.cat((positions, ray_samples.times * 2 - 1), dim=-1)
             points = ops.points_from_pts(positions.reshape(-1, positions.shape[-1]))
         grids = _maybe_frozen(self.grids, self.freeze_space_planes)
@@ -408,7 +439,7 @@ class KPlanesDensityField(Field, _AabbHostMixin):
         if points.D != (4 if len(grids) == 6 else 3):
             raise RuntimeError("dynamic K-Planes density field needs times")
         density = ops.density_field(grids, self.sigma_net.weights[0], self.sigma_net.weights[1], points, relu=self.relu,
-                                    use_mask=_use_mask(len(grids), self.freeze_time_planes))
+                                    use_mask=_use_mask(len(grids), self.freeze_time_planes or self.static_scene))
         return density.view(*batch, 1), None
 
     def get_outputs(self, ray_samples: RaySamples, density_embedding: Optional[torch.Tensor] = None):

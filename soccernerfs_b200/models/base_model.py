@@ -67,6 +67,44 @@ def coherent_rays(model, tile: int = 4):
             field.coherent_ray_tile = old
 
 
+@contextlib.contextmanager
+def static_scene(model):
+    """Render the static part of a dynamic scene: inside, the model's field and every proposal network leave their time
+    planes (XT, YT, ZT) out of each feature product -- the space planes alone, which is the scene with its time planes
+    set to the identity 1 -- so the proposals place samples on the static scene too.  Time is not read: cameras need no
+    times, and their times do not change the result.  Inference only: raises while gradients are enabled.  Outside the
+    context nothing changes; a static model renders as it always does."""
+    if torch.is_grad_enabled():
+        raise RuntimeError("static_scene is an inference mode: use it under torch.no_grad()")
+    field = getattr(model, "field", None)
+    modules = ([field] if field is not None else []) + list(getattr(model, "proposal_networks", []))
+    old = [m.static_scene for m in modules]
+    for m in modules:
+        m.static_scene = True
+    try:
+        yield
+    finally:
+        for m, o in zip(modules, old):
+            m.static_scene = o
+
+
+@contextlib.contextmanager
+def dynamics_output(model, enabled: bool = True):
+    """Ask the model for its per-ray dynamics output ``dynamic`` [N, 1]: the final level's weights composite the
+    samples' dynamics scores, sum_i w_i delta_i, delta = mean over scales and channels of |1 - product of the time planes'
+    interpolants| (ops.hexplane_features_dyn); 0 where the time planes are the identity.  Inference only (the field
+    ignores it while gradients are enabled); no effect on the other outputs."""
+    field = getattr(model, "field", None)
+    old = getattr(field, "dynamic_output", False)
+    if field is not None:
+        field.dynamic_output = enabled
+    try:
+        yield
+    finally:
+        if field is not None:
+            field.dynamic_output = old
+
+
 class Model(nn.Module):
     config: ModelConfig
 

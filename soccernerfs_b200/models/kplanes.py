@@ -292,6 +292,8 @@ class KPlanesModel(Model):
             depth = self.renderer_depth(weights, ray_samples)
             median_rgb = self.medianrgb_renderer(rgb=field_out[FieldHeadNames.RGB], weights=weights)
             outputs = {"rgb": rgb, "accumulation": accumulation, "depth": depth, "median_rgb": median_rgb}
+            if "dynamic" in field_out:  # base_model.dynamics_output: composited like the accumulation, [N, 1]
+                outputs["dynamic"] = torch.sum(weights * field_out["dynamic"], dim=-2)
             if self.training:
                 outputs["weights_list"] = weights_list
                 outputs["ray_samples_list"] = ray_samples_list

@@ -202,6 +202,22 @@ def hexplane_features(ms_planes: Sequence[Sequence[torch.Tensor]], points: Point
     return _Hexplane.apply(points, len(ms_planes), concat, use_mask, post_backward, *flat)
 
 
+def hexplane_features_dyn(ms_planes: Sequence[Sequence[torch.Tensor]], points: Points, concat: bool,
+                          use_mask: int = 0x3F) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Inference only, dynamic fields: ``hexplane_features``' features (the same bits) and the dynamics score [M] of every
+    sample, 1/(K*C) * sum_k sum_c |1 - prod of the time planes' interpolants| (kp_hexplane_fwd_dyn).  No backward."""
+    if torch.is_grad_enabled() and any(p.requires_grad for grids in ms_planes for p in grids):
+        raise RuntimeError("hexplane_features_dyn has no backward: call it under torch.no_grad()")
+    planes = [as_channel_last(p.detach()) for grids in ms_planes for p in grids]
+    n_scales = len(ms_planes)
+    c, m = planes[0].shape[1], points.M
+    out = torch.empty((m, n_scales * c if concat else c), dtype=torch.float32, device=planes[0].device)
+    delta = torch.empty((m,), dtype=torch.float32, device=planes[0].device)
+    call("kp_hexplane_fwd_dyn", _plane_ptrs(planes), _plane_hw(planes), n_scales, len(planes) // n_scales, c, points.struct(), m,
+         int(concat), use_mask, ptr(out), ptr(delta), stream_ptr())
+    return out, delta
+
+
 # ------------------------------------------------------------------------------------------------
 # (a6) fused proposal density field
 # ------------------------------------------------------------------------------------------------
@@ -898,11 +914,17 @@ _COLORMAP_TABLES: Dict = {}
 
 
 def panel_kind(name: str) -> int:
-    """How ``compose_frame`` maps a rendered output: 1 = accumulation (viridis), 2 = a depth (turbo, blended with the
-    accumulation; ns-render's rule: any name containing "depth"), 0 = a colour shown as it is."""
-    if name == "accumulation":
+    """How ``compose_frame`` maps a rendered output: 1 = a scalar in [0, 1] through viridis (accumulation,
+    accumulation_static, the dynamics score ``dynamic``), 2 = a depth (turbo, blended with its accumulation; ns-render's
+    rule: any name containing "depth"), 0 = a colour shown as it is."""
+    if name in ("accumulation", "accumulation_static", "dynamic"):
         return 1
     return 2 if "depth" in name else 0
+
+
+def accumulation_of(name: str) -> str:
+    """The accumulation a depth panel is blended with: the static render's for ``depth_static``, else the frame's."""
+    return "accumulation_static" if name.endswith("_static") else "accumulation"
 
 
 def _colormap_tables(device) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -917,8 +939,9 @@ def _colormap_tables(device) -> Tuple[torch.Tensor, torch.Tensor]:
 def compose_frame(frames: Dict[str, torch.Tensor], names: Sequence[str]) -> torch.Tensor:
     """The outputs ``names`` of one rendered frame (fp32 CUDA [H,W,3] colours, [H,W,1] accumulation / depths) ->
     uint8 [H, W*len(names), 3], side by side in that order, colour-mapped as ``get_image_metrics_and_images`` maps them
-    (utils/colormaps.py; see ``panel_kind``) and quantised as floor(clamp(x, 0, 1) * 255 + 0.5) (kp_compose_frame).
-    A depth panel also needs ``frames["accumulation"]``.  On the current stream, no host synchronisation."""
+    (utils/colormaps.py; see ``panel_kind``) and quantised as floor(clamp(x, 0, 1) * 255 + 0.5) (kp_compose_frame_accs).
+    A depth panel also needs its accumulation (``accumulation_of``): ``frames["accumulation"]``, or
+    ``frames["accumulation_static"]`` for ``depth_static``.  On the current stream, no host synchronisation."""
     names = list(names)
     if not 1 <= len(names) <= COMPOSE_MAX_PANELS:
         raise ValueError(f"compose_frame: 1..{COMPOSE_MAX_PANELS} outputs per frame (got {len(names)})")
@@ -926,9 +949,10 @@ def compose_frame(frames: Dict[str, torch.Tensor], names: Sequence[str]) -> torc
     if missing:
         raise ValueError(f"compose_frame: {missing} not among the frame's outputs {sorted(frames)}")
     kinds = [panel_kind(n) for n in names]
-    acc = frames.get("accumulation") if 2 in kinds else None
-    if 2 in kinds and acc is None:
-        raise ValueError("compose_frame: a depth panel is blended with the accumulation, which the frame lacks")
+    acc_names = [accumulation_of(n) if k == 2 else None for n, k in zip(names, kinds)]
+    lacking = sorted({a for a in acc_names if a is not None and a not in frames})
+    if lacking:
+        raise ValueError(f"compose_frame: a depth panel is blended with its accumulation, which the frame lacks: {lacking}")
     first = frames[names[0]]
     h, w = first.shape[:2]
     panels = []
@@ -941,17 +965,21 @@ def compose_frame(frames: Dict[str, torch.Tensor], names: Sequence[str]) -> torc
         if not t.is_cuda or t.device != first.device:
             raise RuntimeError("compose_frame: the outputs must be CUDA tensors on one device (there is no CPU path)")
         panels.append(t.contiguous())
-    if acc is not None:
+    accs: Dict[str, torch.Tensor] = {}
+    for a in acc_names:
+        if a is None or a in accs:
+            continue
+        acc = frames[a]
         if tuple(acc.shape) != (h, w, 1) or acc.dtype != torch.float32 or acc.device != first.device:
-            raise ValueError(f"compose_frame: accumulation must be fp32 [{h},{w},1] on {first.device}")
-        acc = acc.contiguous()
+            raise ValueError(f"compose_frame: {a} must be fp32 [{h},{w},1] on {first.device}")
+        accs[a] = acc.contiguous()
     turbo, viridis = _colormap_tables(first.device)
     p = len(panels)
     out = torch.empty((h, w * p, 3), dtype=torch.uint8, device=first.device)
     scratch = torch.empty(int(_lib.load().kp_compose_frame_scratch_bytes(h, w, p)), dtype=torch.uint8, device=first.device)
     kind_arr = (c_int32 * p)(*kinds)
-    call("kp_compose_frame", _lib.ptr_array(panels), kind_arr, p, h, w, ptr(acc), ptr(turbo), ptr(viridis),
-         c_void_p(scratch.data_ptr()), c_void_p(out.data_ptr()), stream_ptr())
+    call("kp_compose_frame_accs", _lib.ptr_array(panels), kind_arr, _lib.ptr_array([accs.get(a) for a in acc_names]), p, h, w,
+         ptr(turbo), ptr(viridis), c_void_p(scratch.data_ptr()), c_void_p(out.data_ptr()), stream_ptr())
     return out
 
 
