@@ -338,6 +338,17 @@ int kp_loss_head_bwd(const float* pred, const float* image, int64_t N, const int
  *      graph-capturable. ---- */
 int64_t kp_image_metrics_scratch_bytes(int B, int H, int W);
 int kp_image_metrics(const float* pred, const float* target, int B, int H, int W, void* scratch, float* out, void* stream);
+/* The same metrics split by a region mask: mask uint8 [B,H,W], non-zero = the dynamic region; out fp32 [B,4] =
+ * (psnr_dynamic, ssim_dynamic, psnr_static, ssim_static), the static region being the complement of the mask.  PSNR of
+ * a region R: 10 log10(1 / mse_R), mse_R = the squared error summed (in double) over R's pixels and channels / (3 |R|).
+ * SSIM of R: the mean of kp_image_metrics' SSIM map over the interior windows whose centre pixel (y+5, x+5) lies in R,
+ * all 3 channels, with C1 / C2 from the whole image's data range.  A region without a pixel gets NaN for both, one
+ * without a window centre NaN for its SSIM.  An all-true (all-false) mask gives the dynamic (static) pair bit for bit
+ * equal to kp_image_metrics.  scratch: kp_image_metrics_masked_scratch_bytes(B, H, W) device bytes, 16-byte aligned.
+ * 3 launches, no host synchronisation, no float atomics, graph-capturable. */
+int64_t kp_image_metrics_masked_scratch_bytes(int B, int H, int W);
+int kp_image_metrics_masked(const float* pred, const float* target, const uint8_t* mask, int B, int H, int W, void* scratch,
+                            float* out, void* stream);
 
 /* ---- frame composition for a rendered camera path (the per-frame image work of ns-render, REF/nerfstudio/scripts/
  *      render.py: colour-map every requested output and concatenate them along the width): P <= KP_COMPOSE_MAX_PANELS

@@ -5,6 +5,7 @@ the torch restatement of PSNR + SSIM (utils/image_metrics.py) on the same frames
 
     python scripts/bench_eval.py                                                       # 1 GPU
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 scripts/bench_eval.py   # 8 GPUs (images i % 8 == rank)
+    python scripts/bench_eval.py --regions        # also the per-region metrics, the median masks, Evaluator(regions="median")
 
 Prints one JSON line (rank 0).  The eval targets are the model's own frames plus seeded noise: the metric values are
 not a quality statement, the times are the point.  Kernel timing: CUDA events around each pass, after warm-up, with a
@@ -92,6 +93,46 @@ def kernel_vs_torch(pred, target, reps: int) -> dict:
             "max_abs_diff_ssim": float((ours[:, 1] - ref[:, 1]).abs().max()), "l2_flush": "512 MB written before every pass"}
 
 
+def regions_timing(pred, target, cam_ids, reps: int) -> dict:
+    """--regions: median ms of ops.image_metrics_masked on the batch against ops.image_metrics and the torch
+    restatement (region_psnr_ssim, fp32), with L2 overwritten before every pass; and of median_dynamic_masks."""
+    from soccernerfs_b200 import ops
+    from soccernerfs_b200.engine.evaluator import median_dynamic_masks
+    from soccernerfs_b200.utils import image_metrics
+
+    flush = torch.empty(512 * 2**20 // 4, dtype=torch.float32, device=pred.device)
+
+    def timed(fn):
+        for _ in range(3):
+            fn()
+        times = []
+        for _ in range(reps):
+            flush.fill_(1.0)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            fn()
+            e1.record()
+            torch.cuda.synchronize()
+            times.append(e0.elapsed_time(e1))
+        return sorted(times)[len(times) // 2], times
+
+    mask = median_dynamic_masks(target, cam_ids)
+    ours = ops.image_metrics_masked(pred, target, mask).cpu()
+    ref = image_metrics.region_psnr_ssim(pred, target, mask).cpu()
+    whole = ops.image_metrics(pred, target).cpu()
+    m_ms, m_all = timed(lambda: ops.image_metrics_masked(pred, target, mask))
+    k_ms, k_all = timed(lambda: ops.image_metrics(pred, target))
+    t_ms, _ = timed(lambda: image_metrics.region_psnr_ssim(pred, target, mask))
+    d_ms, d_all = timed(lambda: median_dynamic_masks(target, cam_ids))
+    ok = ~ref.isnan()
+    return {"kp_image_metrics_masked_ms": m_ms, "kp_image_metrics_ms": k_ms, "masked_over_unmasked": m_ms / k_ms,
+            "torch_region_psnr_ssim_ms": t_ms, "median_dynamic_masks_ms": d_ms, "masked_ms_all": m_all,
+            "unmasked_ms_all": k_all, "median_masks_ms_all": d_all,
+            "dynamic_fraction": float(mask.float().mean()), "max_abs_diff_vs_torch": float((ours - ref).abs()[ok].max()),
+            "nan_pattern_equal": bool(torch.equal(ours.isnan(), ref.isnan())),
+            "whole": whole.tolist(), "regions": ours.tolist(), "l2_flush": "512 MB written before every pass"}
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--images", type=int, default=8)
@@ -100,6 +141,9 @@ def main() -> None:
     ap.add_argument("--repeats", type=int, default=3, help="timed calls of get_average_eval_image_metrics")
     ap.add_argument("--kernel-reps", type=int, default=20)
     ap.add_argument("--out", help="also write the JSON result to this file")
+    ap.add_argument("--regions", action="store_true",
+                    help="also time the per-region metrics (kp_image_metrics_masked, median_dynamic_masks) and the "
+                         'Evaluator with regions="median"')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_eval.py measures on a CUDA device; none is visible")
@@ -145,8 +189,29 @@ def main() -> None:
               "gpus": world, "card": card_info(local), "seconds_per_call": sorted(calls)[len(calls) // 2],
               "seconds_per_image": sorted(calls)[len(calls) // 2] / args.images, "seconds_per_call_all": calls,
               "results": res}
+    if args.regions:  # the eval images form one camera's clip: its median is the background the masks leave out
+        cams.ids = torch.zeros(args.images, dtype=torch.int64)
+        dm.eval_cameras.ids = cams.ids
+        t0 = time.perf_counter()
+        region_evaluator = Evaluator(model, dm, rank=rank, world=world, regions="median")
+        torch.cuda.synchronize()
+        construct = time.perf_counter() - t0
+        region_evaluator.get_average_eval_image_metrics(0)
+        region_calls = []
+        for r in range(args.repeats):
+            if world > 1:
+                torch.distributed.barrier()
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            region_res = region_evaluator.get_average_eval_image_metrics(r + 1)
+            region_calls.append(time.perf_counter() - t0)
+            torch.cuda.synchronize()
+        result["regions"] = {"evaluator_construct_s": construct, "seconds_per_call": sorted(region_calls)[len(region_calls) // 2],
+                             "seconds_per_call_all": region_calls, "results": region_res}
     if rank == 0:
         result["kernel"] = kernel_vs_torch(torch.stack(renders), targets, args.kernel_reps)
+        if args.regions:
+            result["regions"]["kernel"] = regions_timing(torch.stack(renders), targets, cams.ids, args.kernel_reps)
         line = json.dumps(result)
         print(line)
         if args.out:

@@ -80,6 +80,8 @@ SIGNATURES = {
     "kp_importance_pixels": ([_P, c_int, c_int64, c_int, _P, c_int, c_int, ctypes.c_uint64, _P, _P, _P], c_int),
     "kp_image_metrics_scratch_bytes": ([c_int, c_int, c_int], c_int64),
     "kp_image_metrics": ([_P, _P, c_int, c_int, c_int, _P, _P, _P], c_int),
+    "kp_image_metrics_masked_scratch_bytes": ([c_int, c_int, c_int], c_int64),
+    "kp_image_metrics_masked": ([_P, _P, _P, c_int, c_int, c_int, _P, _P, _P], c_int),
     "kp_compose_frame_scratch_bytes": ([c_int, c_int, c_int], c_int64),
     "kp_compose_frame": ([_P, POINTER(c_int), c_int, c_int, c_int, _P, _P, _P, _P, _P, _P], c_int),
     "kp_compose_frame_accs": ([_P, POINTER(c_int), _P, c_int, c_int, c_int, _P, _P, _P, _P, _P], c_int),

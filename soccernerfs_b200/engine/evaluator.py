@@ -7,15 +7,22 @@ tensors, and the PSNR / SSIM of all of a rank's images come from one ``ops.image
 instead of the torch restatement and its host synchronisations per image.  With ``world > 1`` rank r renders the images
 ``i % world == r``; one ``all_gather`` brings every image's row to every rank, and each key is averaged in image order,
 so the result does not depend on the world size.
+
+With ``regions`` the same images are also measured per region: ``ops.image_metrics_masked`` gives the PSNR / SSIM of a
+dynamic-region mask and of its complement (``psnr_dynamic`` ... ``ssim_static``).  The masks are the caller's, or
+``median_dynamic_masks`` of the eval images: the pixels that differ from their camera's per-pixel temporal median, which
+for a broadcast clip with moving players is the empty pitch.  These are not the reference's ``DynMetric`` (detector
+boxes), hence keys of their own rather than its ``dpsnr`` / ``dssim``.
 """
 from __future__ import annotations
 
-from typing import Any, Callable, Dict, List, Sequence, Tuple
+import math
+from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple, Union
 
 import torch
 
 from .. import ops
-from ..configs.method_configs import KPLANES_TRAINER
+from ..configs.method_configs import KPLANES_DATAMANAGER, KPLANES_TRAINER
 from ..utils import image_metrics
 from .frame_renderer import FrameRenderer
 
@@ -30,6 +37,46 @@ def average_metrics(rows: Dict[int, Dict[str, float]], keys: Sequence[str]) -> D
     (``float(torch.mean(torch.tensor([...])))``)."""
     order = sorted(rows)
     return {k: float(torch.mean(torch.tensor([rows[i][k] for i in order]))) for k in keys}
+
+
+REGION_KEYS = ("psnr_dynamic", "ssim_dynamic", "psnr_static", "ssim_static")
+
+
+def average_region_metrics(rows: Dict[int, Dict[str, float]], keys: Sequence[str]) -> Dict[str, float]:
+    """``average_metrics``, except that each of ``REGION_KEYS`` is averaged over the images where it is defined (not
+    NaN), still in image order; then ``num_images_dynamic`` / ``num_images_static``: the images whose region has a pixel
+    (an image whose region only touches the 5-pixel border has a PSNR but no SSIM)."""
+    order = sorted(rows)
+    out = {}
+    for k in keys:
+        vals = [rows[i][k] for i in order]
+        if k in REGION_KEYS:
+            vals = [v for v in vals if not math.isnan(v)]
+        out[k] = float(torch.mean(torch.tensor(vals)))
+    out["num_images_dynamic"] = sum(not math.isnan(rows[i]["psnr_dynamic"]) for i in order)
+    out["num_images_static"] = sum(not math.isnan(rows[i]["psnr_static"]) for i in order)
+    return out
+
+
+def median_dynamic_masks(images: torch.Tensor, cam_ids: Optional[torch.Tensor], gamma: float = KPLANES_DATAMANAGER.isg_gamma,
+                         threshold: float = 0.5) -> torch.Tensor:
+    """Dynamic-region masks of a clip, bool [B,H,W]: ``ops.isg_map(images, cam_ids, gamma) >= threshold``.
+
+    That map is the reference's ISG residual (``compute_isg``): per pixel the channel mean of the Geman-McClure distance
+    d^2 / (d^2 + gamma^2) of the frame from its camera's per-pixel temporal median.  Where the players move, the median
+    is the background, so the mask marks what differs from the background in this frame (the IST map would also mark
+    where the players were in neighbouring frames).  The policy: ``threshold`` 0.5 is the residual's midpoint, about
+    |d| >= gamma; ``gamma`` defaults to the preset's ``isg_gamma``.  images: fp32 CUDA [B,H,W,3]; cam_ids [B]: every
+    camera needs at least 3 images, since the median of 1 or 2 frames is not a background."""
+    if cam_ids is None:
+        raise ValueError("median_dynamic_masks: the cameras have no ids; the median is taken per camera")
+    ids = cam_ids.reshape(-1).cpu()
+    if ids.numel() != images.shape[0]:
+        raise ValueError(f"median_dynamic_masks: {ids.numel()} camera ids for {images.shape[0]} images")
+    for cam, n in zip(*(t.tolist() for t in torch.unique(ids, return_counts=True))):
+        if n < 3:
+            raise ValueError(f"median_dynamic_masks: camera {cam} has {n} image(s); its median needs at least 3")
+    return ops.isg_map(images, ids, gamma) >= threshold
 
 
 def pack_rows(rows: Dict[int, Dict[str, float]], keys: Sequence[str], n_rows: int) -> torch.Tensor:
@@ -60,13 +107,28 @@ def eval_report(results: Dict[str, float], experiment_name: str, checkpoint: str
 class Evaluator:
     """Eval metrics of ``model`` on the eval split of ``datamanager`` (a ``DynamicDataManager`` built with
     ``eval_cameras`` / ``eval_images``).  ``rank`` / ``world``: this process' share of ``get_average_eval_image_metrics``
-    (``torch.distributed`` must be initialised when ``world > 1``)."""
+    (``torch.distributed`` must be initialised when ``world > 1``).  ``regions``: None, ``"median"`` (the
+    ``median_dynamic_masks`` of the eval images and ``eval_cameras.ids``, computed here once) or a mask [B_eval,H,W]
+    (non-zero: dynamic), e.g. rasterised player boxes; with it the averages also carry the per-region metrics."""
 
-    def __init__(self, model, datamanager, rank: int = 0, world: int = 1) -> None:
+    regions: Optional[torch.Tensor] = None  # bool [B_eval,H,W] on the device
+
+    def __init__(self, model, datamanager, rank: int = 0, world: int = 1,
+                 regions: Union[None, str, torch.Tensor] = None) -> None:
         if datamanager.eval_cameras is None:
             raise ValueError("Evaluator: the datamanager has no eval split (eval_cameras / eval_images)")
         self.model, self.datamanager = model, datamanager
         self.rank, self.world = rank, world
+        if regions is not None:
+            images = datamanager.eval_image_cache.batch["image"]
+            if isinstance(regions, str):
+                if regions != "median":
+                    raise ValueError(f'Evaluator: regions must be None, "median" or a mask tensor (got {regions!r})')
+                self.regions = median_dynamic_masks(images, datamanager.eval_cameras.ids)
+            elif regions.shape != images.shape[:3]:
+                raise ValueError(f"Evaluator: regions must be [B_eval,H,W] = {tuple(images.shape[:3])} (got {tuple(regions.shape)})")
+            else:
+                self.regions = regions.to(images.device) != 0
         outputs = ["rgb", "depth", "accumulation", "median_rgb"]
         outputs += [f"prop_depth_{i}" for i in range(getattr(model.config, "num_proposal_iterations", 0))]
         # whole frames per rank: the renderer itself is not sharded
@@ -121,13 +183,20 @@ class Evaluator:
         return self._lpips
 
     def _rank_rows(self, mine: Sequence[int]) -> Dict[int, Dict[str, float]]:
-        """Per-image rows {psnr, ssim, [lpips], num_rays_per_sec, fps} of this rank's images."""
+        """Per-image rows {psnr, ssim, [lpips], num_rays_per_sec, fps, [REGION_KEYS, dynamic_fraction]} of this rank's
+        images."""
         if not mine:
             return {}
         renders = [self._render_timed(i) for i in mine]
         pred = torch.stack([rgb for rgb, _ in renders])
-        target = self.datamanager.eval_image_cache.batch["image"][torch.tensor(mine, device=pred.device)]
-        values = ops.image_metrics(pred, target).tolist()  # the one host synchronisation: the events have completed too
+        idx = torch.tensor(mine, device=pred.device)
+        target = self.datamanager.eval_image_cache.batch["image"][idx]
+        values = ops.image_metrics(pred, target)
+        if self.regions is not None:
+            mask = self.regions.to(pred.device)[idx]
+            fraction = mask.flatten(1).sum(1, dtype=torch.float64) / mask[0].numel()
+            values = torch.cat([values.double(), ops.image_metrics_masked(pred, target, mask).double(), fraction[:, None]], 1)
+        values = values.tolist()  # the one host synchronisation: the events have completed too
         lpips = self._lpips_metric(pred.device)
         rows = {}
         for k, i in enumerate(mine):
@@ -137,11 +206,14 @@ class Evaluator:
                 row["lpips"] = float(lpips(torch.moveaxis(target[k], -1, 0)[None], torch.moveaxis(pred[k], -1, 0)[None]))
             row["num_rays_per_sec"] = h * w / renders[k][1]()
             row["fps"] = row["num_rays_per_sec"] / (h * w)
+            if self.regions is not None:
+                row.update(zip(REGION_KEYS + ("dynamic_fraction",), values[k][2:]))
             rows[i] = row
         return rows
 
     def _keys(self, device) -> List[str]:
-        return ["psnr", "ssim"] + (["lpips"] if self._lpips_metric(device) is not None else []) + ["num_rays_per_sec", "fps"]
+        keys = ["psnr", "ssim"] + (["lpips"] if self._lpips_metric(device) is not None else []) + ["num_rays_per_sec", "fps"]
+        return keys if self.regions is None else keys + list(REGION_KEYS) + ["dynamic_fraction"]
 
     def _all_gather(self, rows: Dict[int, Dict[str, float]], keys: Sequence[str], n_images: int) -> Dict[int, Dict[str, float]]:
         import torch.distributed as dist
@@ -154,10 +226,12 @@ class Evaluator:
 
     def get_average_eval_image_metrics(self, step: int = 0) -> Dict[str, float]:
         """Every eval image: ``psnr``, ``ssim`` (and ``lpips`` when available), ``num_rays_per_sec`` and ``fps`` averaged
-        over the images (``VanillaPipeline.get_average_eval_image_metrics``)."""
+        over the images (``VanillaPipeline.get_average_eval_image_metrics``).  With ``regions``, then ``REGION_KEYS``,
+        ``dynamic_fraction`` (the mean share of dynamic pixels), ``num_images_dynamic`` and ``num_images_static``
+        (``average_region_metrics``)."""
         n = len(self.datamanager.eval_cameras)
         rows = self._rank_rows(images_of_rank(n, self.rank, self.world))
         keys = self._keys(self.datamanager.device)
         if self.world > 1:
             rows = self._all_gather(rows, keys, n)
-        return average_metrics(rows, keys)
+        return average_metrics(rows, keys) if self.regions is None else average_region_metrics(rows, keys)

@@ -909,6 +909,39 @@ def image_metrics(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def image_metrics_masked(pred: torch.Tensor, target: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
+    """Per-image (psnr_dynamic, ssim_dynamic, psnr_static, ssim_static) of a batch on the device
+    (kp_image_metrics_masked): pred, target fp32 CUDA [B,H,W,3] with H, W >= 11, mask bool or uint8 [B,H,W] (non-zero:
+    the dynamic region; the static region is the rest) -> fp32 [B,4].  Equal to ``utils.image_metrics.region_psnr_ssim``;
+    NaN for a region without a pixel (SSIM: without a window centre).  No host synchronisation, so it can be captured in
+    a CUDA graph."""
+    if pred.dim() != 4 or pred.shape[-1] != 3 or target.shape != pred.shape:
+        raise ValueError(f"image_metrics_masked: pred and target must both be [B,H,W,3] (got {tuple(pred.shape)}, "
+                         f"{tuple(target.shape)})")
+    if mask.shape != pred.shape[:3]:
+        raise ValueError(f"image_metrics_masked: mask must be [B,H,W] = {tuple(pred.shape[:3])} (got {tuple(mask.shape)})")
+    if pred.dtype != torch.float32 or target.dtype != torch.float32:
+        raise TypeError("image_metrics_masked: pred and target must be float32")
+    if mask.dtype not in (torch.bool, torch.uint8):
+        raise TypeError(f"image_metrics_masked: mask must be bool or uint8 (got {mask.dtype})")
+    if not pred.is_cuda or target.device != pred.device or mask.device != pred.device:
+        raise RuntimeError("image_metrics_masked: pred, target and mask must be CUDA tensors on one device (there is no CPU path)")
+    b, h, w = pred.shape[:3]
+    if h < 11 or w < 11:
+        raise ValueError(f"image_metrics_masked: {h}x{w} images are smaller than the 11x11 SSIM window")
+    pred, target = pred.contiguous(), target.contiguous()
+    mask = mask.contiguous()
+    if mask.dtype == torch.bool:
+        mask = mask.view(torch.uint8)  # one byte, 0 or 1
+    out = torch.empty((b, 4), dtype=torch.float32, device=pred.device)
+    if b == 0:
+        return out
+    scratch = torch.empty(int(_lib.load().kp_image_metrics_masked_scratch_bytes(b, h, w)), dtype=torch.uint8, device=pred.device)
+    call("kp_image_metrics_masked", ptr(pred), ptr(target), c_void_p(mask.data_ptr()), b, h, w, c_void_p(scratch.data_ptr()),
+         ptr(out), stream_ptr())
+    return out
+
+
 COMPOSE_MAX_PANELS = 8
 _COLORMAP_TABLES: Dict = {}
 

@@ -24,6 +24,14 @@ def ssim(preds: torch.Tensor, target: torch.Tensor, kernel_size: int = 11, sigma
          k2: float = 0.03, data_range: Optional[float] = None) -> torch.Tensor:
     """torchmetrics.functional.structural_similarity_index_measure defaults: [B,C,H,W] inputs, gaussian 11x11 window with
     sigma 1.5, reflect padding cropped from the result, data_range = max(range(preds), range(target)), mean over batch."""
+    full = ssim_map(preds, target, kernel_size, sigma, k1, k2, data_range)
+    return full.reshape(full.shape[0], -1).mean(-1).mean()
+
+
+def ssim_map(preds: torch.Tensor, target: torch.Tensor, kernel_size: int = 11, sigma: float = 1.5, k1: float = 0.01,
+             k2: float = 0.03, data_range: Optional[float] = None) -> torch.Tensor:
+    """The SSIM map ``ssim`` averages: [B,C,H-10,W-10] for the default window, entry (y, x) = the window centred on
+    pixel (y+5, x+5)."""
     if data_range is None:
         data_range = float(max(preds.max() - preds.min(), target.max() - target.min()))
     c1, c2 = (k1 * data_range) ** 2, (k2 * data_range) ** 2
@@ -41,8 +49,35 @@ def ssim(preds: torch.Tensor, target: torch.Tensor, kernel_size: int = 11, sigma
     mu_p, mu_t, pp, tt, pt = (out[i * b:(i + 1) * b] for i in range(5))
     sig_p, sig_t, sig_pt = pp - mu_p**2, tt - mu_t**2, pt - mu_p * mu_t
     full = ((2 * mu_p * mu_t + c1) * (2 * sig_pt + c2)) / ((mu_p**2 + mu_t**2 + c1) * (sig_p + sig_t + c2))
-    full = full[..., pad:-pad, pad:-pad]
-    return full.reshape(b, -1).mean(-1).mean()
+    return full[..., pad:-pad, pad:-pad]
+
+
+def region_psnr_ssim(pred: torch.Tensor, target: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
+    """Per-image PSNR and SSIM of a region and of its complement: pred, target [B,H,W,3] with H, W >= 11, mask [B,H,W]
+    (non-zero: the dynamic region) -> [B,4] = (psnr_dynamic, ssim_dynamic, psnr_static, ssim_static) in pred's dtype,
+    on pred's device.  The torch statement of ``ops.image_metrics_masked``:
+
+    - PSNR of a region R: 10 log10(1 / mse_R), mse_R the mean squared error over R's pixels and their 3 channels;
+    - SSIM of R: the mean of ``ssim_map`` (C1 / C2 from the whole image's data range) over the windows whose centre
+      pixel lies in R, all 3 channels;
+    - NaN for a region without a pixel, and for the SSIM of a region without a window centre (one that only touches the
+      5-pixel border)."""
+    if pred.dim() != 4 or pred.shape[-1] != 3 or target.shape != pred.shape or mask.shape != pred.shape[:3]:
+        raise ValueError(f"region_psnr_ssim: pred, target [B,H,W,3] and mask [B,H,W] (got {tuple(pred.shape)}, "
+                         f"{tuple(target.shape)}, {tuple(mask.shape)})")
+    b, h, w = mask.shape
+    if h < 11 or w < 11:
+        raise ValueError(f"region_psnr_ssim: {h}x{w} images are smaller than the 11x11 SSIM window")
+    out = torch.empty((b, 4), dtype=pred.dtype, device=pred.device)
+    for k in range(b):
+        p4, t4 = torch.moveaxis(pred[k], -1, 0)[None], torch.moveaxis(target[k], -1, 0)[None]
+        sq = (pred[k] - target[k]) ** 2
+        full = ssim_map(t4, p4)[0]  # the model's argument order, as get_image_metrics_and_images calls ssim
+        dyn = mask[k] != 0
+        for r, sel in enumerate((dyn, ~dyn)):
+            out[k, 2 * r] = 10.0 * torch.log10(1.0 / sq[sel].mean())
+            out[k, 2 * r + 1] = full[:, sel[5:h - 5, 5:w - 5]].mean()
+    return out
 
 
 def optional_lpips(device):
