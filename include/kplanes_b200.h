@@ -350,6 +350,24 @@ int64_t kp_image_metrics_masked_scratch_bytes(int B, int H, int W);
 int kp_image_metrics_masked(const float* pred, const float* target, const uint8_t* mask, int B, int H, int W, void* scratch,
                             float* out, void* stream);
 
+/* ---- eval depth metrics: rendered depth against ground-truth depth, per image and region.  pred, gt: fp32 [B,H,W]
+ *      (HW = H*W pixels per image); dir_norm: fp32 [B,H,W] or NULL; mask: uint8 [B,H,W] or NULL, non-zero = dynamic.
+ *      Ground truth g = __fmul_rn(gt, dir_norm) in fp32 when dir_norm is given (z-depth -> distance along the unit ray,
+ *      as depth_loss and get_image_metrics_and_images do for is_euclidean_depth=False), else g = gt.  A pixel is valid
+ *      when g is finite and g > 0 (0 / inf: sky and background).  In double: p = max(pred, 1e-6) (a NaN pred stays NaN),
+ *      e = p - g; over the valid pixels of a region, with n_valid of them:
+ *        abs_rel = mean |e| / g,  sq_rel = mean e^2 / g,  rmse = sqrt(mean e^2),  rmse_log = sqrt(mean (log p - log g)^2),
+ *        delta_k = the share with max(p / g, g / p) < 1.25^k, k = 1, 2, 3 (1.25, 1.5625, 1.953125: exact in binary).
+ *      out: double [B,R,8], row = (n_valid, abs_rel, sq_rel, rmse, rmse_log, delta1, delta2, delta3); n_valid = 0 gives
+ *      NaN for the other seven.  R = 1 (the whole image) without a mask, R = 3 (whole, dynamic, static = the complement)
+ *      with one.  Every region adds its pixels in the unmasked pass's order, so an all-true (all-false) mask gives the
+ *      dynamic (static) row bit for bit equal to the whole row and to the unmasked call.  Counts are integers, sums
+ *      doubles.  scratch: kp_depth_metrics_scratch_bytes(B, HW, mask != NULL) device bytes, 8-byte aligned.  2 launches,
+ *      no host synchronisation, no float atomics (bitwise reproducible), graph-capturable. ---- */
+int64_t kp_depth_metrics_scratch_bytes(int B, int64_t HW, int masked);
+int kp_depth_metrics(const float* pred, const float* gt, const float* dir_norm, const uint8_t* mask, int B, int64_t HW,
+                     void* scratch, double* out, void* stream);
+
 /* ---- frame composition for a rendered camera path (the per-frame image work of ns-render, REF/nerfstudio/scripts/
  *      render.py: colour-map every requested output and concatenate them along the width): P <= KP_COMPOSE_MAX_PANELS
  *      panels of one frame -> out uint8 [H, W*P, 3], panel p in columns [p*W, (p+1)*W).  panels: HOST array [P] of fp32

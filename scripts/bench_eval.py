@@ -6,6 +6,7 @@ the torch restatement of PSNR + SSIM (utils/image_metrics.py) on the same frames
     python scripts/bench_eval.py                                                       # 1 GPU
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 scripts/bench_eval.py   # 8 GPUs (images i % 8 == rank)
     python scripts/bench_eval.py --regions        # also the per-region metrics, the median masks, Evaluator(regions="median")
+    python scripts/bench_eval.py --depth          # also the depth metrics (kp_depth_metrics) and the Evaluator with eval depth
 
 Prints one JSON line (rank 0).  The eval targets are the model's own frames plus seeded noise: the metric values are
 not a quality statement, the times are the point.  Kernel timing: CUDA events around each pass, after warm-up, with a
@@ -133,6 +134,44 @@ def regions_timing(pred, target, cam_ids, reps: int) -> dict:
             "whole": whole.tolist(), "regions": ours.tolist(), "l2_flush": "512 MB written before every pass"}
 
 
+def depth_timing(depth, gt, norms, mask, reps: int) -> dict:
+    """--depth: median ms of ops.depth_metrics on the batch against the torch restatement (utils.image_metrics
+    .depth_metrics, float64 terms) and of the masked call against the unmasked one, with L2 overwritten before every
+    pass."""
+    from soccernerfs_b200 import ops
+    from soccernerfs_b200.utils import image_metrics
+
+    flush = torch.empty(512 * 2**20 // 4, dtype=torch.float32, device=depth.device)
+
+    def timed(fn):
+        for _ in range(3):
+            fn()
+        times = []
+        for _ in range(reps):
+            flush.fill_(1.0)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            fn()
+            e1.record()
+            torch.cuda.synchronize()
+            times.append(e0.elapsed_time(e1))
+        return sorted(times)[len(times) // 2], times
+
+    ours, ref = ops.depth_metrics(depth, gt, norms, mask).cpu(), image_metrics.depth_metrics(depth, gt, norms, mask).cpu()
+    k_ms, k_all = timed(lambda: ops.depth_metrics(depth, gt, norms))
+    m_ms, m_all = timed(lambda: ops.depth_metrics(depth, gt, norms, mask))
+    t_ms, _ = timed(lambda: image_metrics.depth_metrics(depth, gt, norms))
+    ok = ~ref.isnan()
+    rel = ((ours - ref).abs() / ref.abs())[..., 1:5][ok[..., 1:5]]
+    bytes_read = depth.numel() * 4 * 3  # pred, ground truth, directions_norm
+    return {"kp_depth_metrics_ms": k_ms, "kp_depth_metrics_masked_ms": m_ms, "masked_over_unmasked": m_ms / k_ms,
+            "torch_depth_metrics_ms": t_ms, "kp_ms_all": k_all, "masked_ms_all": m_all, "kp_bytes_read_min": bytes_read,
+            "kp_effective_gbs": bytes_read / (k_ms * 1e-3) / 1e9, "dynamic_fraction": float(mask.float().mean()),
+            "valid_fraction": float(ours[:, 0, 0].sum() / depth[0].numel() / depth.shape[0]),
+            "counts_and_deltas_equal_torch": bool(torch.equal(ours[..., [0, 5, 6, 7]].nan_to_num(), ref[..., [0, 5, 6, 7]].nan_to_num())),
+            "max_rel_diff_sums_vs_torch": float(rel.max()), "rows": ours.tolist(), "l2_flush": "512 MB written before every pass"}
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--images", type=int, default=8)
@@ -144,6 +183,9 @@ def main() -> None:
     ap.add_argument("--regions", action="store_true",
                     help="also time the per-region metrics (kp_image_metrics_masked, median_dynamic_masks) and the "
                          'Evaluator with regions="median"')
+    ap.add_argument("--depth", action="store_true",
+                    help="also time the depth metrics (kp_depth_metrics against torch, masked against unmasked) and the "
+                         "Evaluator with eval depth against the one without")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_eval.py measures on a CUDA device; none is visible")
@@ -159,15 +201,19 @@ def main() -> None:
     model.eval()
     cams = eval_cameras(args.images, args.height, args.width, dev)
     gen = torch.Generator(device=dev).manual_seed(7)
-    renders, frames = [], []
+    renders, frames, geometry = [], [], []
     with torch.no_grad():
         from soccernerfs_b200.engine.frame_renderer import FrameRenderer
 
-        renderer = FrameRenderer(model, cams)
+        renderer = FrameRenderer(model, cams, outputs=("rgb", "depth", "accumulation", "directions_norm") if args.depth
+                                 else ("rgb", "depth", "accumulation"))
         for i in range(args.images):  # every rank builds the same targets (same model, same seed)
-            f = renderer.render(i, device_frames=True)["rgb"]
+            out = renderer.render(i, device_frames=True)
+            f = out["rgb"]
             renders.append(f)
             frames.append((f + 0.03 * torch.randn(f.shape, generator=gen, device=dev)).clamp(0, 1))
+            if args.depth:
+                geometry.append((out["depth"], out["accumulation"], out["directions_norm"]))
         del renderer
     targets = torch.stack(frames)
     cfg = DynamicDataManagerConfig(use_importance_sampling=False)
@@ -208,8 +254,38 @@ def main() -> None:
             torch.cuda.synchronize()
         result["regions"] = {"evaluator_construct_s": construct, "seconds_per_call": sorted(region_calls)[len(region_calls) // 2],
                              "seconds_per_call_all": region_calls, "results": region_res}
+    if args.depth:  # ground-truth z-depth (the preset's convention): the rendered depth with 5 % noise, 0 where the
+        # frame accumulates less than half (background); the same evaluator with and without it, calls alternating
+        depth, acc, norms = (torch.stack(t)[..., 0] for t in zip(*geometry))
+        gt = depth / norms * torch.exp(0.05 * torch.randn(depth.shape, generator=gen, device=dev))
+        gt[acc < 0.5] = 0.0
+        model.config.is_euclidean_depth = False
+        depth_dm = DynamicDataManager(cfg, cams, targets, device=dev, eval_cameras=cams, eval_images=targets,
+                                      eval_extras={"depth_image": gt[..., None]})
+        depth_evaluator = Evaluator(model, depth_dm, rank=rank, world=world)
+        depth_evaluator.get_average_eval_image_metrics(0)
+        plain_calls, depth_calls = [], []
+        for r in range(args.repeats):
+            for ev_, calls_ in ((evaluator, plain_calls), (depth_evaluator, depth_calls)):
+                if world > 1:
+                    torch.distributed.barrier()
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                res_ = ev_.get_average_eval_image_metrics(r + 1)
+                calls_.append(time.perf_counter() - t0)
+                torch.cuda.synchronize()
+            depth_res = res_
+        result["depth"] = {"seconds_per_call": sorted(depth_calls)[len(depth_calls) // 2],
+                           "seconds_per_call_without_depth": sorted(plain_calls)[len(plain_calls) // 2],
+                           "seconds_per_call_all": depth_calls, "seconds_per_call_without_depth_all": plain_calls,
+                           "results": depth_res}
     if rank == 0:
         result["kernel"] = kernel_vs_torch(torch.stack(renders), targets, args.kernel_reps)
+        if args.depth:  # masks: the median masks of the 8 frames as one camera's clip, as --regions takes them
+            from soccernerfs_b200.engine.evaluator import median_dynamic_masks
+
+            mask = median_dynamic_masks(targets, torch.zeros(args.images, dtype=torch.int64))
+            result["depth"]["kernel"] = depth_timing(depth, gt, norms, mask, args.kernel_reps)
         if args.regions:
             result["regions"]["kernel"] = regions_timing(torch.stack(renders), targets, cams.ids, args.kernel_reps)
         line = json.dumps(result)

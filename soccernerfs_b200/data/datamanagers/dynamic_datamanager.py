@@ -125,14 +125,24 @@ class DynamicDataManager:
 
     def __init__(self, config: DynamicDataManagerConfig, cameras, images: torch.Tensor, device="cuda",
                  extras: Optional[Dict[str, torch.Tensor]] = None, prefetch: bool = False, eval_cameras=None,
-                 eval_images: Optional[torch.Tensor] = None, **sampler_kwargs: Any) -> None:
+                 eval_images: Optional[torch.Tensor] = None, eval_extras: Optional[Dict[str, torch.Tensor]] = None,
+                 **sampler_kwargs: Any) -> None:
         """``prefetch``: the batch ``next_train`` returns was produced on a side stream while the previous step ran, and
         the next one is enqueued there before returning -- the ~0.5 ms of sampler / gather / ray-generation kernels and
         their launch latencies leave the training stream (same batches in the same order as without it).
         ``eval_cameras`` / ``eval_images`` [B,H,W,3]: the eval split, cached on the device beside the train images (without
-        importance maps: eval batches are drawn uniformly)."""
+        importance maps: eval batches are drawn uniformly).  ``eval_extras``: per-pixel maps of the eval images, cached
+        with them as ``extras`` is with the train images; ``depth_image`` [B_eval,H,W,1] (ground-truth depth in the units
+        of the train ``depth_image``) travels with the ``next_eval`` pixels and ``next_eval_image``, and turns on the
+        ``Evaluator``'s depth metrics."""
         from ...model_components.ray_generators import RayGenerator
 
+        if eval_extras is not None and eval_images is None:
+            raise ValueError("eval_extras needs the eval split (eval_cameras and eval_images)")
+        depth = (eval_extras or {}).get("depth_image")
+        if depth is not None and tuple(depth.shape) != (*eval_images.shape[:3], 1):
+            raise ValueError(f"eval_extras['depth_image'] must be [B_eval,H,W,1] = {(*eval_images.shape[:3], 1)} "
+                             f"(got {tuple(depth.shape)})")
         self.config = config
         self.device = torch.device(device)
         self.cameras = cameras.to(self.device)
@@ -155,7 +165,8 @@ class DynamicDataManager:
             self.eval_cameras = eval_cameras.to(self.device)
             if len(self.eval_cameras) != eval_images.shape[0]:
                 raise ValueError(f"{eval_images.shape[0]} eval images for {len(self.eval_cameras)} eval cameras")
-            self.eval_image_cache = DeviceImageCache(eval_images, replace(config, use_importance_sampling=False), device=self.device)
+            self.eval_image_cache = DeviceImageCache(eval_images, replace(config, use_importance_sampling=False), device=self.device,
+                                                     extras=eval_extras)
             self.iter_eval_image_dataloader = iter(self.eval_image_cache)
             self.eval_pixel_sampler = PixelSampler(config.eval_num_rays_per_batch)
             self.eval_ray_generator = RayGenerator(self.eval_cameras)
@@ -213,8 +224,10 @@ class DynamicDataManager:
         return self.eval_ray_generator(batch["indices"]), batch
 
     def next_eval_image(self, step: int) -> Tuple[int, Dict[str, torch.Tensor]]:
-        """-> (camera index, {"image": [H,W,3] device tensor}) of a random eval image (``VanillaDataManager.next_eval_image``:
-        a random draw of the eval dataloader); render the camera with ``engine.frame_renderer.FrameRenderer``."""
+        """-> (camera index, {"image": [H,W,3] device tensor, and "depth_image": [H,W,1] when the eval split has one}) of a
+        random eval image (``VanillaDataManager.next_eval_image``: a random draw of the eval dataloader); render the camera
+        with ``engine.frame_renderer.FrameRenderer``."""
         self._need_eval()
         i = random.randrange(len(self.eval_cameras))
-        return i, {"image": self.eval_image_cache.batch["image"][i]}
+        batch = self.eval_image_cache.batch
+        return i, {k: batch[k][i] for k in ("image", "depth_image") if k in batch}

@@ -13,6 +13,11 @@ dynamic-region mask and of its complement (``psnr_dynamic`` ... ``ssim_static``)
 ``median_dynamic_masks`` of the eval images: the pixels that differ from their camera's per-pixel temporal median, which
 for a broadcast clip with moving players is the empty pitch.  These are not the reference's ``DynMetric`` (detector
 boxes), hence keys of their own rather than its ``dpsnr`` / ``dssim``.
+
+When the eval split carries ground-truth depth (``DynamicDataManager(eval_extras={"depth_image": ...})``), the rendered
+``depth`` frames of the same images go through one ``ops.depth_metrics`` call per rank (``depth_abs_rel`` ...
+``depth_delta3``, per region too with ``regions``): the geometry the preset's depth supervision trains, which colour
+metrics cannot tell apart from a flat billboard that looks right from near the training cameras.
 """
 from __future__ import annotations
 
@@ -55,6 +60,32 @@ def average_region_metrics(rows: Dict[int, Dict[str, float]], keys: Sequence[str
         out[k] = float(torch.mean(torch.tensor(vals)))
     out["num_images_dynamic"] = sum(not math.isnan(rows[i]["psnr_dynamic"]) for i in order)
     out["num_images_static"] = sum(not math.isnan(rows[i]["psnr_static"]) for i in order)
+    return out
+
+
+DEPTH_KEYS = ("depth_abs_rel", "depth_sq_rel", "depth_rmse", "depth_rmse_log", "depth_delta1", "depth_delta2", "depth_delta3")
+REGION_SUFFIXES = ("_dynamic", "_static")
+
+
+def depth_row_keys(regions: bool) -> List[str]:
+    """Per-image depth keys: ``DEPTH_KEYS`` (columns 1-7 of ``ops.depth_metrics``' whole-image row), then with regions
+    the same with ``_dynamic`` and with ``_static``."""
+    return list(DEPTH_KEYS) + ([k + s for s in REGION_SUFFIXES for k in DEPTH_KEYS] if regions else [])
+
+
+def average_depth_metrics(rows: Dict[int, Dict[str, float]], regions: bool) -> Dict[str, float]:
+    """Each of ``depth_row_keys(regions)`` averaged in image order over the images where it is defined (not NaN), with
+    ``num_images_depth`` (the images with a valid ground-truth pixel) after ``DEPTH_KEYS``; with regions
+    ``num_images_depth_dynamic`` / ``num_images_depth_static`` come last."""
+    order = sorted(rows)
+    out: Dict[str, float] = {}
+    for s in ("",) + (REGION_SUFFIXES if regions else ()):
+        for k in DEPTH_KEYS:
+            out[k + s] = float(torch.mean(torch.tensor([v for v in (rows[i][k + s] for i in order) if not math.isnan(v)])))
+        if not s:
+            out["num_images_depth"] = sum(not math.isnan(rows[i]["depth_abs_rel"]) for i in order)
+    for s in REGION_SUFFIXES if regions else ():
+        out["num_images_depth" + s] = sum(not math.isnan(rows[i]["depth_abs_rel" + s]) for i in order)
     return out
 
 
@@ -109,9 +140,11 @@ class Evaluator:
     ``eval_cameras`` / ``eval_images``).  ``rank`` / ``world``: this process' share of ``get_average_eval_image_metrics``
     (``torch.distributed`` must be initialised when ``world > 1``).  ``regions``: None, ``"median"`` (the
     ``median_dynamic_masks`` of the eval images and ``eval_cameras.ids``, computed here once) or a mask [B_eval,H,W]
-    (non-zero: dynamic), e.g. rasterised player boxes; with it the averages also carry the per-region metrics."""
+    (non-zero: dynamic), e.g. rasterised player boxes; with it the averages also carry the per-region metrics.  When the
+    eval image cache holds a ``depth_image``, the averages also carry the depth metrics (``average_depth_metrics``)."""
 
     regions: Optional[torch.Tensor] = None  # bool [B_eval,H,W] on the device
+    depth: bool = False  # the eval split has ground-truth depth
 
     def __init__(self, model, datamanager, rank: int = 0, world: int = 1,
                  regions: Union[None, str, torch.Tensor] = None) -> None:
@@ -129,8 +162,11 @@ class Evaluator:
                 raise ValueError(f"Evaluator: regions must be [B_eval,H,W] = {tuple(images.shape[:3])} (got {tuple(regions.shape)})")
             else:
                 self.regions = regions.to(images.device) != 0
+        self.depth = "depth_image" in datamanager.eval_image_cache.batch
         outputs = ["rgb", "depth", "accumulation", "median_rgb"]
         outputs += [f"prop_depth_{i}" for i in range(getattr(model.config, "num_proposal_iterations", 0))]
+        if self.depth and not getattr(model.config, "is_euclidean_depth", True):
+            outputs.append("directions_norm")  # the ground truth is z-depth: compared along the unit ray
         # whole frames per rank: the renderer itself is not sharded
         self.renderer = FrameRenderer(model, datamanager.eval_cameras, outputs=outputs)
         self._warm: set = set()
@@ -165,16 +201,18 @@ class Evaluator:
         metrics_dict["num_rays"] = h * w
         return metrics_dict, images_dict
 
-    def _render_timed(self, i: int) -> Tuple[torch.Tensor, Callable[[], float]]:
-        """-> (rgb [H,W,3] on the device, seconds of the render: call once the stream has passed the render)."""
+    def _render_timed(self, i: int, depth: bool = False) -> Tuple[Union[torch.Tensor, Callable[[], float], None], ...]:
+        """-> (rgb [H,W,3] on the device, seconds of the render: call once the stream has passed the render); with
+        ``depth`` then also the frame's depth [H,W,1] and its directions_norm [H,W,1] (None when not rendered)."""
         if self._size(i) not in self._warm:  # the first frame of a size captures the tile graphs: not part of the time
             self.renderer.render(i, device_frames=True)
             self._warm.add(self._size(i))
         start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record()
-        rgb = self.renderer.render(i, device_frames=True)["rgb"]
+        out = self.renderer.render(i, device_frames=True)
         end.record()
-        return rgb, lambda: start.elapsed_time(end) / 1e3
+        timed = (out["rgb"], lambda: start.elapsed_time(end) / 1e3)
+        return timed + (out["depth"], out.get("directions_norm")) if depth else timed
 
     def _lpips_metric(self, device):
         if not self._lpips_checked:  # the model's rule: LPIPS only when its pretrained network is available
@@ -183,20 +221,27 @@ class Evaluator:
         return self._lpips
 
     def _rank_rows(self, mine: Sequence[int]) -> Dict[int, Dict[str, float]]:
-        """Per-image rows {psnr, ssim, [lpips], num_rays_per_sec, fps, [REGION_KEYS, dynamic_fraction]} of this rank's
-        images."""
+        """Per-image rows {psnr, ssim, [lpips], num_rays_per_sec, fps, [REGION_KEYS, dynamic_fraction],
+        [depth_row_keys]} of this rank's images."""
         if not mine:
             return {}
-        renders = [self._render_timed(i) for i in mine]
-        pred = torch.stack([rgb for rgb, _ in renders])
+        renders = [self._render_timed(i, depth=True) if self.depth else self._render_timed(i) for i in mine]
+        pred = torch.stack([r[0] for r in renders])
         idx = torch.tensor(mine, device=pred.device)
         target = self.datamanager.eval_image_cache.batch["image"][idx]
         values = ops.image_metrics(pred, target)
+        mask = None
         if self.regions is not None:
             mask = self.regions.to(pred.device)[idx]
             fraction = mask.flatten(1).sum(1, dtype=torch.float64) / mask[0].numel()
             values = torch.cat([values.double(), ops.image_metrics_masked(pred, target, mask).double(), fraction[:, None]], 1)
+        if self.depth:
+            norms = [r[3] for r in renders]
+            depth = ops.depth_metrics(torch.stack([r[2] for r in renders]), self.datamanager.eval_image_cache.batch["depth_image"][idx],
+                                      None if norms[0] is None else torch.stack(norms), mask)
+            values = torch.cat([values.double(), depth[:, :, 1:].flatten(1)], 1)  # (n_valid dropped: NaN marks "undefined")
         values = values.tolist()  # the one host synchronisation: the events have completed too
+        n_colour = 2 if self.regions is None else 7
         lpips = self._lpips_metric(pred.device)
         rows = {}
         for k, i in enumerate(mine):
@@ -207,13 +252,16 @@ class Evaluator:
             row["num_rays_per_sec"] = h * w / renders[k][1]()
             row["fps"] = row["num_rays_per_sec"] / (h * w)
             if self.regions is not None:
-                row.update(zip(REGION_KEYS + ("dynamic_fraction",), values[k][2:]))
+                row.update(zip(REGION_KEYS + ("dynamic_fraction",), values[k][2:n_colour]))
+            if self.depth:
+                row.update(zip(depth_row_keys(self.regions is not None), values[k][n_colour:]))
             rows[i] = row
         return rows
 
     def _keys(self, device) -> List[str]:
         keys = ["psnr", "ssim"] + (["lpips"] if self._lpips_metric(device) is not None else []) + ["num_rays_per_sec", "fps"]
-        return keys if self.regions is None else keys + list(REGION_KEYS) + ["dynamic_fraction"]
+        keys = keys if self.regions is None else keys + list(REGION_KEYS) + ["dynamic_fraction"]
+        return keys + depth_row_keys(self.regions is not None) if self.depth else keys
 
     def _all_gather(self, rows: Dict[int, Dict[str, float]], keys: Sequence[str], n_images: int) -> Dict[int, Dict[str, float]]:
         import torch.distributed as dist
@@ -228,10 +276,14 @@ class Evaluator:
         """Every eval image: ``psnr``, ``ssim`` (and ``lpips`` when available), ``num_rays_per_sec`` and ``fps`` averaged
         over the images (``VanillaPipeline.get_average_eval_image_metrics``).  With ``regions``, then ``REGION_KEYS``,
         ``dynamic_fraction`` (the mean share of dynamic pixels), ``num_images_dynamic`` and ``num_images_static``
-        (``average_region_metrics``)."""
+        (``average_region_metrics``).  With eval depth, then the depth keys (``average_depth_metrics``)."""
         n = len(self.datamanager.eval_cameras)
         rows = self._rank_rows(images_of_rank(n, self.rank, self.world))
         keys = self._keys(self.datamanager.device)
         if self.world > 1:
             rows = self._all_gather(rows, keys, n)
-        return average_metrics(rows, keys) if self.regions is None else average_region_metrics(rows, keys)
+        colour = keys[:len(keys) - len(depth_row_keys(self.regions is not None))] if self.depth else keys
+        out = average_metrics(rows, colour) if self.regions is None else average_region_metrics(rows, colour)
+        if self.depth:
+            out.update(average_depth_metrics(rows, self.regions is not None))
+        return out

@@ -942,6 +942,51 @@ def image_metrics_masked(pred: torch.Tensor, target: torch.Tensor, mask: torch.T
     return out
 
 
+def depth_metrics(pred: torch.Tensor, gt: torch.Tensor, directions_norm: Optional[torch.Tensor] = None,
+                  mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Per-image depth error of rendered depth against ground truth on the device (kp_depth_metrics): pred, gt and
+    ``directions_norm`` fp32 CUDA [B,H,W] or [B,H,W,1], mask bool or uint8 [B,H,W] (non-zero: the dynamic region) ->
+    float64 [B,R,8], row = (n_valid, abs_rel, sq_rel, rmse, rmse_log, delta1, delta2, delta3); R = 1 (whole image)
+    without a mask, 3 (whole, dynamic, static) with one.  With ``directions_norm`` the ground truth is z-depth and is
+    compared as gt * directions_norm (``is_euclidean_depth=False``).  Equal to ``utils.image_metrics.depth_metrics``;
+    NaN for a region without a valid pixel.  No host synchronisation, so it can be captured in a CUDA graph."""
+    maps = {"pred": pred, "gt": gt, "directions_norm": directions_norm}
+    for name, t in maps.items():
+        if t is not None and t.dim() == 4 and t.shape[-1] == 1:
+            maps[name] = t = t.squeeze(-1)
+        if t is not None and t.dim() != 3:
+            raise ValueError(f"depth_metrics: {name} must be [B,H,W] or [B,H,W,1] (got {tuple(t.shape)})")
+    pred, gt, directions_norm = maps["pred"], maps["gt"], maps["directions_norm"]
+    if gt.shape != pred.shape or (directions_norm is not None and directions_norm.shape != pred.shape):
+        raise ValueError(f"depth_metrics: pred, gt and directions_norm must have one shape (got {tuple(pred.shape)}, "
+                         f"{tuple(gt.shape)}, {None if directions_norm is None else tuple(directions_norm.shape)})")
+    if mask is not None and mask.shape != pred.shape:
+        raise ValueError(f"depth_metrics: mask must be [B,H,W] = {tuple(pred.shape)} (got {tuple(mask.shape)})")
+    b, h, w = pred.shape
+    if h * w == 0:
+        raise ValueError(f"depth_metrics: {h}x{w} images have no pixel")
+    if any(t is not None and t.dtype != torch.float32 for t in (pred, gt, directions_norm)):
+        raise TypeError("depth_metrics: pred, gt and directions_norm must be float32")
+    if mask is not None and mask.dtype not in (torch.bool, torch.uint8):
+        raise TypeError(f"depth_metrics: mask must be bool or uint8 (got {mask.dtype})")
+    if not pred.is_cuda or any(t is not None and t.device != pred.device for t in (gt, directions_norm, mask)):
+        raise RuntimeError("depth_metrics: every tensor must be a CUDA tensor on one device (there is no CPU path)")
+    pred, gt = pred.contiguous(), gt.contiguous()
+    directions_norm = None if directions_norm is None else directions_norm.contiguous()
+    if mask is not None:
+        mask = mask.contiguous()
+        if mask.dtype == torch.bool:
+            mask = mask.view(torch.uint8)  # one byte, 0 or 1
+    out = torch.empty((b, 1 if mask is None else 3, 8), dtype=torch.float64, device=pred.device)
+    if b == 0:
+        return out
+    scratch = torch.empty(int(_lib.load().kp_depth_metrics_scratch_bytes(b, h * w, int(mask is not None))), dtype=torch.uint8,
+                          device=pred.device)
+    call("kp_depth_metrics", ptr(pred), ptr(gt), ptr(directions_norm), c_void_p(0 if mask is None else mask.data_ptr()), b,
+         h * w, c_void_p(scratch.data_ptr()), ptr(out), stream_ptr())
+    return out
+
+
 COMPOSE_MAX_PANELS = 8
 _COLORMAP_TABLES: Dict = {}
 

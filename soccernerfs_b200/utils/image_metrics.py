@@ -80,6 +80,56 @@ def region_psnr_ssim(pred: torch.Tensor, target: torch.Tensor, mask: torch.Tenso
     return out
 
 
+DELTA_THRESHOLDS = (1.25, 1.5625, 1.953125)  # 1.25 ** k, k = 1, 2, 3: exact in binary
+
+
+def depth_metrics(pred: torch.Tensor, gt: torch.Tensor, directions_norm: Optional[torch.Tensor] = None,
+                  mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Per-image depth error of rendered depth against ground truth: pred, gt, directions_norm [B,H,W] or [B,H,W,1], mask
+    [B,H,W] (non-zero: the dynamic region) -> float64 [B,R,8] on pred's device, row = (n_valid, abs_rel, sq_rel, rmse,
+    rmse_log, delta1, delta2, delta3); R = 1 (whole image) without a mask, 3 (whole, dynamic, static) with one.  The torch
+    statement of ``ops.depth_metrics``:
+
+    - ground truth g = gt * directions_norm in the inputs' dtype (z-depth to distance along the unit ray, as
+      ``depth_loss`` does for ``is_euclidean_depth=False``), or gt without ``directions_norm``;
+    - a pixel is valid where g is finite and > 0 (sky / background: 0 or inf);
+    - in float64, p = max(pred, 1e-6), e = p - g over a region's valid pixels: abs_rel = mean |e| / g, sq_rel =
+      mean e^2 / g, rmse = sqrt(mean e^2), rmse_log = sqrt(mean (log p - log g)^2), delta_k = the share of
+      max(p / g, g / p) < 1.25^k;
+    - n_valid = 0 and NaN for the other seven in a region without a valid pixel."""
+    pred, gt = (t.squeeze(-1) if t.dim() == 4 and t.shape[-1] == 1 else t for t in (pred, gt))
+    if directions_norm is not None and directions_norm.dim() == 4 and directions_norm.shape[-1] == 1:
+        directions_norm = directions_norm.squeeze(-1)
+    if (pred.dim() != 3 or gt.shape != pred.shape or (directions_norm is not None and directions_norm.shape != pred.shape)
+            or (mask is not None and mask.shape != pred.shape)):
+        raise ValueError(f"depth_metrics: pred, gt, directions_norm and mask must be [B,H,W] (got {tuple(pred.shape)}, "
+                         f"{tuple(gt.shape)}, {None if directions_norm is None else tuple(directions_norm.shape)}, "
+                         f"{None if mask is None else tuple(mask.shape)})")
+    g = gt if directions_norm is None else gt * directions_norm
+    valid = torch.isfinite(g) & (g > 0)
+    p, g = pred.double().clamp_min(1e-6), g.double()
+    regions = [torch.ones_like(valid)] if mask is None else [torch.ones_like(valid), mask != 0, mask == 0]
+    out = torch.full((pred.shape[0], len(regions), 8), float("nan"), dtype=torch.float64, device=pred.device)
+    for b in range(pred.shape[0]):
+        for r, region in enumerate(regions):
+            sel = valid[b] & region[b]
+            pp, gg = p[b][sel], g[b][sel]
+            out[b, r, 0] = pp.numel()
+            if pp.numel() == 0:
+                continue
+            # means as sum / n, correctly rounded: on CUDA, .mean() and "/ n" with a Python n multiply by 1 / n
+            n = torch.tensor(float(pp.numel()), dtype=torch.float64, device=pp.device)
+            e = pp - gg
+            ratio = torch.maximum(pp / gg, gg / pp)
+            out[b, r, 1] = (e.abs() / gg).sum() / n
+            out[b, r, 2] = (e * e / gg).sum() / n
+            out[b, r, 3] = ((e * e).sum() / n).sqrt()
+            out[b, r, 4] = (((pp.log() - gg.log()) ** 2).sum() / n).sqrt()
+            for k, t in enumerate(DELTA_THRESHOLDS):
+                out[b, r, 5 + k] = (ratio < t).sum(dtype=torch.float64) / n
+    return out
+
+
 def optional_lpips(device):
     """torchmetrics' LearnedPerceptualImagePatchSimilarity if importable AND its weights are available, else None."""
     try:
