@@ -368,6 +368,21 @@ int64_t kp_depth_metrics_scratch_bytes(int B, int64_t HW, int masked);
 int kp_depth_metrics(const float* pred, const float* gt, const float* dir_norm, const uint8_t* mask, int B, int64_t HW,
                      void* scratch, double* out, void* stream);
 
+/* ---- eval error maps: per pixel the quantities kp_image_metrics and kp_depth_metrics average, for viewing.  pred, gt:
+ *      fp32 [B,H,W,3], H and W >= 11; outputs fp32 [B,H,W]:
+ *        err       = (|pred_0 - gt_0| + |pred_1 - gt_1| + |pred_2 - gt_2|) / 3;
+ *        ssim      = at 5 <= y < H-5, 5 <= x < W-5 the channel mean of the SSIM of the window centred on (y, x), with
+ *                    kp_image_metrics' window, constants and per-image data_range (each channel's value is the one
+ *                    kp_image_metrics adds to its mean); NaN on the 5-pixel border, where no window lies inside;
+ *        depth_err = |max(depth, 1e-6) - g| / g in double, rounded to fp32, g = __fmul_rn(gt_depth, dir_norm) or gt_depth,
+ *                    NaN where g is not finite or not > 0 (kp_depth_metrics' clamp, product and validity rule).
+ *      depth, gt_depth: fp32 [B,H,W], given together with depth_err or all three NULL; dir_norm: fp32 [B,H,W] or NULL.
+ *      scratch: kp_eval_maps_scratch_bytes(B, H, W) device bytes, 16-byte aligned.  2 launches, no host
+ *      synchronisation, no atomics (bitwise reproducible), graph-capturable. ---- */
+int64_t kp_eval_maps_scratch_bytes(int B, int H, int W);
+int kp_eval_maps(const float* pred, const float* gt, const float* depth, const float* gt_depth, const float* dir_norm, int B,
+                 int H, int W, void* scratch, float* err, float* ssim, float* depth_err, void* stream);
+
 /* ---- frame composition for a rendered camera path (the per-frame image work of ns-render, REF/nerfstudio/scripts/
  *      render.py: colour-map every requested output and concatenate them along the width): P <= KP_COMPOSE_MAX_PANELS
  *      panels of one frame -> out uint8 [H, W*P, 3], panel p in columns [p*W, (p+1)*W).  panels: HOST array [P] of fp32

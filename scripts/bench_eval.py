@@ -7,6 +7,7 @@ the torch restatement of PSNR + SSIM (utils/image_metrics.py) on the same frames
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 scripts/bench_eval.py   # 8 GPUs (images i % 8 == rank)
     python scripts/bench_eval.py --regions        # also the per-region metrics, the median masks, Evaluator(regions="median")
     python scripts/bench_eval.py --depth          # also the depth metrics (kp_depth_metrics) and the Evaluator with eval depth
+    python scripts/bench_eval.py --write-images   # also the error maps (kp_eval_maps) and the eval image / video writers
 
 Prints one JSON line (rank 0).  The eval targets are the model's own frames plus seeded noise: the metric values are
 not a quality statement, the times are the point.  Kernel timing: CUDA events around each pass, after warm-up, with a
@@ -172,6 +173,78 @@ def depth_timing(depth, gt, norms, mask, reps: int) -> dict:
             "max_rel_diff_sums_vs_torch": float(rel.max()), "rows": ours.tolist(), "l2_flush": "512 MB written before every pass"}
 
 
+def maps_timing(pred, target, reps: int) -> dict:
+    """--write-images: median ms of ops.eval_maps on the batch against its torch restatement (fp32: the channel-mean
+    error and utils.image_metrics.ssim_map image by image), with L2 overwritten before every pass."""
+    from soccernerfs_b200 import ops
+    from soccernerfs_b200.utils import image_metrics
+
+    flush = torch.empty(512 * 2**20 // 4, dtype=torch.float32, device=pred.device)
+    p4 = [torch.moveaxis(p, -1, 0)[None] for p in pred]
+    t4 = [torch.moveaxis(t, -1, 0)[None] for t in target]
+
+    def torch_pass():
+        return (pred - target).abs().mean(-1), [image_metrics.ssim_map(t, p)[0].mean(0) for p, t in zip(p4, t4)]
+
+    def timed(fn):
+        for _ in range(3):
+            fn()
+        times = []
+        for _ in range(reps):
+            flush.fill_(1.0)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            fn()
+            e1.record()
+            torch.cuda.synchronize()
+            times.append(e0.elapsed_time(e1))
+        return sorted(times)[len(times) // 2], times
+
+    ours = ops.eval_maps(pred, target)
+    err, ssim = torch_pass()
+    k_ms, k_all = timed(lambda: ops.eval_maps(pred, target))
+    t_ms, _ = timed(torch_pass)
+    b, h, w = pred.shape[:3]
+    bytes_moved = 2 * b * h * w * 3 * 4 * 2 + 2 * b * h * w * 4  # both images read twice (min/max, map), two maps written
+    return {"kp_eval_maps_ms": k_ms, "torch_maps_ms": t_ms, "speedup": t_ms / k_ms, "kp_ms_all": k_all,
+            "kp_bytes_moved_min": bytes_moved, "kp_effective_gbs": bytes_moved / (k_ms * 1e-3) / 1e9,
+            "max_abs_diff_error_vs_torch": float((ours["error"] - err).abs().max()),
+            "max_abs_diff_ssim_vs_torch_fp32": float(max((ours["ssim"][k, 5:h - 5, 5:w - 5] - s).abs().max() for k, s in enumerate(ssim))),
+            "l2_flush": "512 MB written before every pass"}
+
+
+def write_timing(evaluator, n_images: int, repeats: int) -> dict:
+    """--write-images: seconds per image of write_eval_images (PNG and JPEG) and write_eval_videos, each alternated with
+    get_average_eval_image_metrics in the same run, into a temporary directory."""
+    import shutil
+    import tempfile
+
+    out = tempfile.mkdtemp(prefix="bench_eval_images_")
+    jobs = {"metrics": lambda r: evaluator.get_average_eval_image_metrics(r),
+            "images_png": lambda r: evaluator.write_eval_images(os.path.join(out, "png")),
+            "images_jpeg": lambda r: evaluator.write_eval_images(os.path.join(out, "jpeg"), image_format="jpeg"),
+            "videos": lambda r: evaluator.write_eval_videos(os.path.join(out, "video"), 25.0)}
+    try:
+        for fn in jobs.values():  # warm-up
+            fn(0)
+        times = {k: [] for k in jobs}
+        for r in range(repeats):
+            for k, fn in jobs.items():
+                if evaluator.world > 1:
+                    torch.distributed.barrier()
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                fn(r + 1)  # every writer ends once its files are written
+                torch.cuda.synchronize()
+                times[k].append((time.perf_counter() - t0) / n_images)
+        sizes = {k: sum(os.path.getsize(os.path.join(out, k, f)) for f in os.listdir(os.path.join(out, k))) for k in ("png", "jpeg", "video")}
+    finally:
+        shutil.rmtree(out)
+    med = {k: sorted(v)[len(v) // 2] for k, v in times.items()}
+    return {"seconds_per_image": med, "seconds_per_image_all": times, "bytes_written": sizes,
+            "panels": ["gt", "rgb", "error", "ssim"], "overhead_over_metrics": {k: med[k] / med["metrics"] for k in med}}
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--images", type=int, default=8)
@@ -186,6 +259,9 @@ def main() -> None:
     ap.add_argument("--depth", action="store_true",
                     help="also time the depth metrics (kp_depth_metrics against torch, masked against unmasked) and the "
                          "Evaluator with eval depth against the one without")
+    ap.add_argument("--write-images", action="store_true",
+                    help="also time the eval error maps (kp_eval_maps against torch) and writing the eval split as PNG, "
+                         "JPEG and video (write_eval_images / write_eval_videos) against get_average_eval_image_metrics")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_eval.py measures on a CUDA device; none is visible")
@@ -279,7 +355,11 @@ def main() -> None:
                            "seconds_per_call_without_depth": sorted(plain_calls)[len(plain_calls) // 2],
                            "seconds_per_call_all": depth_calls, "seconds_per_call_without_depth_all": plain_calls,
                            "results": depth_res}
+    if args.write_images:
+        result["write_images"] = write_timing(evaluator, args.images, args.repeats)
     if rank == 0:
+        if args.write_images:
+            result["write_images"]["kernel"] = maps_timing(torch.stack(renders), targets, args.kernel_reps)
         result["kernel"] = kernel_vs_torch(torch.stack(renders), targets, args.kernel_reps)
         if args.depth:  # masks: the median masks of the 8 frames as one camera's clip, as --regions takes them
             from soccernerfs_b200.engine.evaluator import median_dynamic_masks

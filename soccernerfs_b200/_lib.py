@@ -84,6 +84,8 @@ SIGNATURES = {
     "kp_image_metrics_masked": ([_P, _P, _P, c_int, c_int, c_int, _P, _P, _P], c_int),
     "kp_depth_metrics_scratch_bytes": ([c_int, c_int64, c_int], c_int64),
     "kp_depth_metrics": ([_P, _P, _P, _P, c_int, c_int64, _P, _P, _P], c_int),
+    "kp_eval_maps_scratch_bytes": ([c_int, c_int, c_int], c_int64),
+    "kp_eval_maps": ([_P, _P, _P, _P, _P, c_int, c_int, c_int, _P, _P, _P, _P, _P], c_int),
     "kp_compose_frame_scratch_bytes": ([c_int, c_int, c_int], c_int64),
     "kp_compose_frame": ([_P, POINTER(c_int), c_int, c_int, c_int, _P, _P, _P, _P, _P, _P], c_int),
     "kp_compose_frame_accs": ([_P, POINTER(c_int), _P, c_int, c_int, c_int, _P, _P, _P, _P, _P], c_int),

@@ -18,10 +18,18 @@ When the eval split carries ground-truth depth (``DynamicDataManager(eval_extras
 ``depth`` frames of the same images go through one ``ops.depth_metrics`` call per rank (``depth_abs_rel`` ...
 ``depth_delta3``, per region too with ``regions``): the geometry the preset's depth supervision trains, which colour
 metrics cannot tell apart from a flat billboard that looks right from near the training cameras.
+
+``write_eval_images`` / ``write_eval_videos`` show where those numbers come from: each eval image is rendered once, its
+per-pixel error, SSIM and depth-error maps come from ``ops.eval_maps``, and the panels (``eval_panels``) are composed
+and, for JPEG and video, encoded on the device through the render side's frame loop (``path_renderer._frame_loop``).
+The per-image rows written beside the images come from ``_measure``, the same kernels ``get_average_eval_image_metrics``
+averages with, one image at a time.
 """
 from __future__ import annotations
 
+import json
 import math
+import os
 from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple, Union
 
 import torch
@@ -128,6 +136,62 @@ def unpack_rows(packed: Sequence[torch.Tensor], keys: Sequence[str]) -> Dict[int
     return rows
 
 
+MAP_PANELS = ("error", "ssim", "depth_error")  # the panels of ops.eval_maps
+
+
+def eval_panels(model, depth: bool, regions: bool) -> List[str]:
+    """The panels ``Evaluator.write_eval_images`` can show: the eval image ``gt``, the renderer's outputs, the error maps;
+    with eval depth the ground-truth depth ``depth_gt`` and ``depth_error``; with regions the ``dynamic_mask``."""
+    names = ["gt", "rgb", "median_rgb", "error", "ssim", "depth", "accumulation"]
+    names += [f"prop_depth_{i}" for i in range(getattr(model.config, "num_proposal_iterations", 0))]
+    names += ["depth_gt", "depth_error"] if depth else []
+    return names + (["dynamic_mask"] if regions else [])
+
+
+def check_eval_panels(available: Sequence[str], panels: Sequence[str], error_range: float, depth_error_range: float) -> List[str]:
+    """The ValueErrors of ``write_eval_images`` / ``write_eval_videos``, raised before anything is rendered."""
+    names = list(panels)
+    if not names:
+        raise ValueError(f"no panels; available panels: {list(available)}")
+    missing = [n for n in names if n not in available]
+    if missing:
+        raise ValueError(f"panel(s) {missing} not available (depth_gt and depth_error need eval depth, dynamic_mask needs "
+                         f"regions); available panels: {list(available)}")
+    if len(names) > ops.COMPOSE_MAX_PANELS:
+        raise ValueError(f"at most {ops.COMPOSE_MAX_PANELS} panels per image (got {len(names)})")
+    for name, r in (("error_range", error_range), ("depth_error_range", depth_error_range)):
+        if isinstance(r, bool) or not isinstance(r, (int, float)) or not (r > 0 and math.isfinite(r)):
+            raise ValueError(f"{name} must be positive and finite (got {r!r})")
+    return names
+
+
+def eval_video_sequences(ids: Optional[torch.Tensor], times: Optional[torch.Tensor], n_images: int) -> Dict[str, List[int]]:
+    """{video file name: eval image indices in play order}: ``camera_{id:03d}.avi`` per camera id with that camera's
+    images ordered by time (equal times in image order); without ids one ``eval.avi`` in image order."""
+    if ids is None:
+        return {"eval.avi": list(range(n_images))}
+    cam = [int(v) for v in ids.reshape(-1).tolist()]
+    t = [0.0] * n_images if times is None else [float(v) for v in times.reshape(-1).tolist()]
+    if len(cam) != n_images or len(t) != n_images:
+        raise ValueError(f"{len(cam)} camera ids and {len(t)} times for {n_images} eval images")
+    return {f"camera_{c:03d}.avi": sorted((i for i in range(n_images) if cam[i] == c), key=lambda i: (t[i], i))
+            for c in sorted(set(cam))}
+
+
+def metrics_file_name(rank: int, world: int, gathered: bool) -> Optional[str]:
+    """The file rank ``rank`` writes the per-image rows to: ``metrics.json`` with one rank, or on rank 0 when the rows
+    were gathered over a process group (None on the other ranks); else ``metrics.rank{r}.json`` with its own rows."""
+    if world == 1 or gathered:
+        return "metrics.json" if rank == 0 else None
+    return f"metrics.rank{rank}.json"
+
+
+def metrics_document(rows: Dict[int, Dict[str, float]], extension: str) -> Dict[str, Any]:
+    """The content of ``metrics.json``: {"images": [{"image": i, "file": "{i:05d}.{extension}", <row>}, ...]} in image
+    order."""
+    return {"images": [dict({"image": i, "file": f"{i:05d}.{extension}"}, **rows[i]) for i in sorted(rows)]}
+
+
 def eval_report(results: Dict[str, float], experiment_name: str, checkpoint: str,
                 method_name: str = KPLANES_TRAINER["method_name"]) -> Dict[str, Any]:
     """The JSON ``ns-eval`` writes: {experiment_name, method_name, checkpoint, results}."""
@@ -220,6 +284,29 @@ class Evaluator:
             self._lpips_checked = True
         return self._lpips
 
+    def _value_keys(self) -> List[str]:
+        """The columns of ``_measure``: psnr, ssim, [REGION_KEYS, dynamic_fraction], [depth_row_keys]."""
+        keys = ["psnr", "ssim"] + (list(REGION_KEYS) + ["dynamic_fraction"] if self.regions is not None else [])
+        return keys + depth_row_keys(self.regions is not None) if self.depth else keys
+
+    def _measure(self, sel: Union[torch.Tensor, slice], pred: torch.Tensor, depth: Optional[torch.Tensor] = None,
+                 norms: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The ``_value_keys`` columns [B, K] on the device of the renders ``pred`` [B,H,W,3] (``depth``, ``norms``
+        [B,H,W,1] with eval depth) of the eval images ``sel`` (an index tensor or a slice).  No host synchronisation.
+        A row depends only on its own image, so one image at a time gives the bits of the whole batch."""
+        batch = self.datamanager.eval_image_cache.batch
+        target = batch["image"][sel]
+        values = ops.image_metrics(pred, target)
+        mask = None
+        if self.regions is not None:
+            mask = self.regions.to(pred.device)[sel]
+            fraction = mask.flatten(1).sum(1, dtype=torch.float64) / mask[0].numel()
+            values = torch.cat([values.double(), ops.image_metrics_masked(pred, target, mask).double(), fraction[:, None]], 1)
+        if self.depth:
+            depth = ops.depth_metrics(depth, batch["depth_image"][sel], norms, mask)
+            values = torch.cat([values.double(), depth[:, :, 1:].flatten(1)], 1)  # (n_valid dropped: NaN marks "undefined")
+        return values
+
     def _rank_rows(self, mine: Sequence[int]) -> Dict[int, Dict[str, float]]:
         """Per-image rows {psnr, ssim, [lpips], num_rays_per_sec, fps, [REGION_KEYS, dynamic_fraction],
         [depth_row_keys]} of this rank's images."""
@@ -228,20 +315,13 @@ class Evaluator:
         renders = [self._render_timed(i, depth=True) if self.depth else self._render_timed(i) for i in mine]
         pred = torch.stack([r[0] for r in renders])
         idx = torch.tensor(mine, device=pred.device)
-        target = self.datamanager.eval_image_cache.batch["image"][idx]
-        values = ops.image_metrics(pred, target)
-        mask = None
-        if self.regions is not None:
-            mask = self.regions.to(pred.device)[idx]
-            fraction = mask.flatten(1).sum(1, dtype=torch.float64) / mask[0].numel()
-            values = torch.cat([values.double(), ops.image_metrics_masked(pred, target, mask).double(), fraction[:, None]], 1)
+        depth = norms = None
         if self.depth:
-            norms = [r[3] for r in renders]
-            depth = ops.depth_metrics(torch.stack([r[2] for r in renders]), self.datamanager.eval_image_cache.batch["depth_image"][idx],
-                                      None if norms[0] is None else torch.stack(norms), mask)
-            values = torch.cat([values.double(), depth[:, :, 1:].flatten(1)], 1)  # (n_valid dropped: NaN marks "undefined")
-        values = values.tolist()  # the one host synchronisation: the events have completed too
-        n_colour = 2 if self.regions is None else 7
+            depth = torch.stack([r[2] for r in renders])
+            norms = None if renders[0][3] is None else torch.stack([r[3] for r in renders])
+        values = self._measure(idx, pred, depth, norms).tolist()  # the one host synchronisation: the events have completed too
+        keys = self._value_keys()
+        target = self.datamanager.eval_image_cache.batch["image"][idx]
         lpips = self._lpips_metric(pred.device)
         rows = {}
         for k, i in enumerate(mine):
@@ -251,10 +331,7 @@ class Evaluator:
                 row["lpips"] = float(lpips(torch.moveaxis(target[k], -1, 0)[None], torch.moveaxis(pred[k], -1, 0)[None]))
             row["num_rays_per_sec"] = h * w / renders[k][1]()
             row["fps"] = row["num_rays_per_sec"] / (h * w)
-            if self.regions is not None:
-                row.update(zip(REGION_KEYS + ("dynamic_fraction",), values[k][2:n_colour]))
-            if self.depth:
-                row.update(zip(depth_row_keys(self.regions is not None), values[k][n_colour:]))
+            row.update(zip(keys[2:], values[k][2:]))
             rows[i] = row
         return rows
 
@@ -287,3 +364,118 @@ class Evaluator:
         if self.depth:
             out.update(average_depth_metrics(rows, self.regions is not None))
         return out
+
+    # ---- the eval images as files ----
+    def _eval_frame(self, i: int, names: Sequence[str], error_range: float, depth_error_range: float,
+                    values: Optional[Dict[int, torch.Tensor]] = None) -> torch.Tensor:
+        """Render eval image i once and compose ``names`` on the device (uint8 [H, W*P, 3]); with ``values``, also put
+        its ``_measure`` row (on the device) in ``values[i]``."""
+        out = self.renderer.render(i, device_frames=True)
+        batch = self.datamanager.eval_image_cache.batch
+        pred, target = out["rgb"], batch["image"][i]
+        norms = out.get("directions_norm")
+        depth = gt_depth = None
+        if self.depth:
+            depth, gt_depth = out["depth"], batch["depth_image"][i]
+        if values is not None:
+            values[i] = self._measure(slice(i, i + 1), pred[None], None if depth is None else depth[None],
+                                      None if norms is None else norms[None])
+        frames = dict(out, gt=target)
+        if any(n in MAP_PANELS for n in names):
+            maps = ops.eval_maps(pred[None], target[None], None if depth is None else depth[None],
+                                 None if gt_depth is None else gt_depth[None], None if norms is None else norms[None])
+            frames["error"] = (maps["error"][0] / error_range)[..., None]
+            frames["ssim"] = (1 - maps["ssim"][0])[..., None]  # bright = bad, as for the error; the NaN border shows as 0
+            if depth is not None:
+                frames["depth_error"] = (maps["depth_error"][0] / depth_error_range)[..., None]  # NaN (invalid) shows as 0
+        if "depth_gt" in names:
+            g = gt_depth if norms is None else gt_depth * norms  # z-depth -> distance along the ray, as the metrics compare
+            valid = torch.isfinite(g) & (g > 0)
+            # invalid pixels: white (accumulation 0) and the valid minimum, so they set neither near nor far
+            frames["depth_gt"] = torch.where(valid, g, torch.where(valid, g, math.inf).amin())
+            frames["depth_gt_valid"] = valid.float()
+        if "dynamic_mask" in names:
+            frames["dynamic_mask"] = self.regions[i].float()[..., None]
+        return ops.compose_frame(frames, names)
+
+    def _check_write(self, panels, error_range: float, depth_error_range: float) -> List[str]:
+        return check_eval_panels(eval_panels(self.model, self.depth, self.regions is not None), panels, error_range,
+                                 depth_error_range)
+
+    def write_eval_images(self, output_dir: Union[str, os.PathLike], panels: Sequence[str] = ("gt", "rgb", "error", "ssim"),
+                          image_format: str = "png", jpeg_quality: int = 95, error_range: float = 0.25,
+                          depth_error_range: float = 0.25) -> List[int]:
+        """Write this rank's eval images (``i % world == rank``) as ``output_dir/{i:05d}.png`` (PIL on the host) or
+        ``.jpg`` (``image_format="jpeg"``, encoded on the device): the ``panels`` side by side (``eval_panels``).
+        ``error``: viridis of the per-pixel error / ``error_range``; ``ssim``: viridis of 1 - the per-pixel SSIM (the
+        5-pixel border, where no window lies inside, shows as 0); ``depth_gt``: the ground-truth depth through turbo over
+        its own near / far, white where it is invalid; ``depth_error``: viridis of the relative depth error /
+        ``depth_error_range`` (0 where the ground truth is invalid); ``dynamic_mask``: the ``regions`` mask.  Values
+        beyond a range show as its top colour.
+
+        Each image is rendered once; maps, composition and JPEG run on the device while the previous image is written.
+        Also writes the per-image rows (psnr, ssim, the region and depth keys; bit for bit the rows
+        ``get_average_eval_image_metrics`` averages) to ``metrics.json`` (``metrics_document``): with a process group
+        rank 0 writes every rank's rows, without one each rank of several writes ``metrics.rank{r}.json``.  Returns the
+        image indices this rank wrote."""
+        from .path_renderer import IMAGE_FORMATS, _frame_loop, check_jpeg_quality, file_writer
+
+        names = self._check_write(panels, error_range, depth_error_range)
+        if image_format not in IMAGE_FORMATS:
+            raise ValueError(f"image_format {image_format!r} is not one of {IMAGE_FORMATS}")
+        check_jpeg_quality(jpeg_quality)
+        out = os.fspath(output_dir)
+        os.makedirs(out, exist_ok=True)
+        n = len(self.datamanager.eval_cameras)
+        mine = images_of_rank(n, self.rank, self.world)
+        h, w = self.datamanager.eval_image_cache.batch["image"].shape[1:3]
+        values: Dict[int, torch.Tensor] = {}
+        _frame_loop(lambda i: self._eval_frame(i, names, error_range, depth_error_range, values), mine, (h, w * len(names)),
+                    self.datamanager.device, None if image_format == "png" else jpeg_quality, file_writer(out, image_format))
+        keys = self._value_keys()
+        table = torch.cat([values[i] for i in mine]).tolist() if mine else []
+        rows = {i: dict(zip(keys, table[k])) for k, i in enumerate(mine)}
+        gathered = self.world > 1 and torch.distributed.is_available() and torch.distributed.is_initialized()
+        if gathered:
+            rows = self._all_gather(rows, keys, n)
+        name = metrics_file_name(self.rank, self.world, gathered)
+        if name is not None:
+            with open(os.path.join(out, name), "w", encoding="utf-8") as f:
+                json.dump(metrics_document(rows, "png" if image_format == "png" else "jpg"), f, indent=1)
+        return mine
+
+    def write_eval_videos(self, output_dir: Union[str, os.PathLike], fps: float,
+                          panels: Sequence[str] = ("gt", "rgb", "error", "ssim"), jpeg_quality: int = 95,
+                          error_range: float = 0.25, depth_error_range: float = 0.25) -> Dict[str, List[int]]:
+        """Write the eval split as Motion-JPEG AVIs at ``fps`` frames per second: ``camera_{id:03d}.avi`` per eval camera
+        id with its images in time order, or one ``eval.avi`` in image order without ids (``eval_video_sequences``);
+        each frame is ``panels`` side by side, as ``write_eval_images`` composes them.  The k-th frame of a video goes to
+        rank ``k % world``, which encodes it into its part file.  With one rank the videos are written at once; with a
+        process group the ranks meet at a barrier and rank 0 assembles them; without one the caller runs
+        ``assemble_video(path, world, fps)`` for each returned path once every rank is done.  ``fps`` is required:
+        eval frames are usually subsampled from the clip, so only the caller knows their rate.  Returns {video path:
+        the image indices this rank encoded into it}."""
+        from .path_renderer import assemble_video, check_jpeg_quality, write_part
+
+        names = self._check_write(panels, error_range, depth_error_range)
+        check_jpeg_quality(jpeg_quality)
+        if isinstance(fps, bool) or not isinstance(fps, (int, float)) or not (fps > 0 and math.isfinite(fps)):
+            raise ValueError(f"fps must be positive and finite (got {fps!r})")
+        out = os.fspath(output_dir)
+        os.makedirs(out, exist_ok=True)
+        cams = self.datamanager.eval_cameras
+        h, w = self.datamanager.eval_image_cache.batch["image"].shape[1:3]
+        written = {}
+        for name, seq in eval_video_sequences(cams.ids, cams.times, len(cams)).items():
+            path = os.path.join(out, name)
+            written[path] = write_part(path, self.rank, lambda i: self._eval_frame(i, names, error_range, depth_error_range),
+                                       seq[self.rank::self.world], (h, w * len(names)), self.datamanager.device, jpeg_quality)
+        if self.world == 1:
+            for path in written:
+                assemble_video(path, 1, fps)
+        elif torch.distributed.is_available() and torch.distributed.is_initialized():
+            torch.distributed.barrier()
+            if self.rank == 0:
+                for path in written:
+                    assemble_video(path, self.world, fps)
+        return written

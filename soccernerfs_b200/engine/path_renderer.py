@@ -104,14 +104,9 @@ def _land_jpeg(done: torch.cuda.Event, data: torch.Tensor, ring: List[torch.Tens
     return write(i, host)
 
 
-def _frame_loop(model, cameras: Cameras, names: List[str], rank: int, world: int, crop: Optional[CropData],
-                jpeg_quality: Optional[int], write: Callable, collect: Optional[Callable] = None) -> List[int]:
-    """The render loop of every output format.  Frame i of this rank (``i % world == rank``) is rendered, composed and,
-    with a ``jpeg_quality``, encoded on the device; a copy stream moves it into a ring of pinned host buffers and
-    ``write(i, data)`` runs on a pool thread once it has landed: ``data`` is the composed uint8 image [H, W*P, 3], or
-    the JPEG file's bytes (uint8 [n]; the length is copied first, then exactly n bytes).  ``collect(i, result)`` gets
-    the results of ``write`` on this thread in frame order.  The loop itself never synchronises with the device; it
-    waits only for the pool when every ring buffer is still in use.  Returns the frame indices of this rank."""
+def _path_frames(model, cameras: Cameras, names: List[str], crop: Optional[CropData]):
+    """-> (produce, context, (H, W*P)): ``produce(i)`` renders frame i of the path and composes ``names`` on the device
+    (uint8 [H, W*P, 3]); it runs inside ``context`` (the crop's background colour)."""
     dev = model.device
     if cameras.device != dev:
         cameras = cameras.to(dev)
@@ -119,17 +114,31 @@ def _frame_loop(model, cameras: Cameras, names: List[str], rank: int, world: int
     for n in names:  # each depth panel is blended with its own accumulation
         if ops.panel_kind(n) == 2 and ops.accumulation_of(n) not in outputs:
             outputs.append(ops.accumulation_of(n))
-    mine = images_of_rank(len(cameras), rank, world)
     aabb_box = None
     bg = None
     if crop is not None:
         aabb_box = crop.scene_box
         bg = crop.background_color.to(dev, torch.float32)  # on the device: the tile graphs read it, no copy in the capture
     renderer = FrameRenderer(model, cameras, outputs=outputs, aabb_box=aabb_box)  # whole frames per rank
-    h, w = cameras._height_host[0], cameras._width_host[0]
+    context = background_color_override_context(bg) if bg is not None else contextlib.nullcontext()
+    return (lambda i: ops.compose_frame(renderer.render(i, device_frames=True), names)), context, \
+        (cameras._height_host[0], cameras._width_host[0] * len(names))
+
+
+def _frame_loop(produce: Callable[[int], torch.Tensor], mine: Sequence[int], size: Tuple[int, int], dev,
+                jpeg_quality: Optional[int], write: Callable, collect: Optional[Callable] = None) -> List[int]:
+    """The write loop of every output format.  For each frame i of ``mine`` in order, ``produce(i)`` gives the composed
+    uint8 image [H, W', 3] (``size`` = (H, W')) on the current stream, which is encoded on the device with a
+    ``jpeg_quality``; a copy stream moves it into a ring of pinned host buffers and ``write(i, data)`` runs on a pool
+    thread once it has landed: ``data`` is the composed image, or the JPEG file's bytes (uint8 [n]; the length is copied
+    first, then exactly n bytes).  ``collect(i, result)`` gets the results of ``write`` on this thread in frame order.
+    The loop itself never synchronises with the device; it waits only for the pool when every ring buffer is still in
+    use, so the device produces frame k+1 while frame k is written.  Returns ``mine``."""
+    mine = list(mine)
+    h, w = size
     slots = min(RING_SLOTS, len(mine))
     # JPEG: sized like the raw image, grown by the pool thread in the rare case a file is larger
-    shape = (h, w * len(names), 3) if jpeg_quality is None else (h * w * len(names) * 3,)
+    shape = (h, w, 3) if jpeg_quality is None else (h * w * 3,)
     ring = [torch.empty(shape, dtype=torch.uint8).pin_memory() for _ in range(slots)]
     lengths = torch.empty(max(slots, 1), dtype=torch.int64).pin_memory() if jpeg_quality is not None else None
     pending: List[Optional[Future]] = [None] * slots
@@ -142,14 +151,12 @@ def _frame_loop(model, cameras: Cameras, names: List[str], rank: int, world: int
         if collect is not None:
             collect(mine[k], result)
 
-    with ThreadPoolExecutor(max_workers=max(1, slots)) as pool, \
-            (background_color_override_context(bg) if bg is not None else contextlib.nullcontext()):
+    with ThreadPoolExecutor(max_workers=max(1, slots)) as pool:
         for k, i in enumerate(mine):
             slot = k % slots
             if k >= slots:
                 finish(k - slots)  # ring full: this buffer's frame is still being written
-            frames = renderer.render(i, device_frames=True)
-            image = ops.compose_frame(frames, names)
+            image = produce(i)
             if jpeg_quality is None:
                 copy_stream.wait_stream(main)
                 with torch.cuda.stream(copy_stream):
@@ -186,7 +193,15 @@ def render_camera_path(model, cameras: Cameras, output_dir: Union[str, os.PathLi
     check_jpeg_quality(jpeg_quality)
     out = os.fspath(output_dir)
     os.makedirs(out, exist_ok=True)
+    produce, context, size = _path_frames(model, cameras, list(rendered_output_names), crop)
+    with context:
+        return _frame_loop(produce, images_of_rank(len(cameras), rank, world), size, model.device,
+                           None if image_format == "png" else jpeg_quality, file_writer(out, image_format))
 
+
+def file_writer(out: str, image_format: str) -> Callable:
+    """The ``write`` of ``_frame_loop`` for image files: a composed image to ``out/{i:05d}.png`` through PIL, or the JPEG
+    bytes to ``out/{i:05d}.jpg``."""
     def write_png(i: int, image: torch.Tensor) -> None:
         from PIL import Image
 
@@ -196,9 +211,7 @@ def render_camera_path(model, cameras: Cameras, output_dir: Union[str, os.PathLi
         with open(os.path.join(out, f"{i:05d}.jpg"), "wb") as f:
             f.write(data.numpy().tobytes())
 
-    if image_format == "png":
-        return _frame_loop(model, cameras, list(rendered_output_names), rank, world, crop, None, write_png)
-    return _frame_loop(model, cameras, list(rendered_output_names), rank, world, crop, jpeg_quality, write_jpeg)
+    return write_png if image_format == "png" else write_jpeg
 
 
 # ---- Motion-JPEG AVI (RIFF AVI 1.0): every frame a baseline JPEG in a '00dc' chunk of 'movi', all keyframes ----
@@ -210,6 +223,18 @@ _AVIIF_KEYFRAME = 0x10
 def part_path(output_path: Union[str, os.PathLike], rank: int) -> str:
     """The file rank ``rank`` writes its encoded frames to before ``assemble_video`` interleaves them."""
     return f"{os.fspath(output_path)}.part{rank}"
+
+
+def write_part(output_path: Union[str, os.PathLike], rank: int, produce: Callable[[int], torch.Tensor], frames: Sequence[int],
+               size: Tuple[int, int], dev, jpeg_quality: int) -> List[int]:
+    """Encode ``produce(i)`` of each of ``frames`` in order on the device and append the JPEGs to rank ``rank``'s part file
+    of ``output_path`` (records of uint32 little-endian n, n bytes).  Returns ``frames``."""
+    with open(part_path(output_path, rank), "wb") as part:
+
+        def append(i: int, data: bytes) -> None:
+            part.write(struct.pack("<I", len(data)) + data)
+
+        return _frame_loop(produce, frames, size, dev, jpeg_quality, lambda i, data: data.numpy().tobytes(), append)
 
 
 def _read_part(path: str) -> List[Tuple[int, int]]:
@@ -304,13 +329,9 @@ def render_camera_path_video(model, cameras: Cameras, output_path: Union[str, os
     fps = len(cameras) / seconds
     out_dir = os.path.dirname(os.path.abspath(output_path))
     os.makedirs(out_dir, exist_ok=True)
-    with open(part_path(output_path, rank), "wb") as part:
-
-        def append(i: int, data: bytes) -> None:
-            part.write(struct.pack("<I", len(data)) + data)
-
-        mine = _frame_loop(model, cameras, list(rendered_output_names), rank, world, crop, jpeg_quality,
-                           lambda i, data: data.numpy().tobytes(), append)
+    produce, context, size = _path_frames(model, cameras, list(rendered_output_names), crop)
+    with context:
+        mine = write_part(output_path, rank, produce, images_of_rank(len(cameras), rank, world), size, model.device, jpeg_quality)
     if world == 1:
         assemble_video(output_path, 1, fps)
     elif torch.distributed.is_available() and torch.distributed.is_initialized():

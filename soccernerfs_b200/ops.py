@@ -987,21 +987,75 @@ def depth_metrics(pred: torch.Tensor, gt: torch.Tensor, directions_norm: Optiona
     return out
 
 
+def eval_maps(pred: torch.Tensor, gt: torch.Tensor, depth: Optional[torch.Tensor] = None, gt_depth: Optional[torch.Tensor] = None,
+              directions_norm: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+    """Per-pixel error maps of a batch on the device (kp_eval_maps): pred, gt fp32 CUDA [B,H,W,3] with H, W >= 11; depth,
+    gt_depth and directions_norm fp32 [B,H,W] or [B,H,W,1] -> fp32 [B,H,W] maps in physical units:
+
+    - ``error``: the channel mean of |pred - gt|;
+    - ``ssim``: the channel mean of the SSIM window centred on each pixel (``image_metrics``' window, constants and data
+      range: ``utils.image_metrics.ssim_map`` averaged over channels), NaN on the 5-pixel border;
+    - ``depth_error`` (with ``depth`` and ``gt_depth``): |max(depth, 1e-6) - g| / g, g = gt_depth * directions_norm (fp32)
+      or gt_depth, NaN where g is not finite or not > 0 (``depth_metrics``' rule).
+
+    No host synchronisation, so it can be captured in a CUDA graph."""
+    if pred.dim() != 4 or pred.shape[-1] != 3 or gt.shape != pred.shape:
+        raise ValueError(f"eval_maps: pred and gt must both be [B,H,W,3] (got {tuple(pred.shape)}, {tuple(gt.shape)})")
+    if (depth is None) != (gt_depth is None):
+        raise ValueError("eval_maps: depth and gt_depth are given together")
+    if directions_norm is not None and depth is None:
+        raise ValueError("eval_maps: directions_norm needs depth and gt_depth")
+    maps = {"depth": depth, "gt_depth": gt_depth, "directions_norm": directions_norm}
+    for name, t in maps.items():
+        if t is not None and t.dim() == 4 and t.shape[-1] == 1:
+            maps[name] = t = t.squeeze(-1)
+        if t is not None and t.shape != pred.shape[:3]:
+            raise ValueError(f"eval_maps: {name} must be [B,H,W] or [B,H,W,1] = {tuple(pred.shape[:3])} (got {tuple(t.shape)})")
+    depth, gt_depth, directions_norm = maps["depth"], maps["gt_depth"], maps["directions_norm"]
+    b, h, w = pred.shape[:3]
+    if h < 11 or w < 11:
+        raise ValueError(f"eval_maps: {h}x{w} images are smaller than the 11x11 SSIM window")
+    tensors = [t for t in (pred, gt, depth, gt_depth, directions_norm) if t is not None]
+    if any(t.dtype != torch.float32 for t in tensors):
+        raise TypeError("eval_maps: every input must be float32")
+    if not pred.is_cuda or any(t.device != pred.device for t in tensors):
+        raise RuntimeError("eval_maps: every tensor must be a CUDA tensor on one device (there is no CPU path)")
+    pred, gt = pred.contiguous(), gt.contiguous()
+    depth, gt_depth, directions_norm = (None if t is None else t.contiguous() for t in (depth, gt_depth, directions_norm))
+    out = {"error": torch.empty((b, h, w), dtype=torch.float32, device=pred.device),
+           "ssim": torch.empty((b, h, w), dtype=torch.float32, device=pred.device)}
+    if depth is not None:
+        out["depth_error"] = torch.empty((b, h, w), dtype=torch.float32, device=pred.device)
+    if b == 0:
+        return out
+    scratch = torch.empty(int(_lib.load().kp_eval_maps_scratch_bytes(b, h, w)), dtype=torch.uint8, device=pred.device)
+    call("kp_eval_maps", ptr(pred), ptr(gt), ptr(depth), ptr(gt_depth), ptr(directions_norm), b, h, w,
+         c_void_p(scratch.data_ptr()), ptr(out["error"]), ptr(out["ssim"]), ptr(out.get("depth_error")), stream_ptr())
+    return out
+
+
 COMPOSE_MAX_PANELS = 8
 _COLORMAP_TABLES: Dict = {}
 
 
+SCALAR_PANELS = ("accumulation", "accumulation_static", "dynamic", "error", "ssim", "depth_error", "dynamic_mask")
+
+
 def panel_kind(name: str) -> int:
-    """How ``compose_frame`` maps a rendered output: 1 = a scalar in [0, 1] through viridis (accumulation,
-    accumulation_static, the dynamics score ``dynamic``), 2 = a depth (turbo, blended with its accumulation; ns-render's
-    rule: any name containing "depth"), 0 = a colour shown as it is."""
-    if name in ("accumulation", "accumulation_static", "dynamic"):
+    """How ``compose_frame`` maps a rendered output: 1 = a scalar in [0, 1] through viridis (``SCALAR_PANELS``: the
+    accumulations, the dynamics score ``dynamic`` and the eval maps the Evaluator scales into [0, 1]), 2 = a depth (turbo,
+    blended with its accumulation; ns-render's rule: any other name containing "depth"), 0 = a colour shown as it is."""
+    if name in SCALAR_PANELS:
         return 1
     return 2 if "depth" in name else 0
 
 
 def accumulation_of(name: str) -> str:
-    """The accumulation a depth panel is blended with: the static render's for ``depth_static``, else the frame's."""
+    """The accumulation a depth panel is blended with: the static render's for ``depth_static``, the ground truth's
+    validity mask ``depth_gt_valid`` (white where it has no depth) for the eval ground truth ``depth_gt``, else the
+    frame's."""
+    if name == "depth_gt":
+        return "depth_gt_valid"
     return "accumulation_static" if name.endswith("_static") else "accumulation"
 
 
